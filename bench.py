@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the RNN-T joint + transducer-loss hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one fused joint+loss forward AND backward over one synthetic batch.
   N = 1: B=32, T=400, U=100, H=1024, V=1024 -- BASELINE.json configs[1], the configuration the metric is quoted on.
@@ -130,6 +130,23 @@ def synth_inputs(torch, seed, device, b=B, t=T, u=U, pin=False, view=True):
     if view:
         d["enc"] = d["enc"].permute(0, 2, 1)
     return d
+
+
+def dump_outputs(torch, out_dir, loss, s_):
+    """What one step hands its caller -- the mean loss and the gradients of enc, pred, W and b -- as float32 .npy files
+    under out_dir, so that two builds can be compared output for output.  d_enc (52 MB at B=32) is kept for a fixed,
+    seeded quarter of its (b, t) frames (d_enc_sample.npy, frames in ascending b * T + t order); the whole dump stays
+    near 30 MB."""
+    import numpy as np
+    d_enc = s_["enc"].grad
+    nb, nt = d_enc.shape[:2]
+    frames = torch.randperm(nb * nt, generator=torch.Generator().manual_seed(0))[: nb * nt // 4].sort().values
+    frames = frames.to(d_enc.device)
+    arrays = dict(loss=loss.detach(), d_enc_sample=d_enc[frames // nt, frames % nt], d_pred=s_["pred"].grad,
+                  dW=s_["W"].grad, db=s_["b"].grad)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.float().cpu().numpy())
 
 
 # ----------------------------------------------------------------------------------------------- CPU arm
@@ -433,6 +450,8 @@ def run_gpu_arm(args):
     head = timed_region(args.steps, sets, not args.no_kernel_profile, True)
     ms_total = head["ms"]
     loss_val = float(head["last"].detach())
+    if args.dump_outputs and rank == 0:     # before the secondary loops below overwrite the gradients of these sets
+        dump_outputs(torch, args.dump_outputs, head["last"], sets[(args.steps - 1) % len(sets)])
 
     # ---- secondary numbers (single GPU only): every tile in the backward; a >= 3 s sustained loop under the power cap
     dense_ms, sustained = None, None
@@ -650,7 +669,11 @@ def main():
                     help="feed a dense (B,T,H) encoder tensor instead of the (B,H,T) view the reference model produces")
     ap.add_argument("--all-tiles", action="store_true",
                     help="backward processes every half-tile of the lattice (also those whose fp16 gradients are all zero)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and gradients of the last timed step to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference_arm(args)

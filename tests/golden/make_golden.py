@@ -22,7 +22,10 @@ from rnnt.predictor import ConvPredictor  # noqa: E402
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
-def loss_case(name, B, T, U, H, V, T_len, U_len, seed):
+def loss_case(name, B, T, U, H, V, T_len, U_len, seed, dW_rows=None):
+    """dW_rows=n keeps the file of a wide case under 1 MB: the float inputs are replaced by the seed and their checksums
+    (tests/helpers.py::load_loss_golden re-creates them), only a seeded choice of n rows of dW and no dense logits are
+    stored."""
     torch.manual_seed(seed)
     joint = JointNetwork(-1, -1, H, V)
     enc = torch.randn(B, H, T).permute(0, 2, 1).contiguous().requires_grad_(True)   # model.py:28 layout, made dense
@@ -37,8 +40,7 @@ def loss_case(name, B, T, U, H, V, T_len, U_len, seed):
     costs.sum().backward()
     mean = torchaudio.functional.rnnt_loss(logits=logits.detach(), targets=targets, logit_lengths=T_len,
                                            target_lengths=U_len, blank=-1, clamp=-1, reduction="mean")
-    np.savez_compressed(
-        os.path.join(HERE, name + ".npz"),
+    out = dict(
         enc=enc.detach().numpy(), pred=pred.detach().numpy(),
         W=joint.joint_ln.weight.detach().numpy(), b=joint.joint_ln.bias.detach().numpy(),
         targets=targets.numpy(), T_len=T_len.numpy(), U_len=U_len.numpy(),
@@ -48,6 +50,14 @@ def loss_case(name, B, T, U, H, V, T_len, U_len, seed):
         logits=logits.detach().numpy().astype(np.float32) if logits.numel() < 200000 else np.zeros(0, np.float32),
         dlogits=logits.grad.numpy() if logits.numel() < 200000 else np.zeros(0, np.float32),
     )
+    if dW_rows is not None:
+        for k in ("enc", "pred", "W", "b"):
+            out["chk." + k] = np.abs(out.pop(k).astype(np.float64)).sum()
+        rows = np.sort(np.random.default_rng(seed).choice(V, dW_rows, replace=False)).astype(np.int32)
+        out.update(seed=np.int64(seed), B=np.int32(B), T=np.int32(T), U=np.int32(U), H=np.int32(H), V=np.int32(V),
+                   dW=out["dW"][rows], dW_rows=rows)
+        del out["logits"], out["dlogits"]
+    np.savez_compressed(os.path.join(HERE, name + ".npz"), **out)
     print(name, "costs", costs.detach().numpy())
 
 
@@ -209,7 +219,7 @@ if __name__ == "__main__":
     # mid case: kernel-tile friendly sizes, ragged
     loss_case("loss_mid", B=3, T=37, U=13, H=128, V=256, T_len=[37, 20, 31], U_len=[13, 9, 4], seed=12)
     # wide case (H=V=512; the full H=V=1024 width is checked against the live oracle), short lattice
-    loss_case("loss_wide", B=2, T=19, U=9, H=512, V=512, T_len=[19, 11], U_len=[7, 9], seed=13)
+    loss_case("loss_wide", B=2, T=19, U=9, H=512, V=512, T_len=[19, 11], U_len=[7, 9], seed=13, dW_rows=384)
     decode_case("decode_small", n_utt=6, T=24, H=64, V=48, E=32, seed=21, max_length=40, scale=3.0, blank_bias=2.2)
     # round 2: pre-projection joint, the RNNTModel.forward glue, and decode at the full BASELINE configs[4] width
     proj_case("loss_proj", B=3, T=21, U=6, Fa=48, Ft=40, H=64, V=32, T_len=[21, 13, 17], U_len=[6, 2, 5], seed=31)

@@ -2,6 +2,7 @@
 from __future__ import annotations
 
 import ctypes as C
+import os
 
 import numpy as np
 import torch
@@ -66,6 +67,25 @@ def decode_full_setup(g):
     assert cs(joint.joint_ln.weight) == float(g["chk.joint_w"])
     assert cs(feats) == float(g["chk.feats"])
     return rnnt_b200.RNNTModel(predictor, torch.nn.Identity(), joint), feats, T_len
+
+
+def load_loss_golden(golden_dir, name):
+    """Arrays of tests/golden/<name>.npz (make_golden.py::loss_case) as a dict.  A case stored without its float inputs
+    is re-created from its seed in loss_case's drawing order and verified against the stored checksums.  Such a case
+    may keep only the rows `dW_rows` of dW; for the others `dW_rows` is every row."""
+    g = dict(np.load(os.path.join(golden_dir, name + ".npz")))
+    if "enc" not in g:
+        import rnnt_b200
+        B, T, U, H, V = (int(g[k]) for k in ("B", "T", "U", "H", "V"))
+        torch.manual_seed(int(g["seed"]))
+        joint = rnnt_b200.JointNetwork(-1, -1, H, V)
+        g["enc"] = torch.randn(B, H, T).permute(0, 2, 1).contiguous().numpy()
+        g["pred"] = torch.randn(B, U + 1, H).numpy()
+        g["W"], g["b"] = joint.joint_ln.weight.detach().numpy(), joint.joint_ln.bias.detach().numpy()
+        for k in ("enc", "pred", "W", "b"):
+            assert float(np.abs(g[k].astype(np.float64)).sum()) == float(g["chk." + k]), k
+    g.setdefault("dW_rows", np.arange(g["W"].shape[0]))
+    return g
 
 
 def make_inputs(B, T, U, H, V, seed=1234, ragged=False, device="cuda", scale=1.0):
