@@ -133,6 +133,49 @@ int rnnt_b200_greedy_decode(const float* enc, int64_t enc_sb, int64_t enc_st, co
                             int max_per_frame, int32_t* tokens, int32_t* n_tokens, float* margins_out, void* scratch,
                             void* stream);
 
+/* Streaming greedy decode: the loop of rnnt_b200_greedy_decode fed one chunk of encoder frames per call, for B slots
+ * (one live stream each) whose decoder state outlives the call.  Decoding an utterance in any sequence of consecutive
+ * chunks (zero-length ones included, other slots reset or fed in between, any slot, any B) gives the same tokens and
+ * per-step margins, bit for bit, as rnnt_b200_greedy_decode on the whole utterance with the same max_len and
+ * max_per_frame.
+ *
+ * state: rnnt_b200_greedy_decode_state_bytes(B, H, V, E) bytes, caller-owned, 128-byte aligned; its layout is that of
+ * the one-shot scratch.  It holds, per slot: the token count n (0 = empty slot, else 1 + tokens emitted, which is the
+ * predictor's next input position), the emit flag, the linear output `lin` and LayerNorm'd predictor features `feats`
+ * (H each), and the conv tap accumulators of conv1 (3E) and conv2 (5E); plus the two per-symbol tables
+ * (LayerNorm(embedding) (V, E) and conv1's tap products (V, 3E)) and the per-call scratch (frame counters, row lists,
+ * joint hidden rows, logits, conv outputs).  Its first 64 bytes hold the eight int64 counters of the last call, as for
+ * the one-shot scratch.
+ *
+ * rnnt_b200_greedy_decode_stream_init builds the symbol tables from the weights and empties every slot.  Run it
+ * before the first call and again whenever the weights change.
+ *
+ * rnnt_b200_greedy_decode_stream consumes enc (B, Tc, H) fp32 (strides (enc_sb, enc_st, 1), multiples of 4): slot b
+ * takes the first chunk_len[b] frames (clamped to [0, Tc]).  Slots with reset[b] != 0 (reset may be NULL) start a new
+ * utterance first: predictor state zeroed, the seed blank run through the predictor, n = 1 (the seed is counted, as
+ * rnnt/model.py:53,64 does).  Every other non-empty slot continues where its last call stopped, with the rule of
+ * rnnt/model.py:108-123.  A slot is finished when n == max_len and ignores frames until it is reset; empty slots
+ * ignore frames too.  A call always leaves a slot on a frame boundary (a frame is only left after a blank or the
+ * max_per_frame cap), so no per-frame counter crosses calls.  tokens (B, max_len) int32, caller-owned and kept
+ * between calls: the k-th token of the slot's utterance goes to column k-1, so this call added
+ * tokens[b, n_before-1 : n_after-1] (n_before = 1 for a reset slot).  n_tokens (B) int32 receives n after the call.
+ * margins_out (optional, (Tc + min(Tc * max_per_frame, max_len - 1) + 1, B) fp32, caller-initialised) receives the
+ * top-2 logit gap at [step, b] for every step of this call slot b was active in (steps 0, 1, ... of the call).
+ * Use the same max_len and max_per_frame for every call of a state. */
+size_t rnnt_b200_greedy_decode_state_bytes(int B, int H, int V, int E);
+int rnnt_b200_greedy_decode_stream_init(const float* joint_w, const float* joint_b, const float* emb,
+                                        const float* ln1_w, const float* ln1_b, const float* conv1_w,
+                                        const float* conv1_b, const float* conv2_w, const float* conv2_b,
+                                        const float* lin_w, const float* lin_b, const float* ln2_w, const float* ln2_b,
+                                        int B, int H, int V, int E, void* state, void* stream);
+int rnnt_b200_greedy_decode_stream(const float* enc, int64_t enc_sb, int64_t enc_st, const int32_t* chunk_len,
+                                   const int32_t* reset, const float* joint_w, const float* joint_b, const float* emb,
+                                   const float* ln1_w, const float* ln1_b, const float* conv1_w, const float* conv1_b,
+                                   const float* conv2_w, const float* conv2_b, const float* lin_w, const float* lin_b,
+                                   const float* ln2_w, const float* ln2_b, int B, int Tc, int H, int V, int E,
+                                   int blank, int max_len, int max_per_frame, int32_t* tokens, int32_t* n_tokens,
+                                   float* margins_out, void* state, void* stream);
+
 /* Optional pre-projections of the joint (rnnt/joint.py:8-12, 26-30: audio_ln / text_ln of the non-"convjs" configs) as
  * tcgen05 GEMMs ahead of the fused call, with their backward.  Row-major contiguous fp32 tensors:
  *   fwd:  y[M,N] = x[M,K] . W[N,K]^T + bias[N]        (M = B*T or B*U1 rows, K = in features, N = hidden_features)

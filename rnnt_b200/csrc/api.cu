@@ -375,6 +375,39 @@ size_t rnnt_b200_greedy_decode_scratch_bytes(int B, int H, int V, int E) {
   return rb::greedy_decode_scratch_bytes(B, H, V, E);
 }
 
+size_t rnnt_b200_greedy_decode_state_bytes(int B, int H, int V, int E) {
+  if (B <= 0 || H <= 0 || V <= 1 || E <= 0) return 0;
+  return rb::greedy_decode_scratch_bytes(B, H, V, E);
+}
+
+namespace {
+
+// Arguments of the decode entries that are checked before anything touches a device.
+int check_decode(int B, int T, int H, int V, int E, int blank, int max_len, int max_per_frame, int64_t enc_sb,
+                 int64_t enc_st, const void* state) {
+  RB_REQUIRE(B > 0 && T >= 0 && H > 0 && V > 1 && E > 0 && max_len >= 1 && max_per_frame >= 0, -1, "invalid shape");
+  RB_REQUIRE(blank >= 0 && blank < V, -4, "blank index out of range");
+  RB_REQUIRE(H % 4 == 0 && E % 4 == 0 && enc_st % 4 == 0 && enc_sb % 4 == 0, -2,
+             "decode kernel needs hidden / embedding sizes and strides that are multiples of 4");
+  RB_REQUIRE(state != nullptr && (reinterpret_cast<uintptr_t>(state) & 127) == 0, -3,
+             "decode scratch must be 128-byte aligned");
+  return 0;
+}
+
+rb::DecodeArgs decode_args(const float* joint_w, const float* joint_b, const float* emb, const float* ln1_w,
+                           const float* ln1_b, const float* conv1_w, const float* conv1_b, const float* conv2_w,
+                           const float* conv2_b, const float* lin_w, const float* lin_b, const float* ln2_w,
+                           const float* ln2_b, int B, int H, int V, int E) {
+  rb::DecodeArgs a{};
+  a.Wj = joint_w; a.bj = joint_b; a.emb = emb; a.ln1_w = ln1_w; a.ln1_b = ln1_b;
+  a.w1 = conv1_w; a.b1 = conv1_b; a.w2 = conv2_w; a.b2 = conv2_b; a.wl = lin_w; a.bl = lin_b;
+  a.ln2_w = ln2_w; a.ln2_b = ln2_b;
+  a.B = B; a.H = H; a.V = V; a.E = E; a.NS = V;
+  return a;
+}
+
+}  // namespace
+
 int rnnt_b200_greedy_decode(const float* enc, int64_t enc_sb, int64_t enc_st, const int32_t* T_len,
                             const float* joint_w, const float* joint_b, const float* emb, const float* ln1_w,
                             const float* ln1_b, const float* conv1_w, const float* conv1_b, const float* conv2_w,
@@ -382,19 +415,50 @@ int rnnt_b200_greedy_decode(const float* enc, int64_t enc_sb, int64_t enc_st, co
                             const float* ln2_b, int B, int T, int H, int V, int E, int blank, int max_len,
                             int max_per_frame, int32_t* tokens, int32_t* n_tokens, float* margins_out, void* scratch,
                             void* stream) {
-  RB_REQUIRE(B > 0 && T > 0 && H > 0 && V > 1 && E > 0 && max_len >= 1 && max_per_frame >= 0, -1, "invalid shape");
-  RB_REQUIRE(blank >= 0 && blank < V, -4, "blank index out of range");
-  RB_REQUIRE(H % 4 == 0 && E % 4 == 0 && enc_st % 4 == 0 && enc_sb % 4 == 0, -2,
-             "decode kernel needs hidden / embedding sizes and strides that are multiples of 4");
-  rb::DecodeArgs a{};
-  a.enc = enc; a.enc_sb = enc_sb; a.enc_st = enc_st; a.T_len = T_len;
-  a.Wj = joint_w; a.bj = joint_b; a.emb = emb; a.ln1_w = ln1_w; a.ln1_b = ln1_b;
-  a.w1 = conv1_w; a.b1 = conv1_b; a.w2 = conv2_w; a.b2 = conv2_b; a.wl = lin_w; a.bl = lin_b;
-  a.ln2_w = ln2_w; a.ln2_b = ln2_b;
-  a.B = B; a.T = T; a.H = H; a.V = V; a.E = E; a.NS = V; a.blank = blank; a.max_len = max_len;
-  a.max_per_frame = max_per_frame; a.max_steps = T + max_len + 1;
-  a.tokens = tokens; a.ntok = n_tokens; a.margins = margins_out;
+  RB_REQUIRE(T > 0, -1, "invalid shape");
+  if (int rc = check_decode(B, T, H, V, E, blank, max_len, max_per_frame, enc_sb, enc_st, scratch)) return rc;
+  // one launch: build the tables, reset every slot, consume the whole utterance
+  rb::DecodeArgs a = decode_args(joint_w, joint_b, emb, ln1_w, ln1_b, conv1_w, conv1_b, conv2_w, conv2_b, lin_w, lin_b,
+                                 ln2_w, ln2_b, B, H, V, E);
+  a.enc = enc; a.enc_sb = enc_sb; a.enc_st = enc_st; a.T_len = T_len; a.T = T;
+  a.init = 1; a.reset_all = 1; a.reset = nullptr;
+  a.blank = blank; a.max_len = max_len; a.max_per_frame = max_per_frame; a.max_steps = T + max_len + 1;
+  a.tokens = tokens; a.n_tokens = n_tokens; a.margins = margins_out;
   return rb::launch_greedy_decode(a, static_cast<float*>(scratch), static_cast<cudaStream_t>(stream));
+}
+
+int rnnt_b200_greedy_decode_stream_init(const float* joint_w, const float* joint_b, const float* emb,
+                                        const float* ln1_w, const float* ln1_b, const float* conv1_w,
+                                        const float* conv1_b, const float* conv2_w, const float* conv2_b,
+                                        const float* lin_w, const float* lin_b, const float* ln2_w, const float* ln2_b,
+                                        int B, int H, int V, int E, void* state, void* stream) {
+  if (int rc = check_decode(B, 0, H, V, E, 0, 1, 0, 0, 0, state)) return rc;
+  rb::DecodeArgs a = decode_args(joint_w, joint_b, emb, ln1_w, ln1_b, conv1_w, conv1_b, conv2_w, conv2_b, lin_w, lin_b,
+                                 ln2_w, ln2_b, B, H, V, E);
+  a.init = 1; a.reset_all = 0; a.reset = nullptr;
+  a.T = 0; a.max_len = 1; a.max_per_frame = 0; a.max_steps = 0;      // no slot is live: the step loop exits at once
+  return rb::launch_greedy_decode(a, static_cast<float*>(state), static_cast<cudaStream_t>(stream));
+}
+
+int rnnt_b200_greedy_decode_stream(const float* enc, int64_t enc_sb, int64_t enc_st, const int32_t* chunk_len,
+                                   const int32_t* reset, const float* joint_w, const float* joint_b, const float* emb,
+                                   const float* ln1_w, const float* ln1_b, const float* conv1_w, const float* conv1_b,
+                                   const float* conv2_w, const float* conv2_b, const float* lin_w, const float* lin_b,
+                                   const float* ln2_w, const float* ln2_b, int B, int Tc, int H, int V, int E,
+                                   int blank, int max_len, int max_per_frame, int32_t* tokens, int32_t* n_tokens,
+                                   float* margins_out, void* state, void* stream) {
+  if (int rc = check_decode(B, Tc, H, V, E, blank, max_len, max_per_frame, enc_sb, enc_st, state)) return rc;
+  RB_REQUIRE(chunk_len != nullptr && tokens != nullptr && n_tokens != nullptr, -1,
+             "decode stream: chunk_len, tokens and n_tokens are required");
+  rb::DecodeArgs a = decode_args(joint_w, joint_b, emb, ln1_w, ln1_b, conv1_w, conv1_b, conv2_w, conv2_b, lin_w, lin_b,
+                                 ln2_w, ln2_b, B, H, V, E);
+  a.enc = enc; a.enc_sb = enc_sb; a.enc_st = enc_st; a.T_len = chunk_len; a.T = Tc;
+  a.init = 0; a.reset_all = 0; a.reset = reset;
+  a.blank = blank; a.max_len = max_len; a.max_per_frame = max_per_frame;
+  // steps of one launch: every step of a slot either consumes a frame or emits a token
+  a.max_steps = static_cast<int>(Tc + std::min<int64_t>(static_cast<int64_t>(Tc) * max_per_frame, max_len - 1) + 1);
+  a.tokens = tokens; a.n_tokens = n_tokens; a.margins = margins_out;
+  return rb::launch_greedy_decode(a, static_cast<float*>(state), static_cast<cudaStream_t>(stream));
 }
 
 size_t rnnt_b200_linear_workspace_bytes(int64_t M, int K, int N, int backward, int flags) {

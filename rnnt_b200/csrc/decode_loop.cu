@@ -20,6 +20,11 @@
 //   P5  z = gelu(conv2) from the tap products of the new conv1 output   P6  lin = linear(z)
 // P5-P6 only run in steps where some utterance emitted.  Every dot product is accumulated in a fixed order (thread-
 // strided partial sums, then one fixed warp butterfly), so results are deterministic.
+//
+// Streaming: the per-slot loop state (predictor accumulators, lin / feats, token count, emit flag) and the symbol tables
+// live in a caller-owned state buffer, so one launch can continue every slot where the previous one stopped.  A launch
+// optionally builds the tables (init), seeds the slots being reset and consumes each slot's frames of this chunk.  The
+// one-shot decode is the launch that does all three for every slot; there is one step loop for both.
 #include <cooperative_groups.h>
 
 #include <algorithm>
@@ -404,28 +409,56 @@ __global__ void __launch_bounds__(kThreads, 1) greedy_decode_kernel(DecodeArgs p
     stage(wl_s, l_hi - l_lo, E, p.resident & 8, off_l);
   }
 
-  // ---- init: conv tap accumulators = 0 (left zero padding), LayerNorm(embedding) table for every symbol, seed token =
-  // blank for every utterance, everyone "emits" the seed so the predictor runs once
-  for (int i = cta * kThreads + tid; i < B * 3 * E; i += G * kThreads) p.acc1[i] = 0.f;
-  for (int i = cta * kThreads + tid; i < B * 5 * E; i += G * kThreads) p.acc2[i] = 0.f;
-  if (cta == 0) {
-    for (int b = tid; b < B; b += kThreads) {
-      p.t_idx[b] = 0; p.per[b] = 0; p.ntok[b] = 1; p.emit[b] = 1; rows_emit[b] = b; p.last_tok[b] = p.blank;
+  // A slot joins a step while it is live (ntok >= 1), not finished and has frames of this launch left.  Between launches
+  // a slot's state sits on a frame boundary: a frame is only left after a blank or the per-frame cap (per = 0), and a
+  // slot that finishes mid-frame stays finished until it is reset.  So t_idx and per restart at 0 every launch.
+  auto is_reset = [&](int b) { return p.reset_all || (p.reset != nullptr && __ldg(p.reset + b) != 0); };
+  auto is_active = [&](int b) {
+    const int nt = __ldcg(p.ntok + b);
+    return nt >= 1 && nt < p.max_len && __ldcg(p.t_idx + b) < min(__ldg(p.T_len + b), p.T);
+  };
+
+  // ---- per launch: frame counters = 0; reset slots get zero conv tap accumulators (the left zero padding), ntok = 1 and
+  // "emit" the seed blank so the predictor runs once; init empties the other slots
+  if (cta == 0 && tid < 32) {
+    int n = 0;
+    for (int b0 = 0; b0 < B; b0 += 32) {
+      const int b = b0 + tid;
+      const bool r = b < B && is_reset(b);
+      if (b < B) {
+        p.t_idx[b] = 0; p.per[b] = 0;
+        if (r) { p.ntok[b] = 1; p.emit[b] = 1; p.last_tok[b] = p.blank; }
+        else if (p.init) { p.ntok[b] = 0; p.emit[b] = 0; }
+      }
+      const unsigned m = __ballot_sync(0xffffffffu, r);
+      if (r) rows_emit[n + __popc(m & ((1u << tid) - 1))] = b;
+      n += __popc(m);
     }
-    if (tid == 0) { counts[0] = 0; counts[1] = B; counts[2] = 0; }
+    if (tid == 0) { counts[0] = 0; counts[1] = n; counts[2] = 0; }
   }
-  for (int v = cta; v < p.NS; v += G)
-    block_layer_norm(p.emb + static_cast<long long>(v) * E, p.ln1_w, p.ln1_b, p.emb_ln + static_cast<long long>(v) * E, E, red);
-  grid_barrier(bar_counter, bar_target);
-  // ---- conv1 tap table: t1[v][j][o] = W1_j[o, :] . LN(emb[v]) for every symbol v (this CTA's output channels)
-  {
-    GemvEpi epi{2, 3, nullptr, nullptr, E};
-    gemv_phase<false>(w1_s, nullptr, e_lo, e_hi, E, 3 * E, p.emb_ln, E, nullptr, p.NS, p.t1, 3 * E, epi, xstage);
+  for (int b = cta; b < B; b += G) {
+    if (!is_reset(b)) continue;
+    for (int i = tid; i < 3 * E; i += kThreads) p.acc1[static_cast<long long>(b) * 3 * E + i] = 0.f;
+    for (int i = tid; i < 5 * E; i += kThreads) p.acc2[static_cast<long long>(b) * 5 * E + i] = 0.f;
   }
-  lap(3);
-  grid_barrier(bar_counter, bar_target);
-  // ---- the seed blank at position 0 of every utterance
-  for (int b = cta; b < B; b += G) conv1_update(p, b, p.blank, 0);
+  if (p.init) {
+    // ---- LayerNorm(embedding) table for every symbol
+    for (int v = cta; v < p.NS; v += G)
+      block_layer_norm(p.emb + static_cast<long long>(v) * E, p.ln1_w, p.ln1_b, p.emb_ln + static_cast<long long>(v) * E, E, red);
+    grid_barrier(bar_counter, bar_target);
+    // ---- conv1 tap table: t1[v][j][o] = W1_j[o, :] . LN(emb[v]) for every symbol v (this CTA's output channels)
+    {
+      GemvEpi epi{2, 3, nullptr, nullptr, E};
+      gemv_phase<false>(w1_s, nullptr, e_lo, e_hi, E, 3 * E, p.emb_ln, E, nullptr, p.NS, p.t1, 3 * E, epi, xstage);
+    }
+    lap(3);
+    grid_barrier(bar_counter, bar_target);
+  } else {
+    __syncthreads();            // this CTA's zeroed accumulators before its own seed updates
+  }
+  // ---- the seed blank at position 0 of every reset slot
+  for (int b = cta; b < B; b += G)
+    if (is_reset(b)) conv1_update(p, b, p.blank, 0);
   grid_barrier(bar_counter, bar_target);
   lap(7);
 
@@ -455,9 +488,8 @@ __global__ void __launch_bounds__(kThreads, 1) greedy_decode_kernel(DecodeArgs p
     for (int b = cta; b < B; b += G) {
       if (__ldcg(p.emit + b)) block_layer_norm(p.lin + static_cast<long long>(b) * H, p.ln2_w, p.ln2_b, p.feats + static_cast<long long>(b) * H, H, red);
       __syncthreads();
-      const int t = __ldcg(p.t_idx + b);
-      const bool active = t < p.T_len[b] && __ldcg(p.ntok + b) < p.max_len;
-      if (active) {
+      if (is_active(b)) {
+        const int t = __ldcg(p.t_idx + b);
         const float* e = p.enc + b * p.enc_sb + static_cast<long long>(t) * p.enc_st;
         for (int i = tid; i < H; i += kThreads) p.hbuf[static_cast<long long>(b) * H + i] = tanhf(__ldg(e + i) + p.feats[static_cast<long long>(b) * H + i]);
       }
@@ -468,7 +500,7 @@ __global__ void __launch_bounds__(kThreads, 1) greedy_decode_kernel(DecodeArgs p
         int n = 0;
         for (int b0 = 0; b0 < B; b0 += 32) {
           const int b = b0 + tid;
-          const bool a = b < B && __ldcg(p.t_idx + b) < p.T_len[b] && __ldcg(p.ntok + b) < p.max_len;
+          const bool a = b < B && is_active(b);
           const unsigned m = __ballot_sync(0xffffffffu, a);
           if (a) rows_act[n + __popc(m & ((1u << tid) - 1))] = b;
           n += __popc(m);
@@ -528,12 +560,16 @@ __global__ void __launch_bounds__(kThreads, 1) greedy_decode_kernel(DecodeArgs p
     grid_barrier(bar_counter, bar_target);
     lap(7);
   }
+  // every exit of the loop follows a grid barrier, so all ntok updates are visible here
+  if (cta == 0 && p.n_tokens != nullptr)
+    for (int b = tid; b < B; b += kThreads) p.n_tokens[b] = __ldcg(p.ntok + b);
 }
 
 }  // namespace
 
-// Scratch layout: [8 x int64 phase timers | float regions, each padded to a multiple of 4 floats so that every region
-// starts 16-byte aligned whatever B, V, E are (cp.async / float4 need it) | int regions].
+// State / scratch layout: [8 x int64 phase timers | barrier line | float regions, each padded to a multiple of 4 floats
+// so that every region starts 16-byte aligned whatever B, V, E are (cp.async / float4 need it) | int regions].  The
+// one-shot decode and the streaming decoder share it (include/rnnt_b200.h lists what persists between launches).
 namespace {
 inline size_t pad4(size_t n) { return (n + 3) & ~static_cast<size_t>(3); }
 constexpr size_t kTimerBytes = 128;
@@ -545,7 +581,7 @@ size_t greedy_decode_scratch_bytes(int B, int H, int V, int E) {
   const size_t floats = 3 * pad4(b * H) /*feats, hbuf, lin*/ + pad4(b * V) /*logits*/ + pad4(b * 3 * E) + pad4(b * 5 * E) +
                         2 * pad4(b * E) /*ynew, z*/ + pad4(static_cast<size_t>(V) * E) /*LayerNorm(embedding) table*/ +
                         pad4(static_cast<size_t>(V) * 3 * E) /*conv1 tap table*/;
-  const size_t ints = b * 6 + 16;
+  const size_t ints = b * 7 + 16;
   return kTimerBytes + kBarBytes + floats * 4 + ints * 4 + 256;
 }
 
@@ -588,6 +624,7 @@ int launch_greedy_decode(DecodeArgs a, float* scratch, cudaStream_t stream) {
   a.emb_ln = f; f += pad4(static_cast<size_t>(a.NS) * E);
   a.t1 = f; f += pad4(static_cast<size_t>(a.NS) * 3 * E);
   int* ip = reinterpret_cast<int*>(f);
+  a.ntok = ip; ip += B;
   a.t_idx = ip; ip += B;
   a.per = ip; ip += B;
   a.emit = ip; ip += B;

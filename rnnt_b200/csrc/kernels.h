@@ -77,10 +77,19 @@ struct DwArgs {
   int ksplit;
 };
 
+// One launch of the persistent greedy decode.  The per-slot decoder state lives in the caller's state buffer (carved by
+// the launcher), so a launch continues every live slot where the previous launch on the same buffer stopped:
+//   init     build the two per-symbol tables and mark every slot empty (n_tokens 0)
+//   reset    slots that start a new utterance before this launch's frames: predictor state zeroed, seed blank run
+//   T_len    frames each slot consumes in this launch, clamped to [0, T]
+// The one-shot decode is init + every slot reset + T_len = the utterance lengths.
 struct DecodeArgs {
   const float* enc;        // (B,T,H) fp32, H contiguous
   long long enc_sb, enc_st;
-  const int* T_len;        // (B) frames per utterance
+  const int* T_len;        // (B) frames per slot in this launch (may be null when no slot is live)
+  int init;                // 1: build the symbol tables and empty every slot first
+  int reset_all;           // 1: every slot is reset (else the slots with reset[b] != 0)
+  const int* reset;        // (B) or null
   const float* Wj; const float* bj;                       // joint_ln (V,H), (V)
   const float* emb; const float* ln1_w; const float* ln1_b;   // embedding (NS,E), input LayerNorm (E)
   const float* w1; const float* b1;                       // conv1 as (E, 3E): taps oldest..newest
@@ -91,9 +100,12 @@ struct DecodeArgs {
   int weight_floats;       // floats of dynamic shared memory taken by the resident weight slices (staging follows)
   int resident;            // bit i: weight matrix i (joint, conv2, conv1, linear) has its per-CTA slice in shared memory
   int* tokens;             // (B, max_len) emitted tokens (seed blank excluded)
-  int* ntok;               // (B) 1 + number of emitted tokens
-  // scratch (carved by the launcher)
-  float *feats, *hbuf, *logits, *acc1, *acc2, *ynew, *z, *lin, *emb_ln, *t1 /* conv1 tap table (NS, 3E) */, *margins;
+  int* n_tokens;           // (B) output copy of ntok at the end of the launch (may be null)
+  float* margins;          // (max_steps, B) top-2 logit gap per step (may be null)
+  // state (carved by the launcher): kept across launches -- feats, lin, acc1, acc2, emb_ln, t1, ntok, emit, last_tok;
+  // per-launch scratch -- hbuf, logits, ynew, z, t_idx, per, rows, flags
+  float *feats, *hbuf, *logits, *acc1, *acc2, *ynew, *z, *lin, *emb_ln, *t1 /* conv1 tap table (NS, 3E) */;
+  int* ntok;               // (B) 0 = empty slot, else 1 + number of emitted tokens (the predictor's next position)
   int *t_idx, *per, *emit, *rows, *last_tok, *flags;
   unsigned* bar;           // grid-barrier counters (one per 128-byte line)
   int NS;                  // number of symbols = rows of the embedding table

@@ -423,6 +423,25 @@ def joint_argmax(audio_rows, text_rows, weight, bias, return_margin: bool = Fals
     return (tokens, margin) if return_margin else tokens
 
 
+def _check_decode_sizes(predictor, joint_weight, H):
+    if predictor.linear.out_features != H or joint_weight.shape[1] != H:
+        raise RuntimeError("predictor output, encoder features and joint hidden size must agree")
+    if predictor.conv1.conv.kernel_size[0] != 3 or predictor.conv2.conv.kernel_size[0] != 5:
+        raise RuntimeError("decode kernel expects ConvPredictor's kernel sizes 3 and 5")
+
+
+def _decode_params(joint_weight, joint_bias, p, dev):
+    """The 13 weight tensors of the decode entries, fp32 contiguous on `dev`, conv weights re-laid as (E, k*E) with
+    taps ordered oldest..newest."""
+    E = p.embedding.embedding_dim
+    f = lambda t: t.detach().to(dev, torch.float32).contiguous()
+    w1 = f(p.conv1.conv.weight.detach().permute(0, 2, 1).reshape(E, -1))
+    w2 = f(p.conv2.conv.weight.detach().permute(0, 2, 1).reshape(E, -1))
+    return [f(joint_weight), f(joint_bias), f(p.embedding.weight), f(p.input_layer_norm.weight),
+            f(p.input_layer_norm.bias), w1, f(p.conv1.conv.bias), w2, f(p.conv2.conv.bias), f(p.linear.weight),
+            f(p.linear.bias), f(p.output_layer_norm.weight), f(p.output_layer_norm.bias)]
+
+
 def greedy_decode(audio_features, audio_feature_lens, joint_weight, joint_bias, predictor, blank: int,
                   max_length: int = 200, max_outputs_per_step: int = 10, return_margins: bool = False):
     """Batched greedy decode (rnnt/model.py:90-128 for every utterance of a batch) in ONE persistent CUDA kernel.
@@ -435,19 +454,10 @@ def greedy_decode(audio_features, audio_feature_lens, joint_weight, joint_bias, 
     dev = audio_features.device
     B, T, H = audio_features.shape
     V = joint_weight.shape[0]
-    p = predictor
-    E = p.embedding.embedding_dim
-    if p.linear.out_features != H or joint_weight.shape[1] != H:
-        raise RuntimeError("predictor output, encoder features and joint hidden size must agree")
-    if p.conv1.conv.kernel_size[0] != 3 or p.conv2.conv.kernel_size[0] != 5:
-        raise RuntimeError("decode kernel expects ConvPredictor's kernel sizes 3 and 5")
-    f = lambda t: t.detach().to(dev, torch.float32).contiguous()
-    enc = f(audio_features)
-    w1 = f(p.conv1.conv.weight.detach().permute(0, 2, 1).reshape(E, -1))
-    w2 = f(p.conv2.conv.weight.detach().permute(0, 2, 1).reshape(E, -1))
-    params = [f(joint_weight), f(joint_bias), f(p.embedding.weight), f(p.input_layer_norm.weight),
-              f(p.input_layer_norm.bias), w1, f(p.conv1.conv.bias), w2, f(p.conv2.conv.bias), f(p.linear.weight),
-              f(p.linear.bias), f(p.output_layer_norm.weight), f(p.output_layer_norm.bias)]
+    _check_decode_sizes(predictor, joint_weight, H)
+    E = predictor.embedding.embedding_dim
+    enc = audio_features.detach().to(dev, torch.float32).contiguous()
+    params = _decode_params(joint_weight, joint_bias, predictor, dev)
     lens = audio_feature_lens.to(dev, torch.int32).clamp(max=T).contiguous()
     max_len = max(int(max_length), 1)
     tokens = torch.zeros(B, max_len, dtype=torch.int32, device=dev)
@@ -468,3 +478,120 @@ def greedy_decode(audio_features, audio_feature_lens, joint_weight, joint_bias, 
         ml = margins.t().tolist()
         return result, [[x for x in ml[b] if x != float("inf")] for b in range(B)]
     return result
+
+
+class StreamingGreedyDecoder:
+    """Greedy decode of `slots` live streams whose encoder frames arrive chunk by chunk, in the persistent decode kernel
+    (`rnnt_b200_greedy_decode_stream`).  The decoder state of every slot stays on the device between calls.
+
+    `reset(slots)` makes slots start a new utterance at the next `decode_chunk`; every other live slot continues where
+    its previous call stopped.  However an utterance's frames are split into chunks, its tokens (and per-step margins)
+    are bit-identical to `greedy_decode` on the whole utterance with the same max_length / max_outputs_per_step.  The
+    weights are re-laid for the kernel once and the per-symbol tables are built from them: call `refresh()` after the
+    weights change (it empties every slot)."""
+
+    def __init__(self, joint, predictor, slots: int, max_length: int = 200, max_outputs_per_step: int = 10):
+        from .model import _is_conv_predictor, _is_lstm_predictor
+        if _is_lstm_predictor(predictor):
+            raise ValueError("streaming decode needs a ConvPredictor; decode an LSTM predictor with "
+                             "RNNTModel.greedy_decode_features")
+        if not _is_conv_predictor(predictor):
+            raise ValueError("Unknown predictor type")
+        if hasattr(joint, "audio_ln") or hasattr(joint, "text_ln"):
+            raise ValueError("streaming decode does not support a joint with audio_ln / text_ln pre-projections")
+        if int(slots) < 1:
+            raise ValueError("slots must be >= 1")
+        weight = joint.joint_ln.weight
+        _check_decode_sizes(predictor, weight, weight.shape[1])
+        _require_cuda(weight)
+        self.joint, self.predictor = joint, predictor
+        self.slots = int(slots)
+        self.max_length = max(int(max_length), 1)
+        self.max_outputs_per_step = int(max_outputs_per_step)
+        self.blank = int(joint.blank_idx)
+        self.dev = weight.device
+        self.V, self.H = weight.shape
+        self.E = predictor.embedding.embedding_dim
+        L = _lib.lib()
+        S = self.slots
+        i32 = dict(dtype=torch.int32, device=self.dev)
+        self.state = torch.empty(L.rnnt_b200_greedy_decode_state_bytes(S, self.H, self.V, self.E), dtype=torch.uint8,
+                                 device=self.dev)
+        self.tokens = torch.zeros(S, self.max_length, **i32)     # column k-1 = k-th token of the slot's utterance
+        self.n_tokens = torch.zeros(S, **i32)                    # 0 = empty slot, else 1 + tokens (seed blank counted)
+        self._reset_mask = torch.zeros(S, **i32)
+        self._pending = set()                                    # host copy of the reset mask
+        self._n_host = [0] * S                                   # host copy of n_tokens
+        self.refresh()
+
+    def refresh(self) -> None:
+        """Re-read the joint and predictor weights and rebuild the per-symbol tables.  Empties every slot (resets
+        already requested stay pending)."""
+        self._params = _decode_params(self.joint.joint_ln.weight, self.joint.joint_ln.bias, self.predictor, self.dev)
+        with torch.cuda.device(self.dev):
+            _lib.check(_lib.lib().rnnt_b200_greedy_decode_stream_init(
+                *[t.data_ptr() for t in self._params], self.slots, self.H, self.V, self.E, self.state.data_ptr(),
+                _stream_ptr(self.dev)), "greedy_decode_stream_init")
+        self.n_tokens.zero_()
+        self._n_host = [0] * self.slots
+
+    def reset(self, slots) -> None:
+        """Start a new utterance in each of `slots` (an int or an iterable of ints) at the next decode_chunk."""
+        idx = [int(slots)] if isinstance(slots, int) else [int(s) for s in slots]
+        if any(s < 0 or s >= self.slots for s in idx):
+            raise IndexError(f"slot index out of range [0, {self.slots})")
+        if idx:
+            self._reset_mask[torch.tensor(idx, device=self.dev)] = 1
+            self._pending.update(idx)
+
+    @property
+    def finished(self) -> torch.Tensor:
+        """(slots,) bool: the slot's utterance reached max_length tokens (seed blank counted) and ignores frames."""
+        return self.n_tokens >= self.max_length
+
+    def transcript(self, slot: int) -> list:
+        """Every token the slot's current utterance has emitted so far."""
+        return self.tokens[slot, : max(self._n_host[slot] - 1, 0)].tolist()
+
+    def decode_chunk(self, features, lens=None, return_margins: bool = False):
+        """Feed the next chunk of encoder frames: features (slots, Tc, H) (any strides, e.g. the permuted view of the
+        encoder's (slots, H, Tc) output), lens (slots,) = frames of the chunk each slot takes (default Tc, clamped to
+        [0, Tc]).  Returns the tokens this call added per slot (and, optionally, the top-2 logit margins of every step
+        the slot took in this call).  Synchronises once, to return the tokens."""
+        _require_cuda(features)
+        S, H = self.slots, self.H
+        if features.dim() != 3 or features.shape[0] != S or features.shape[2] != H:
+            raise RuntimeError(f"expected features (slots={S}, Tc, H={H}), got {tuple(features.shape)}")
+        Tc = features.shape[1]
+        enc = features.detach().to(self.dev, torch.float32).contiguous()
+        if lens is None:
+            chunk = torch.full((S,), Tc, dtype=torch.int32, device=self.dev)
+        else:
+            chunk = torch.as_tensor(lens).to(self.dev, torch.int32).clamp(0, Tc).contiguous()
+            if chunk.shape != (S,):
+                raise RuntimeError(f"expected lens of shape ({S},), got {tuple(chunk.shape)}")
+        most = min(Tc * self.max_outputs_per_step, self.max_length - 1)     # tokens one call can add to a slot
+        margins = (torch.full((Tc + most + 1, S), float("inf"), device=self.dev) if return_margins else None)
+        start = [0 if b in self._pending else max(n - 1, 0) for b, n in enumerate(self._n_host)]
+        L = _lib.lib()
+        with torch.cuda.device(self.dev):
+            _lib.check(L.rnnt_b200_greedy_decode_stream(
+                enc.data_ptr(), enc.stride(0), enc.stride(1), chunk.data_ptr(), self._reset_mask.data_ptr(),
+                *[t.data_ptr() for t in self._params], S, Tc, H, self.V, self.E, self.blank, self.max_length,
+                self.max_outputs_per_step, self.tokens.data_ptr(), self.n_tokens.data_ptr(),
+                margins.data_ptr() if return_margins else None, self.state.data_ptr(), _stream_ptr(self.dev)),
+                "greedy_decode_stream")
+            self._reset_mask.zero_()
+            self._pending.clear()
+            # the columns this call can have written, gathered on the device: one copy to the host
+            cols = (torch.tensor(start, dtype=torch.int64, device=self.dev).view(S, 1)
+                    + torch.arange(most, device=self.dev)).clamp(max=self.max_length - 1)
+            rows = torch.cat([self.n_tokens.view(S, 1), self.tokens.gather(1, cols)], 1).tolist()
+        global _last_decode_phase_cycles
+        _last_decode_phase_cycles = self.state[:64].view(torch.int64)
+        self._n_host = [r[0] for r in rows]
+        new = [rows[b][1: 1 + max(rows[b][0] - 1, 0) - start[b]] for b in range(S)]
+        if return_margins:
+            ml = margins.t().tolist()
+            return new, [[x for x in ml[b] if x != float("inf")] for b in range(S)]
+        return new

@@ -88,6 +88,12 @@ class RNNTModel(torch.nn.Module):
         finally:
             self.predictor.train(was_training)
 
+    def streaming_decoder(self, slots: int, max_length: int = 200, max_outputs_per_step: int = 10):
+        """A `StreamingGreedyDecoder` over this model's joint and (ConvPredictor-shaped) predictor with `slots` streams:
+        feed it the encoder's output chunk by chunk (e.g. from `AudioEncoder.streaming_forward`)."""
+        from .functional import StreamingGreedyDecoder
+        return StreamingGreedyDecoder(self.joint, self.predictor, slots, max_length, max_outputs_per_step)
+
     @torch.no_grad()
     def _greedy_decode_features_hostloop(self, audio_features, audio_feature_lens, max_length: int = 200,
                                          max_outputs_per_step: int = 10):
