@@ -15,18 +15,15 @@ using rb::kTileM;
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
-// Diagnostic knobs (read once per process; none of them changes results except RNNT_B200_DBG / RNNT_B200_NO_DB, which
-// exist to measure what parts of a kernel cost):
+// Diagnostic knobs (read once per process), which exist to measure what parts of a kernel cost:
 //   RNNT_B200_DBG      bit mask handed to the joint kernels (1 skip epilogue math, 2 skip producer math, 8 print grids, ...)
 //   RNNT_B200_NO_DB    leave db out of the dW kernel (db is then NOT computed)
-//   RNNT_B200_COMM_SMS SMs the last dh launch leaves idle when the caller passed a dw_done event (for a concurrent collective)
-struct EnvKnobs { int dbg; bool no_db; int comm_sms; };
+struct EnvKnobs { int dbg; bool no_db; };
 const EnvKnobs& env_knobs() {
   static const EnvKnobs k = [] {
     EnvKnobs e{};
     const char* s = getenv("RNNT_B200_DBG");      e.dbg = s ? atoi(s) : 0;
     e.no_db = getenv("RNNT_B200_NO_DB") != nullptr;
-    s = getenv("RNNT_B200_COMM_SMS");             e.comm_sms = s ? atoi(s) : 0;
     return e;
   }();
   return k;
@@ -34,7 +31,8 @@ const EnvKnobs& env_knobs() {
 inline int round_up(int x, int a) { return (x + a - 1) / a * a; }
 
 struct WsLayout {
-  size_t tile_off, wb, bias2, h_scratch, coef, flags, tile_list, g_ring, h_ring, fx, total_fwd, total_bwd;
+  size_t tile_off, status, gscale, n_active, wb, bias2, h_scratch, coef, flags, tile_list, g_ring, h_ring, fx, total_fwd,
+      total_bwd;
   int Hp, Vp, scratch_tiles;
 };
 
@@ -45,7 +43,12 @@ WsLayout ws_layout(int B, int T, int U1, int H, int V, int64_t ring_tiles, bool 
   w.Hp = round_up(H, 64);
   w.Vp = round_up(V, 256);
   size_t off = 0;
-  w.tile_off = off; off = align_up(off + (static_cast<size_t>(B) + 6) * sizeof(int), 1024);   // + status, {S, 1/S}, n_active
+  // tile-table region (documented in rnnt_b200.h): B+1 prefix sums, then status, {S, 1/S}, n_active and one spare word
+  w.tile_off = off;
+  w.status = w.tile_off + (static_cast<size_t>(B) + 1) * sizeof(int);
+  w.gscale = w.status + sizeof(int);
+  w.n_active = w.gscale + 2 * sizeof(float);
+  off = align_up(w.n_active + 2 * sizeof(int), 1024);
   w.wb = off;       off = align_up(off + static_cast<size_t>(w.Vp) * w.Hp * 2, 1024);
   w.bias2 = off;    off = align_up(off + static_cast<size_t>(w.Vp) * 4, 1024);
   const size_t common = off;
@@ -98,6 +101,115 @@ int check_common(const void* enc, int64_t& enc_sb, int64_t& enc_st, int64_t& enc
   return 0;
 }
 
+// What the backward passes to the prologue beyond the forward's arguments (check_layout normalises the d_enc strides in
+// place, as it does the encoder's).
+struct BwdArgs {
+  const float* d_enc;
+  int64_t &denc_sb, &denc_st, &denc_sh;
+  int64_t ring_tiles;
+  bool deterministic;
+  const float* dcost;
+};
+
+// One call of a fused-loss entry as its prologue leaves it: the workspace (offsets: ws_layout) carved into typed
+// pointers, the tensor map over the fp16 W, and the batch fields of the kernel arguments.
+struct LossCall {
+  WsLayout w;
+  int* tile_off;          // [B+1] prefix sums of half-tiles per utterance
+  int* status;            // non-zero when a length is out of range
+  float* gscale;          // backward: {S, 1/S}
+  int* n_active;          // backward: number of active half-tiles in sub_list
+  __half* Wb;             // W as fp16 [Vp, Hp], zero-padded
+  float* bias2;           // [Vp]
+  __half* h_scratch;      // forward without a residual buffer: per-CTA activation rows
+  float4* coef;           // backward (the regions from here on reuse the forward's h_scratch): (B,T,U1) coefficients
+  unsigned char* flags;   // one per half-tile: active in the backward
+  int* sub_list;          // work list of active half-tiles, order preserved
+  __half* g_ring;         // logit gradients of one chunk of the work list
+  __half* h_ring;         // activations of that chunk, recomputed when the caller keeps no residual buffer
+  long long *fx_enc, *fx_pred, *fx_w, *fx_b;   // deterministic mode: fixed-point shadows of d_enc, d_pred, dW, db
+  CUtensorMap tmW;        // fp16 W, 64(k) x 128(v) boxes
+  rb::BatchArgs base;
+};
+
+// The part both fused-loss entries share (bwd == nullptr for the forward): check every argument before anything touches
+// a device, carve the workspace, enqueue the tile table and the fp16 copy of W, build the tensor map over that copy,
+// and fill the batch fields of the kernel arguments.
+int loss_prologue(LossCall& c, const float* enc, int64_t enc_sb, int64_t enc_st, int64_t enc_sh, const float* pred,
+                  const float* W, const float* bias, const int32_t* targets, const int32_t* T_len,
+                  const int32_t* U_len, int B, int T, int U1, int H, int V, int blank, const void* hidden,
+                  BwdArgs* bwd, int32_t* err_flag, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+  int rc = check_common(enc, enc_sb, enc_st, enc_sh, pred, B, T, U1, H, V, &blank);
+  if (rc) return rc;
+  RB_REQUIRE((reinterpret_cast<uintptr_t>(W) & 15) == 0, -3, "W must be 16-byte aligned");
+  RB_REQUIRE((reinterpret_cast<uintptr_t>(hidden) & 127) == 0, -3, "hidden must be 128-byte aligned");
+  if (bwd) {
+    rc = check_layout("d_enc", bwd->denc_sb, bwd->denc_st, bwd->denc_sh, B, T, H);
+    if (rc) return rc;
+    RB_REQUIRE((reinterpret_cast<uintptr_t>(bwd->d_enc) & 15) == 0, -3, "d_enc must be 16-byte aligned");
+    const int64_t TH = static_cast<int64_t>(T) * H;
+    RB_REQUIRE((bwd->denc_sh == 1 && bwd->denc_st == H && bwd->denc_sb == TH) ||
+                   (bwd->denc_st == 1 && bwd->denc_sh == T && bwd->denc_sb == TH),
+               -3, "d_enc must be a dense (B,T,H) tensor or a dense (B,H,T) tensor viewed as (B,T,H)");
+    RB_REQUIRE(bwd->ring_tiles >= 1 && bwd->ring_tiles * kTileM < (1ll << 30), -8, "ring_tiles out of range");
+  }
+  const bool deterministic = bwd && bwd->deterministic;
+  const WsLayout& w = c.w = ws_layout(B, T, U1, H, V, bwd ? bwd->ring_tiles : 0, hidden != nullptr, deterministic);
+  const size_t need = bwd ? w.total_bwd : w.total_fwd;
+  RB_REQUIRE(workspace != nullptr && workspace_bytes >= need, -7, "workspace too small: need %zu bytes", need);
+  RB_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, -7, "workspace must be 256-byte aligned");
+
+  uint8_t* p = static_cast<uint8_t*>(workspace);
+  c.tile_off = reinterpret_cast<int*>(p + w.tile_off);
+  c.status = reinterpret_cast<int*>(p + w.status);
+  c.gscale = reinterpret_cast<float*>(p + w.gscale);
+  c.n_active = reinterpret_cast<int*>(p + w.n_active);
+  c.Wb = reinterpret_cast<__half*>(p + w.wb);
+  c.bias2 = reinterpret_cast<float*>(p + w.bias2);
+  c.h_scratch = reinterpret_cast<__half*>(p + w.h_scratch);
+  c.coef = reinterpret_cast<float4*>(p + w.coef);
+  c.flags = p + w.flags;
+  c.sub_list = reinterpret_cast<int*>(p + w.tile_list);
+  c.g_ring = reinterpret_cast<__half*>(p + w.g_ring);
+  c.h_ring = reinterpret_cast<__half*>(p + w.h_ring);
+  if (deterministic) {   // d_enc (B,T,H), d_pred (B,U1,H), dW (V,H), db (V)
+    c.fx_enc = reinterpret_cast<long long*>(p + w.fx);
+    c.fx_pred = c.fx_enc + static_cast<size_t>(B) * T * H;
+    c.fx_w = c.fx_pred + static_cast<size_t>(B) * U1 * H;
+    c.fx_b = c.fx_w + static_cast<size_t>(V) * H;
+  }
+
+  rc = rb::launch_tile_table(T_len, U_len, B, T, U1, c.tile_off, c.status, err_flag, bwd ? bwd->dcost : nullptr,
+                             bwd ? c.gscale : nullptr, stream);
+  if (rc) return rc;
+  rc = rb::launch_convert_weights(W, bias, V, H, w.Vp, w.Hp, c.Wb, c.bias2, stream);
+  if (rc) return rc;
+  rc = rb::make_tmap_2d(&c.tmW, c.Wb, 2, w.Hp, w.Vp, static_cast<uint64_t>(w.Hp) * 2, 64, 128);
+  if (rc) return rc;
+
+  rb::BatchArgs& a = c.base;
+  a.enc = enc; a.enc_sb = enc_sb; a.enc_st = enc_st; a.enc_sh = enc_sh;
+  a.pred = pred; a.pred_sb = static_cast<long long>(U1) * H; a.pred_su = H;
+  a.bias2 = c.bias2; a.targets = targets; a.tgt_ld = U1 - 1;
+  a.T_len = T_len; a.U_len = U_len; a.tile_off = c.tile_off;
+  a.B = B; a.T = T; a.U1 = U1; a.H = H; a.Hp = w.Hp; a.V = V; a.Vp = w.Vp; a.blank = blank;
+  // the forward covers every half-tile from slot 0 in one launch; the backward walks its work list a ring at a time
+  a.slot_cap = bwd ? static_cast<int>(2 * bwd->ring_tiles) : 0x3fffffff;
+  a.sub_list = bwd ? c.sub_list : nullptr;
+  a.n_active = bwd ? c.n_active : nullptr;
+  a.gscale = bwd ? c.gscale : nullptr;
+  a.h_map = hidden ? 0 : bwd ? 1 : 2;
+  return 0;
+}
+
+// An fp16 [rows, cols] buffer of activations (cols = Hp) or logit gradients (cols = Vp) in boxes 64 columns wide: 64 rows
+// (one half-tile) and 128 rows (two adjacent ones)
+int make_row_maps(CUtensorMap* m64, CUtensorMap* m128, const __half* buf, uint64_t rows, int cols) {
+  int rc = rb::make_tmap_2d(m64, buf, 2, cols, rows, static_cast<uint64_t>(cols) * 2, 64, 64);
+  if (rc) return rc;
+  return rb::make_tmap_2d(m128, buf, 2, cols, rows, static_cast<uint64_t>(cols) * 2, 64, 128);
+}
+
 }  // namespace
 
 extern "C" {
@@ -146,50 +258,26 @@ int rnnt_b200_joint_loss_fwd(const float* enc, int64_t enc_sb, int64_t enc_st, i
                              float* lp, float* lse, float* alpha, float* beta, void* hidden, int32_t* status,
                              void* workspace, size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  int rc = check_common(enc, enc_sb, enc_st, enc_sh, pred, B, T, U1, H, V, &blank);
-  if (rc) return rc;
-  const WsLayout w = ws_layout(B, T, U1, H, V, 0, hidden != nullptr);
-  RB_REQUIRE((reinterpret_cast<uintptr_t>(W) & 15) == 0, -3, "W must be 16-byte aligned");
-  RB_REQUIRE((reinterpret_cast<uintptr_t>(hidden) & 127) == 0, -3, "hidden must be 128-byte aligned");
-  RB_REQUIRE(workspace != nullptr && workspace_bytes >= w.total_fwd, -7, "workspace too small: need %zu bytes",
-             w.total_fwd);
-  RB_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, -7, "workspace must be 256-byte aligned");
-  uint8_t* ws = static_cast<uint8_t*>(workspace);
-  int* tile_off = reinterpret_cast<int*>(ws + w.tile_off);
-  __half* Wb = reinterpret_cast<__half*>(ws + w.wb);
-  float* bias2 = reinterpret_cast<float*>(ws + w.bias2);
-
-  rc = rb::launch_tile_table(T_len, U_len, B, T, U1, tile_off, status, nullptr, nullptr, stream);
-  if (rc) return rc;
-  rc = rb::launch_convert_weights(W, bias, V, H, w.Vp, w.Hp, Wb, bias2, stream);
+  LossCall c{};
+  int rc = loss_prologue(c, enc, enc_sb, enc_st, enc_sh, pred, W, bias, targets, T_len, U_len, B, T, U1, H, V, blank,
+                         hidden, nullptr, status, workspace, workspace_bytes, stream);
   if (rc) return rc;
 
   const int64_t max_tiles = rnnt_b200_max_tiles(B, T, U1);
   // activation rows h = tanh(enc+pred): the caller's residual buffer (one 64-row block per half-tile) or a
   // small per-CTA scratch when no backward will follow
-  __half* hbuf = hidden ? static_cast<__half*>(hidden) : reinterpret_cast<__half*>(ws + w.h_scratch);
-  const uint64_t hrows = static_cast<uint64_t>(hidden ? max_tiles : w.scratch_tiles) * kTileM;
-  CUtensorMap tmW, tmH, tmH2;
-  rc = rb::make_tmap_2d(&tmW, Wb, 2, w.Hp, w.Vp, static_cast<uint64_t>(w.Hp) * 2, 64, 128);
-  if (rc) return rc;
-  rc = rb::make_tmap_2d(&tmH, hbuf, 2, w.Hp, hrows, static_cast<uint64_t>(w.Hp) * 2, 64, 64);
-  if (rc) return rc;
-  rc = rb::make_tmap_2d(&tmH2, hbuf, 2, w.Hp, hrows, static_cast<uint64_t>(w.Hp) * 2, 64, 128);
+  __half* hbuf = hidden ? static_cast<__half*>(hidden) : c.h_scratch;
+  const uint64_t hrows = static_cast<uint64_t>(hidden ? max_tiles : c.w.scratch_tiles) * kTileM;
+  CUtensorMap tmH, tmH2;
+  rc = make_row_maps(&tmH, &tmH2, hbuf, hrows, c.w.Hp);
   if (rc) return rc;
 
-  rb::JointArgs a{};
-  a.enc = enc; a.enc_sb = enc_sb; a.enc_st = enc_st; a.enc_sh = enc_sh;
-  a.pred = pred; a.pred_sb = static_cast<long long>(U1) * H; a.pred_su = H;
-  a.bias2 = bias2; a.targets = targets; a.tgt_ld = U1 - 1;
-  a.T_len = T_len; a.U_len = U_len; a.tile_off = tile_off;
-  a.B = B; a.T = T; a.U1 = U1; a.H = H; a.Hp = w.Hp; a.V = V; a.Vp = w.Vp; a.blank = blank;
-  a.slot_begin = 0; a.slot_cap = 0x3fffffff; a.sub_list = nullptr; a.n_active = nullptr;
+  rb::JointArgs a{c.base};
+  a.lp = lp; a.lse = lse; a.h_out = hbuf;
   a.dbg = env_knobs().dbg;
-  a.lp = lp; a.lse = lse; a.coef = nullptr; a.dcost = nullptr; a.gscale = nullptr; a.clamp = 0.f;
-  a.h_out = hbuf; a.h_map = hidden ? 0 : 2; a.g_ring = nullptr;
-  rc = rb::launch_joint_gemm(0, true, tmW, tmH, tmH2, a, 2 * max_tiles, stream);
+  rc = rb::launch_joint_gemm(0, true, c.tmW, tmH, tmH2, a, 2 * max_tiles, stream);
   if (rc) return rc;
-  return rb::launch_lattice(lp, T_len, U_len, B, T, U1, alpha, beta, costs, tile_off + B + 1, stream);
+  return rb::launch_lattice(lp, T_len, U_len, B, T, U1, alpha, beta, costs, c.status, stream);
 }
 
 int rnnt_b200_joint_loss_bwd(const float* enc, int64_t enc_sb, int64_t enc_st, int64_t enc_sh, const float* pred,
@@ -200,44 +288,18 @@ int rnnt_b200_joint_loss_bwd(const float* enc, int64_t enc_sb, int64_t enc_st, i
                              int64_t denc_sh, float* d_pred, float* dW, float* dbias, int64_t ring_tiles, int flags,
                              void* dw_done_event, void* workspace, size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  int rc = check_common(enc, enc_sb, enc_st, enc_sh, pred, B, T, U1, H, V, &blank);
-  if (rc) return rc;
-  rc = check_layout("d_enc", denc_sb, denc_st, denc_sh, B, T, H);
-  if (rc) return rc;
-  RB_REQUIRE((reinterpret_cast<uintptr_t>(d_enc) & 15) == 0, -3, "d_enc must be 16-byte aligned");
-  RB_REQUIRE((reinterpret_cast<uintptr_t>(W) & 15) == 0, -3, "W must be 16-byte aligned");
-  RB_REQUIRE((denc_sh == 1 && denc_st == H && denc_sb == static_cast<int64_t>(T) * H) ||
-                 (denc_st == 1 && denc_sh == T && denc_sb == static_cast<int64_t>(T) * H),
-             -3, "d_enc must be a dense (B,T,H) tensor or a dense (B,H,T) tensor viewed as (B,T,H)");
-  RB_REQUIRE(ring_tiles >= 1 && ring_tiles * kTileM < (1ll << 30), -8, "ring_tiles out of range");
-  RB_REQUIRE(H % 4 == 0, -2, "hidden_features must be a multiple of 4");
   const bool deterministic = (flags & RNNT_B200_DETERMINISTIC) != 0;
-  const WsLayout w = ws_layout(B, T, U1, H, V, ring_tiles, hidden != nullptr, deterministic);
-  RB_REQUIRE(workspace != nullptr && workspace_bytes >= w.total_bwd, -7, "workspace too small: need %zu bytes",
-             w.total_bwd);
-  RB_REQUIRE((reinterpret_cast<uintptr_t>(hidden) & 127) == 0, -3, "hidden must be 128-byte aligned");
-  RB_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, -7, "workspace must be 256-byte aligned");
-  uint8_t* ws = static_cast<uint8_t*>(workspace);
-  int* tile_off = reinterpret_cast<int*>(ws + w.tile_off);
-  __half* Wb = reinterpret_cast<__half*>(ws + w.wb);
-  float* bias2 = reinterpret_cast<float*>(ws + w.bias2);
-  float4* coef = reinterpret_cast<float4*>(ws + w.coef);
-  __half* g_ring = reinterpret_cast<__half*>(ws + w.g_ring);
-  // activations: the forward's residual buffer (rows = half-tile id * 64) or, recomputed, a ring like g's
-  __half* h_src = hidden ? const_cast<__half*>(static_cast<const __half*>(hidden))
-                         : reinterpret_cast<__half*>(ws + w.h_ring);
-  const uint64_t ring_rows = static_cast<uint64_t>(ring_tiles) * kTileM;
-  const int h_map = hidden ? 0 : 1;
+  BwdArgs bwd{d_enc, denc_sb, denc_st, denc_sh, ring_tiles, deterministic, dcost};
+  LossCall c{};
+  int rc = loss_prologue(c, enc, enc_sb, enc_st, enc_sh, pred, W, bias, targets, T_len, U_len, B, T, U1, H, V, blank,
+                         hidden, &bwd, nullptr, workspace, workspace_bytes, stream);
+  if (rc) return rc;
 
   // accumulation targets: the fp32 outputs themselves (atomics), or 64-bit fixed-point shadows (deterministic mode)
   const size_t n_enc = static_cast<size_t>(B) * T * H, n_pred = static_cast<size_t>(B) * U1 * H;
   const size_t n_w = static_cast<size_t>(V) * H;
-  long long* fx_enc = deterministic ? reinterpret_cast<long long*>(ws + w.fx) : nullptr;
-  long long* fx_pred = deterministic ? fx_enc + n_enc : nullptr;
-  long long* fx_w = deterministic ? fx_pred + n_pred : nullptr;
-  long long* fx_b = deterministic ? fx_w + n_w : nullptr;
   if (deterministic) {
-    RB_CUDA_CHECK(cudaMemsetAsync(fx_enc, 0, (n_enc + n_pred + n_w + V) * 8, stream));
+    RB_CUDA_CHECK(cudaMemsetAsync(c.fx_enc, 0, (n_enc + n_pred + n_w + V) * 8, stream));
   } else {
     RB_CUDA_CHECK(cudaMemsetAsync(d_enc, 0, n_enc * 4, stream));
     RB_CUDA_CHECK(cudaMemsetAsync(d_pred, 0, n_pred * 4, stream));
@@ -246,38 +308,26 @@ int rnnt_b200_joint_loss_bwd(const float* enc, int64_t enc_sb, int64_t enc_st, i
   }
 
   const int64_t max_tiles = rnnt_b200_max_tiles(B, T, U1);
-  float* gscale = reinterpret_cast<float*>(tile_off + B + 2);
-  rc = rb::launch_tile_table(T_len, U_len, B, T, U1, tile_off, nullptr, dcost, gscale, stream);
+  rc = rb::launch_coef(lp, lse, alpha, beta, dcost, c.gscale, T_len, U_len, B, T, U1, c.coef, stream);
   if (rc) return rc;
-  rc = rb::launch_convert_weights(W, bias, V, H, w.Vp, w.Hp, Wb, bias2, stream);
-  if (rc) return rc;
-  rc = rb::launch_coef(lp, lse, alpha, beta, dcost, gscale, T_len, U_len, B, T, U1, coef, stream);
-  if (rc) return rc;
-  int* n_active = tile_off + B + 4;
-  int* sub_list = reinterpret_cast<int*>(ws + w.tile_list);    // active half-tiles, order preserved
-  rc = rb::launch_tile_activity(coef, T_len, U_len, tile_off, B, T, U1, max_tiles,
-                                (flags & RNNT_B200_ALL_TILES) ? 1 : 0,
-                                reinterpret_cast<unsigned char*>(ws + w.flags), sub_list, n_active, stream);
+  rc = rb::launch_tile_activity(c.coef, T_len, U_len, c.tile_off, B, T, U1, max_tiles,
+                                (flags & RNNT_B200_ALL_TILES) ? 1 : 0, c.flags, c.sub_list, c.n_active, stream);
   if (rc) return rc;
 
+  // activations: the forward's residual buffer (rows = half-tile id * 64) or, recomputed, a ring like g's
+  const __half* h_src = hidden ? static_cast<const __half*>(hidden) : c.h_ring;
+  const uint64_t ring_rows = static_cast<uint64_t>(ring_tiles) * kTileM;
   const uint64_t h_rows = hidden ? static_cast<uint64_t>(max_tiles) * kTileM : ring_rows;
-  CUtensorMap tmW, tmWmn, tmG128, tmHk, tmHk2, tmGmn, tmHmn;
-  // W [Vp, Hp]: K-major boxes (64 k x 128 v) for the recompute, MN-major boxes (64 k_h x 64 v) for dh
-  rc = rb::make_tmap_2d(&tmW, Wb, 2, w.Hp, w.Vp, static_cast<uint64_t>(w.Hp) * 2, 64, 128);
+  const int Hp = c.w.Hp, Vp = c.w.Vp;
+  CUtensorMap tmWmn, tmHk, tmHk2, tmGmn, tmG128;
+  // W [Vp, Hp]: MN-major boxes (64 k_h x 64 v) for dh.  Activations: the 64-row boxes serve as the K-major operand of
+  // the logit recompute and the MN-major operand of dW.  Gradient ring: 64 x 128 K-major boxes for dh (two work-list
+  // slots per CTA of a pair), 64 x 64 boxes for the MN-major dW operand
+  rc = rb::make_tmap_2d(&tmWmn, c.Wb, 2, Hp, Vp, static_cast<uint64_t>(Hp) * 2, 64, 64);
   if (rc) return rc;
-  rc = rb::make_tmap_2d(&tmWmn, Wb, 2, w.Hp, w.Vp, static_cast<uint64_t>(w.Hp) * 2, 64, 64);
+  rc = make_row_maps(&tmHk, &tmHk2, h_src, h_rows, Hp);
   if (rc) return rc;
-  // activations: 64 x 64 boxes (one half-tile), K-major for the logit recompute and MN-major for the dW operand;
-  // gradient ring: 64 x 128 K-major boxes for dh (two work-list slots per CTA of a pair), 64 x 64 boxes for the MN-major dW operand
-  rc = rb::make_tmap_2d(&tmHk, h_src, 2, w.Hp, h_rows, static_cast<uint64_t>(w.Hp) * 2, 64, 64);
-  if (rc) return rc;
-  rc = rb::make_tmap_2d(&tmHk2, h_src, 2, w.Hp, h_rows, static_cast<uint64_t>(w.Hp) * 2, 64, 128);
-  if (rc) return rc;
-  rc = rb::make_tmap_2d(&tmG128, g_ring, 2, w.Vp, ring_rows, static_cast<uint64_t>(w.Vp) * 2, 64, 128);
-  if (rc) return rc;
-  rc = rb::make_tmap_2d(&tmGmn, g_ring, 2, w.Vp, ring_rows, static_cast<uint64_t>(w.Vp) * 2, 64, 64);
-  if (rc) return rc;
-  rc = rb::make_tmap_2d(&tmHmn, h_src, 2, w.Hp, h_rows, static_cast<uint64_t>(w.Hp) * 2, 64, 64);
+  rc = make_row_maps(&tmGmn, &tmG128, c.g_ring, ring_rows, Vp);
   if (rc) return rc;
 
   // The work list is walked in chunks of as many slots (half-tiles of 64 rows) as the ring holds.  Per chunk: G (logit
@@ -285,56 +335,41 @@ int rnnt_b200_joint_loss_bwd(const float* enc, int64_t enc_sb, int64_t enc_st, i
   // `dw_done_event` lets the caller start their all-reduce while the dh GEMM of that chunk is still running.
   const int64_t max_slots = 2 * max_tiles, ring_slots = 2 * ring_tiles;
   const int64_t nchunks = (max_slots + ring_slots - 1) / ring_slots;
-  for (int64_t c = 0; c < nchunks; ++c) {
-    const int slot_begin = static_cast<int>(c * ring_slots);
-    const int64_t chunk_slots = std::min<int64_t>(ring_slots, max_slots - c * ring_slots);
-    rb::JointArgs a{};
-    a.enc = enc; a.enc_sb = enc_sb; a.enc_st = enc_st; a.enc_sh = enc_sh;
-    a.pred = pred; a.pred_sb = static_cast<long long>(U1) * H; a.pred_su = H;
-    a.bias2 = bias2; a.targets = targets; a.tgt_ld = U1 - 1;
-    a.T_len = T_len; a.U_len = U_len; a.tile_off = tile_off;
-    a.B = B; a.T = T; a.U1 = U1; a.H = H; a.Hp = w.Hp; a.V = V; a.Vp = w.Vp; a.blank = blank;
-    a.slot_begin = slot_begin; a.slot_cap = static_cast<int>(ring_slots); a.sub_list = sub_list; a.n_active = n_active;
+  for (int64_t k = 0; k < nchunks; ++k) {
+    c.base.slot_begin = static_cast<int>(k * ring_slots);
+    const int64_t chunk_slots = std::min<int64_t>(ring_slots, max_slots - k * ring_slots);
+    rb::JointArgs a{c.base};
+    a.lp = const_cast<float*>(lp); a.coef = c.coef; a.dcost = dcost; a.clamp = clamp;
+    a.h_out = const_cast<__half*>(h_src); a.g_ring = c.g_ring;
     a.dbg = env_knobs().dbg;
-    a.lp = const_cast<float*>(lp); a.lse = nullptr; a.coef = coef; a.dcost = dcost; a.gscale = gscale; a.clamp = clamp;
-    a.h_out = h_src; a.h_map = h_map; a.g_ring = g_ring;
-    rc = rb::launch_joint_gemm(1, hidden == nullptr, tmW, tmHk, tmHk2, a, chunk_slots, stream);
+    rc = rb::launch_joint_gemm(1, hidden == nullptr, c.tmW, tmHk, tmHk2, a, chunk_slots, stream);
     if (rc) return rc;
 
-    rb::DwArgs g{};
-    g.n_active = n_active; g.sub_list = sub_list; g.h_map = h_map; g.tile_off = tile_off; g.B = B; g.H = H; g.Hp = w.Hp; g.V = V; g.Vp = w.Vp;
-    g.slot_begin = slot_begin; g.slot_cap = static_cast<int>(ring_slots); g.dW = dW; g.db = dbias; g.gscale = gscale;
-    g.dW_fx = fx_w; g.db_fx = fx_b;
-    if (env_knobs().no_db) g.db = nullptr;
-    rc = rb::launch_dw_gemm(tmGmn, tmHmn, g, chunk_slots, stream);
+    rb::DwArgs g{c.base};
+    g.dW = dW; g.db = env_knobs().no_db ? nullptr : dbias; g.dW_fx = c.fx_w; g.db_fx = c.fx_b;
+    rc = rb::launch_dw_gemm(tmGmn, tmHk, g, chunk_slots, stream);
     if (rc) return rc;
-    if (c == nchunks - 1) {
+    if (k == nchunks - 1) {
       if (deterministic) {
-        rc = rb::launch_finalize_fixed(fx_w, dW, 1, V, H, 0, H, 1, gscale, stream);
+        rc = rb::launch_finalize_fixed(c.fx_w, dW, 1, V, H, 0, H, 1, c.gscale, stream);
         if (rc) return rc;
-        rc = rb::launch_finalize_fixed(fx_b, dbias, 1, 1, V, 0, 0, 1, gscale, stream);
+        rc = rb::launch_finalize_fixed(c.fx_b, dbias, 1, 1, V, 0, 0, 1, c.gscale, stream);
         if (rc) return rc;
       }
       if (dw_done_event) RB_CUDA_CHECK(cudaEventRecord(static_cast<cudaEvent_t>(dw_done_event), stream));
     }
 
-    rb::DhArgs d{};
-    d.enc = enc; d.enc_sb = enc_sb; d.enc_st = enc_st; d.enc_sh = enc_sh;
-    d.pred = pred; d.pred_sb = static_cast<long long>(U1) * H; d.pred_su = H; d.gscale = gscale; d.sub_list = sub_list; d.n_active = n_active;
-    d.T_len = T_len; d.U_len = U_len; d.tile_off = tile_off;
-    d.B = B; d.T = T; d.U1 = U1; d.H = H; d.Hp = w.Hp; d.Vp = w.Vp;
-    d.slot_begin = slot_begin; d.slot_cap = static_cast<int>(ring_slots);
+    rb::DhArgs d{c.base};
     d.d_enc = d_enc; d.denc_sb = denc_sb; d.denc_st = denc_st; d.denc_sh = denc_sh; d.d_pred = d_pred;
-    d.d_enc_fx = fx_enc; d.d_pred_fx = fx_pred;
-    // with a dW-done event the caller is about to run a collective next to this kernel: leave it a few SMs
-    d.spare_pairs = (dw_done_event && c == nchunks - 1) ? env_knobs().comm_sms / 2 : 0;
+    d.d_enc_fx = c.fx_enc; d.d_pred_fx = c.fx_pred;
     rc = rb::launch_dh_gemm(tmG128, tmWmn, d, chunk_slots, stream);
     if (rc) return rc;
   }
   if (deterministic) {
-    rc = rb::launch_finalize_fixed(fx_enc, d_enc, B, T, H, denc_sb, denc_st, denc_sh, gscale, stream);
+    rc = rb::launch_finalize_fixed(c.fx_enc, d_enc, B, T, H, denc_sb, denc_st, denc_sh, c.gscale, stream);
     if (rc) return rc;
-    rc = rb::launch_finalize_fixed(fx_pred, d_pred, 1, static_cast<long long>(B) * U1, H, 0, H, 1, gscale, stream);
+    rc = rb::launch_finalize_fixed(c.fx_pred, d_pred, 1, static_cast<long long>(B) * U1, H, 0, H, 1, c.gscale,
+                                   stream);
     if (rc) return rc;
   }
   return 0;

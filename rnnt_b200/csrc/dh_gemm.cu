@@ -223,8 +223,7 @@ int launch_dh_gemm(const CUtensorMap& tmG, const CUtensorMap& tmWmn, const DhArg
   const size_t smem = SmemLayout::total + 1024;
   RB_CUDA_CHECK(cudaFuncSetAttribute(dh_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const long long items = ((chunk_slots + 3) / 4) * ((args.Hp + 255) / 256);
-  int pairs = max_cta_pairs(reinterpret_cast<const void*>(dh_gemm_kernel), kNumThreads, smem);
-  pairs = std::max(1, pairs - args.spare_pairs);     // SMs left free for a concurrent collective (data-parallel callers)
+  const int pairs = max_cta_pairs(reinterpret_cast<const void*>(dh_gemm_kernel), kNumThreads, smem);
   const int grid = 2 * static_cast<int>(std::max<long long>(1, std::min<long long>(pairs, items)));
   dh_gemm_kernel<<<grid, kNumThreads, smem, stream>>>(tmG, tmWmn, args);
   RB_CUDA_CHECK(cudaGetLastError());

@@ -11,7 +11,9 @@
 
 namespace rb {
 
-struct JointArgs {
+// What the kernels of the fused loss (joint GEMM, dh, dW) share: the joint's inputs, the batch's lengths and tile table,
+// the sizes, the window of work-list slots a launch covers, and the gradient scale.  Not every kernel reads every field.
+struct BatchArgs {
   const float* enc;       // (B,T,H) fp32 with element strides (enc_sb, enc_st, enc_sh): H-contiguous (enc_sh == 1) or
   long long enc_sb, enc_st, enc_sh;   // the T-contiguous view of the encoder's (B,H,T) output (enc_st == 1)
   const float* pred;      // (B,U1,H) fp32, H contiguous
@@ -24,34 +26,26 @@ struct JointArgs {
   const int* tile_off;    // [B+1] prefix sum of half-tiles (16 t x 4 u) per utterance; tile_off[B] = total
   int B, T, U1, H, Hp, V, Vp, blank;
   int slot_begin, slot_cap;   // process work-list slots (half-tiles, 64 rows) [slot_begin, min(count, slot_begin + slot_cap))
-  const int* sub_list;    // G: slot -> half-tile id (active ones only); nullptr (F) = identity over all half-tiles
-  const int* n_active;    // G: number of slots in sub_list
+  const int* sub_list;    // backward: slot -> half-tile id (active ones only), ring rows [64 i, 64 i + 64) hold
+                          // sub_list[slot_begin + i]; nullptr (forward) = identity over all half-tiles
+  const int* n_active;    // backward: number of slots in sub_list
+  const float* gscale;    // backward: {S, 1/S} power-of-two gradient scale
+  int h_map;              // rows of a half-tile in the activation buffer: 0 = half_id*64 (saved residual), 1 = ring
+                          // slot*64 (backward recompute), 2 = per-CTA scratch (forward without a residual buffer)
+};
+
+struct JointArgs : BatchArgs {
   float* lp;              // F: output (B,T,U1,2) log-probs (blank, label); G: the same tensor, read-only
   float* lse;             // F: (B,T,U1) log-sum-exp of the logits (natural log)
   const float4* coef;     // G: (B,T,U1) (gamma*dc*S, eB*dc*S, eE*dc*S, lse)
   const float* dcost;     // G: (B) or nullptr (only used to scale the clamp bound)
-  const float* gscale;    // G: {S, 1/S} power-of-two gradient scale
   float clamp;            // G: <= 0 disables (torchaudio's clamp argument, rnnt/model.py:40 passes -1)
   __half* h_out;          // producers: activation rows h = tanh(enc+pred) as fp16 [rows, Hp] (same buffer tmH reads)
-  int h_map;              // rows of a half-tile in that buffer: 0 = half_id*64 (saved residual), 1 = ring slot*64
-                          // (backward recompute), 2 = per-CTA scratch (forward without a residual buffer)
   __half* g_ring;         // G: gradient ring [ring_tiles*128, Vp] fp16
   int dbg;                // diagnostics only (RNNT_B200_DBG): 1 = skip epilogue math, 2 = skip producer math
 };
 
-struct DhArgs {
-  const float* enc;       // (B,T,H) fp32, strides as in JointArgs (tanh' is recomputed from the inputs)
-  long long enc_sb, enc_st, enc_sh;
-  const float* pred;      // (B,U1,H)
-  long long pred_sb, pred_su;
-  const float* gscale;    // {S, 1/S}
-  const int* sub_list;    // slot -> half-tile id; ring rows [64 i, 64 i + 64) hold sub_list[slot_begin + i]
-  const int* n_active;
-  const int* T_len;
-  const int* U_len;
-  const int* tile_off;
-  int B, T, U1, H, Hp, Vp;
-  int slot_begin, slot_cap;
+struct DhArgs : BatchArgs {   // tanh' is recomputed from enc and pred
   float* d_enc;          // (B,T,H) fp32 with element strides (denc_sb, denc_st, denc_sh), accumulated with atomics
   long long denc_sb, denc_st, denc_sh;   // (caller zero-fills)
   float* d_pred;         // (B,U1,H) contiguous
@@ -59,19 +53,11 @@ struct DhArgs {
   // dense (B,T,H) / (B,U1,H) row-major, converted to d_enc / d_pred by finalize_fixed_kernel
   long long* d_enc_fx;
   long long* d_pred_fx;
-  int spare_pairs;       // CTA pairs (2 SMs each) the launch leaves idle so that a concurrent NCCL kernel finds SMs
 };
 
-struct DwArgs {
-  const int* n_active;   // number of work-list slots (ring rows of this chunk = slots in range * 64)
-  const int* sub_list;   // slot -> half-tile id (row block of the saved activations when h_map == 0)
-  int h_map;             // 0 = activations come from the forward's residual buffer (rows half_id*64), 1 = from the ring
-  const int* tile_off;
-  int B, H, Hp, V, Vp;
-  int slot_begin, slot_cap;
+struct DwArgs : BatchArgs {   // ring rows of a chunk = slots in range * 64; h_map is 0 or 1
   float* dW;             // (V,H) fp32, accumulated with atomics (caller zero-fills)
   float* db;             // (V) fp32, accumulated with atomics (column sums of g, taken from the A stages)
-  const float* gscale;   // {S, 1/S}
   long long* dW_fx;      // deterministic mode: 64-bit fixed-point accumulators (V,H) / (V), else nullptr
   long long* db_fx;
   int ksplit;
@@ -128,8 +114,10 @@ int launch_dw_gemm(const CUtensorMap& tmGmn, const CUtensorMap& tmHmn, const DwA
                    cudaStream_t stream);   // picks args.ksplit itself
 
 // prep / small kernels (prep.cu, lattice.cu, decode.cu)
-int launch_tile_table(const int* T_len, const int* U_len, int B, int T, int U1, int* tile_off, int* err_flag,
-                      const float* dcost, float* gscale, cudaStream_t stream);
+// status: internal word, non-zero when a length is out of range (read by the lattice); err_flag: optional copy for the
+// caller; gscale (optional): {S, 1/S} derived from dcost
+int launch_tile_table(const int* T_len, const int* U_len, int B, int T, int U1, int* tile_off, int* status,
+                      int* err_flag, const float* dcost, float* gscale, cudaStream_t stream);
 int launch_convert_weights(const float* W, const float* bias, int V, int H, int Vp, int Hp, __half* Wh,
                            float* bias2, cudaStream_t stream);
 // status (optional): device flag written by the tile table; a non-zero flag turns every cost into NaN

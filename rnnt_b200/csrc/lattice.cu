@@ -18,8 +18,9 @@ namespace {
 // Also derives the exact power-of-two scale S that maps max_b |dcost_b| into [2^(kGradShift-1), 2^kGradShift): the backward
 // stores logit-gradients in fp16 as g*S (full use of fp16's range whatever the loss scaling) and its epilogues apply 1/S.
 __global__ void tile_table_kernel(const int* __restrict__ T_len, const int* __restrict__ U_len, int B, int T, int U1,
-                                  int* __restrict__ tile_off, int* __restrict__ err_flag,
-                                  const float* __restrict__ dcost, float* __restrict__ gscale) {
+                                  int* __restrict__ tile_off, int* __restrict__ status,
+                                  int* __restrict__ err_flag, const float* __restrict__ dcost,
+                                  float* __restrict__ gscale) {
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
   int acc = 0, bad = 0;
   tile_off[0] = 0;
@@ -47,7 +48,7 @@ __global__ void tile_table_kernel(const int* __restrict__ T_len, const int* __re
     acc += ((Tb + kTileT - 1) / kTileT) * ((Ub + 1 + kHalfU - 1) / kHalfU);     // half-tiles of 16(t) x 4(u)
     tile_off[b + 1] = acc;
   }
-  tile_off[B + 1] = bad;          // internal status word: the lattice kernel turns the costs into NaN when it is set
+  *status = bad;                  // the lattice kernel turns the costs into NaN when it is set
   if (err_flag) *err_flag = bad;
 }
 
@@ -230,7 +231,7 @@ __global__ void coef_kernel(const float* __restrict__ lp, const float* __restric
 __global__ void tile_activity_kernel(const float4* __restrict__ coef, const int* __restrict__ T_len,
                                      const int* __restrict__ U_len, const int* __restrict__ tile_off, int B, int T,
                                      int U1, int dense, unsigned char* __restrict__ flags) {
-  const int total = __ldg(tile_off + B);
+  const int total = __ldg(&tile_off[B]);
   const int lane = threadIdx.x & 31;
   const int w0 = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int nw = (gridDim.x * blockDim.x) >> 5;
@@ -261,7 +262,7 @@ __global__ void tile_activity_kernel(const float4* __restrict__ coef, const int*
 __global__ void tile_compact_kernel(const unsigned char* __restrict__ flags, const int* __restrict__ tile_off, int B,
                                     int* __restrict__ sub_list, int* __restrict__ n_active) {
   __shared__ int sums[1024];
-  const int total = __ldg(tile_off + B);
+  const int total = __ldg(&tile_off[B]);
   const int per = (total + blockDim.x - 1) / blockDim.x;
   const int lo = min(total, (int)threadIdx.x * per), hi = min(total, lo + per);
   int cnt = 0;
@@ -371,10 +372,10 @@ int launch_finalize_fixed(const long long* fx, float* out, long long n0, long lo
   return 0;
 }
 
-int launch_tile_table(const int* T_len, const int* U_len, int B, int T, int U1, int* tile_off, int* err_flag,
-                      const float* dcost, float* gscale, cudaStream_t stream) {
+int launch_tile_table(const int* T_len, const int* U_len, int B, int T, int U1, int* tile_off, int* status,
+                      int* err_flag, const float* dcost, float* gscale, cudaStream_t stream) {
   ProfScope prof_(kProfPrep, stream);
-  tile_table_kernel<<<1, 32, 0, stream>>>(T_len, U_len, B, T, U1, tile_off, err_flag, dcost, gscale);
+  tile_table_kernel<<<1, 32, 0, stream>>>(T_len, U_len, B, T, U1, tile_off, status, err_flag, dcost, gscale);
   RB_CUDA_CHECK(cudaGetLastError());
   return 0;
 }
