@@ -75,8 +75,10 @@ int rnnt_b200_joint_loss_fwd(const float* enc, int64_t enc_sb, int64_t enc_st, i
  * Outputs are overwritten, all fp32: d_enc = a dense (B,T,H) tensor (strides (T*H, H, 1)) or a dense (B,H,T) tensor
  * viewed as (B,T,H) (strides (T*H, 1, T): the gradient lands in the encoder's own layout), d_pred (B,U1,H), dW (V,H),
  * dbias (V) -- dW / dbias may point into a flat all-reduce bucket.
- * Half-tiles (16 t x 4 u lattice blocks) whose scaled logit-gradients are all below fp16 resolution (occupancy < 2^-25
- * of max|dcost|) are exactly zero in the gradient ring and are skipped; RNNT_B200_ALL_TILES disables the skipping.
+ * Half-tiles (16 t x 4 u lattice blocks) whose logit-gradients are all at most 2^-25 of max|dcost| are skipped: they
+ * are left out of the work list, so they add nothing to d_enc, d_pred, dW and dbias, although their gradients need not
+ * be zero.  The work list holds, in order, exactly the half-tiles with a valid cell whose gradient coefficients exceed
+ * that bound; RNNT_B200_ALL_TILES disables the skipping.
  * RNNT_B200_DETERMINISTIC replaces the fp32 atomics (d_enc, d_pred, dW, dbias are sums over CTAs) by 64-bit
  * fixed-point accumulation, which is order-independent: gradients are bit-identical from run to run.
  * dw_done_event (optional cudaEvent_t, may be NULL) is recorded on `stream` as soon as dW and dbias are final, before

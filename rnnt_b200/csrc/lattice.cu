@@ -223,7 +223,7 @@ __global__ void coef_kernel(const float* __restrict__ lp, const float* __restric
 }
 
 // ---- occupancy sparsity of the backward.  The logit-gradients of a cell are bounded by max(|gamma'|,|eB'|,|eE'|)
-// (coef already carries dcost * S).  A HALF-TILE (16 t x 4 u = 64 cells) whose cells are all below 2^-25 of the largest
+// (coef already carries dcost * S).  A HALF-TILE (16 t x 4 u = 64 cells) whose cells are all at most 2^-25 of the largest
 // possible gradient entry max_b |dcost_b| (kSkipBelow; half the resolution fp32 has for that entry) is dropped from the
 // backward's work list: what it would add to dh / dW / db is below the rounding of the terms that dominate them.
 // One warp per half-tile, then a single-block compaction (order preserved).  In dense mode (RNNT_B200_ALL_TILES) every

@@ -75,6 +75,12 @@ def _check_index_tensors(targets, logit_lengths, target_lengths):
         raise RuntimeError("targets must be contiguous")
 
 
+def _check_blank(blank, V):
+    """torchaudio's check and message: blank < 0 counts from the end of the vocabulary."""
+    if not -V <= int(blank) < V:
+        raise RuntimeError("blank must be within [0, logits.shape[-1])")
+
+
 def pick_ring_tiles(B: int, T: int, U1: int, H: int, V: int, ring_bytes: Optional[int] = None,
                     have_hidden: bool = False) -> int:
     """Tiles per backward chunk: the batch's tile bound split into equal chunks of at most `ring_bytes`."""
@@ -292,6 +298,7 @@ def joint_rnnt_loss(audio_frame, text_frame, weight, bias, targets, logit_length
     _check_index_tensors(targets, logit_lengths, target_lengths)
     if targets.shape[0] != audio_frame.shape[0] or targets.shape[1] != text_frame.shape[1] - 1:
         raise RuntimeError("output length mismatch")
+    _check_blank(blank, weight.shape[0])
     if validate:
         _validate_lengths(audio_frame.shape[1], text_frame.shape[1], logit_lengths, target_lengths)
     costs, lp, lse, alpha, beta = _FusedJointLoss.apply(audio_frame, text_frame, weight.float(), bias.float(),
@@ -370,6 +377,7 @@ def rnnt_loss(logits, targets, logit_lengths, target_lengths, blank: int = -1, c
         raise RuntimeError("logits must be 4-D (batch, time, target, class)")
     _check_index_tensors(targets, logit_lengths, target_lengths)
     _validate_lengths(logits.shape[1], logits.shape[2], logit_lengths, target_lengths)
+    _check_blank(blank, logits.shape[-1])
     costs = _DenseLoss.apply(logits, targets, logit_lengths, target_lengths, int(blank), float(clamp))
     return _reduce(costs, reduction)
 

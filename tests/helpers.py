@@ -108,11 +108,13 @@ def make_inputs(B, T, U, H, V, seed=1234, ragged=False, device="cuda", scale=1.0
     return dict(enc=to(enc), pred=to(pred), W=to(W), b=to(b), targets=to(targets), T_len=to(T_len), U_len=to(U_len))
 
 
-def fused_raw(inp, ring_tiles=None, dcost=None, clamp=-1.0, flags=0, save_hidden=True):
+def fused_raw(inp, ring_tiles=None, dcost=None, clamp=-1.0, flags=0, save_hidden=True, blank=-1, fill=None):
     """Call the C-ABI forward + backward directly; returns outputs plus the raw workspace and its layout.
     save_hidden=False exercises the memory-lean mode (per-SM scratch in the forward, recomputing backward).
     flags: 1 = RNNT_B200_ALL_TILES, 2 = RNNT_B200_DETERMINISTIC.  inp["enc"] may be H-contiguous or the T-contiguous
-    permuted view of a (B,H,T) tensor; d_enc is produced in the same layout."""
+    permuted view of a (B,H,T) tensor; d_enc is produced in the same layout.  fill: a byte value the workspace, `hidden`
+    and every output are filled with before the calls (default zeros), so a test can vary memory the kernels must
+    overwrite."""
     from rnnt_b200 import _lib
     from rnnt_b200.functional import _stream_ptr, pick_ring_tiles
     L = _lib.lib()
@@ -128,10 +130,12 @@ def fused_raw(inp, ring_tiles=None, dcost=None, clamp=-1.0, flags=0, save_hidden
     hp, vp = C.c_int(0), C.c_int(0)
     _lib.check(L.rnnt_b200_debug_ws_layout(B, T, U1, H, V, ring_tiles, int(save_hidden), offs, C.byref(hp),
                                            C.byref(vp)), "layout")
-    ws = torch.zeros(int(offs[6]), dtype=torch.uint8, device=dev)
-    hidden = torch.zeros(L.rnnt_b200_hidden_bytes(B, T, U1, H), dtype=torch.uint8, device=dev) if save_hidden else None
+    byte = 0 if fill is None else int(fill)
+    raw = lambda n: torch.full((n,), byte, dtype=torch.uint8, device=dev)
+    ws = raw(int(offs[6]))
+    hidden = raw(L.rnnt_b200_hidden_bytes(B, T, U1, H)) if save_hidden else None
     hptr = hidden.data_ptr() if save_hidden else None
-    f = lambda *s: torch.zeros(*s, dtype=torch.float32, device=dev)
+    f = lambda *s: raw(4 * int(np.prod(s))).view(torch.float32).view(*s)
     d_enc = f(B, H, T).permute(0, 2, 1) if (enc.stride(1) == 1 and T > 1) else f(B, T, H)
     out = dict(costs=f(B), lp=f(B, T, U1, 2), lse=f(B, T, U1), alpha=f(B, T, U1), beta=f(B, T, U1),
                d_enc=d_enc, d_pred=f(B, U1, H), dW=f(V, H), db=f(V))
@@ -139,7 +143,7 @@ def fused_raw(inp, ring_tiles=None, dcost=None, clamp=-1.0, flags=0, save_hidden
     st = _stream_ptr(dev)
     _lib.check(L.rnnt_b200_joint_loss_fwd(
         enc.data_ptr(), enc.stride(0), enc.stride(1), enc.stride(2), pred.data_ptr(), W.data_ptr(), b.data_ptr(),
-        targets.data_ptr(), T_len.data_ptr(), U_len.data_ptr(), B, T, U1, H, V, -1, out["costs"].data_ptr(),
+        targets.data_ptr(), T_len.data_ptr(), U_len.data_ptr(), B, T, U1, H, V, blank, out["costs"].data_ptr(),
         out["lp"].data_ptr(), out["lse"].data_ptr(), out["alpha"].data_ptr(), out["beta"].data_ptr(),
         hptr, status.data_ptr(), ws.data_ptr(), ws.numel(), st), "fwd")
     torch.cuda.synchronize()
@@ -147,7 +151,7 @@ def fused_raw(inp, ring_tiles=None, dcost=None, clamp=-1.0, flags=0, save_hidden
         dcost = torch.ones(B, dtype=torch.float32, device=dev)
     _lib.check(L.rnnt_b200_joint_loss_bwd(
         enc.data_ptr(), enc.stride(0), enc.stride(1), enc.stride(2), pred.data_ptr(), W.data_ptr(), b.data_ptr(),
-        targets.data_ptr(), T_len.data_ptr(), U_len.data_ptr(), B, T, U1, H, V, -1, out["lp"].data_ptr(),
+        targets.data_ptr(), T_len.data_ptr(), U_len.data_ptr(), B, T, U1, H, V, blank, out["lp"].data_ptr(),
         out["lse"].data_ptr(), out["alpha"].data_ptr(), out["beta"].data_ptr(), hptr, dcost.data_ptr(), float(clamp),
         d_enc.data_ptr(), d_enc.stride(0), d_enc.stride(1), d_enc.stride(2), out["d_pred"].data_ptr(),
         out["dW"].data_ptr(), out["db"].data_ptr(), ring_tiles, flags, None, ws.data_ptr(), ws.numel(), st), "bwd")
@@ -170,6 +174,24 @@ def ring_views(out):
     B = out["costs"].numel()
     scale = ws[offs[0] + (B + 2) * 4: offs[0] + (B + 4) * 4].view(torch.float32)   # {S, 1/S}
     return g, h, float(scale[0])
+
+
+def ws_views(out):
+    """Typed views of the workspace regions rnnt_b200_debug_ws_layout documents, as a backward call left them: tile_off
+    [B+1] (prefix sums of half-tiles), W16 [Vp, Hp] fp16, bias2 [Vp] (bias * log2 e), coef (B,T,U1,4), g ring
+    [ring_tiles*128, Vp] fp16, h ring [ring_tiles*128, Hp] fp16 (None with a saved residual), work list [n_active] int32,
+    S and 1/S."""
+    ws, offs, Hp, Vp = out["ws"], out["offs"], out["Hp"], out["Vp"]
+    B, T, U1 = out["lse"].shape
+    rows = out["ring_tiles"] * 128
+    region = lambda off, n, dt: ws[off: off + n * dt.itemsize].view(dt)
+    meta = region(offs[0], B + 5, torch.int32)
+    gs = region(offs[0] + (B + 2) * 4, 2, torch.float32)
+    return dict(tile_off=meta[:B + 1], W16=region(offs[1], Vp * Hp, torch.float16).view(Vp, Hp),
+                bias2=region(offs[2], Vp, torch.float32), coef=region(offs[3], B * T * U1 * 4, torch.float32).view(B, T, U1, 4),
+                g=region(offs[4], rows * Vp, torch.float16).view(rows, Vp),
+                h=None if offs[5] < 0 else region(offs[5], rows * Hp, torch.float16).view(rows, Hp),
+                work_list=region(offs[7], out["active_halves"], torch.int32), S=float(gs[0]), inv_S=float(gs[1]))
 
 
 def tile_rows(T_len, U_len, out=None):
@@ -195,7 +217,7 @@ def tile_rows(T_len, U_len, out=None):
     return rows
 
 
-def torch_reference(inp, emulate_bf16=False, dcost=None, device=None):
+def torch_reference(inp, emulate_bf16=False, dcost=None, device=None, blank=-1):
     """fp32 torch restatement on the SAME device (oracle/ref_path.py semantics), optionally with the joint GEMM
     operands (tanh output, W) rounded to fp16 as the kernels do, to separate kernel bugs from precision."""
     import torchaudio
@@ -213,7 +235,7 @@ def torch_reference(inp, emulate_bf16=False, dcost=None, device=None):
     else:
         Wq = W
     logits = torch.nn.functional.linear(h, Wq, b)
-    costs = torchaudio.functional.rnnt_loss(logits, inp["targets"], inp["T_len"], inp["U_len"], blank=-1, clamp=-1,
+    costs = torchaudio.functional.rnnt_loss(logits, inp["targets"], inp["T_len"], inp["U_len"], blank=blank, clamp=-1,
                                             reduction="none")
     costs.backward(torch.ones_like(costs) if dcost is None else dcost)
     return dict(costs=costs.detach(), d_enc=enc.grad, d_pred=pred.grad, dW=W.grad, db=b.grad,
