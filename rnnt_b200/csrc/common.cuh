@@ -93,30 +93,9 @@ __device__ __forceinline__ void tma_load_2d(uint32_t smem_dst, const void* tmap,
 }
 // ---------------------------------------------------------------------------------------------
 // tcgen05 / TMEM
-__device__ __forceinline__ void tmem_alloc(uint32_t smem_result_addr, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_result_addr),
-               "r"(ncols)
-               : "memory");
-}
-__device__ __forceinline__ void tmem_relinquish() {
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
-// D[tmem] (+)= A[smem] * B[smem]; one thread issues for the CTA.
-__device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
-                                         uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
 // mbarrier arrives when all previously issued tcgen05.mma of this thread have completed
 // (implies tcgen05.fence::before_thread_sync).
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
@@ -168,27 +147,6 @@ __device__ __forceinline__ void tma_load_2d_pair(uint32_t smem_dst, const void* 
       "l"(reinterpret_cast<uint64_t>(tmap)), "r"(bar_cluster_addr), "r"(c0), "r"(c1)
       : "memory");
 }
-__device__ __forceinline__ void tmem_alloc_pair(uint32_t smem_result_addr, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_result_addr),
-               "r"(ncols)
-               : "memory");
-}
-__device__ __forceinline__ void tmem_relinquish_pair() {
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-// D[tmem of both CTAs] (+)= A[smem of both CTAs, 128 rows each] * B[smem of both CTAs, N/2 rows each]; leader CTA only.
-__device__ __forceinline__ void umma_f16_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
-                                              uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
 // arrives on the mbarrier at this shared-memory offset in every CTA of `cta_mask` once all MMAs issued so far are done
 __device__ __forceinline__ void umma_commit_pair(uint32_t bar, uint16_t cta_mask) {
   asm volatile(
@@ -203,11 +161,6 @@ __device__ __forceinline__ void umma_commit_pair(uint32_t bar, uint16_t cta_mask
 // Shared-memory matrix descriptor, 128-byte swizzle, descriptor version 1:
 //   [0,14) start address >> 4 | [16,30) leading byte offset >> 4 | [32,46) stride byte offset >> 4
 //   [46,48) version = 1 | [61,64) layout type (2 = SWIZZLE_128B)
-// K-major operand tile (rows = M or N, 64 bf16 of K per 128-byte row, 8-row 1024-byte swizzle atoms):
-//   SBO = 1024 (next 8-row group), LBO unused (1).  Advance K by 16 elements = +32 bytes on the start address.
-// MN-major operand tile (rows = K, 64 bf16 of M/N per 128-byte row):
-//   SBO = 1024 (next 8 K-rows), LBO = byte stride between 64-element M/N blocks.
-//   Advance K by 16 rows = +2048 bytes on the start address.
 __device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
   uint64_t d = 0;
   d |= static_cast<uint64_t>((saddr & 0x3FFFF) >> 4);

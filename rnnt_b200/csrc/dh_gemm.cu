@@ -15,8 +15,8 @@
 // halves of TMEM so the epilogue of item i overlaps the MMAs of item i+1.
 #include <algorithm>
 
-#include "common.cuh"
 #include "kernels.h"
+#include "tc_kernel.cuh"
 
 namespace rb {
 namespace {
@@ -34,18 +34,19 @@ struct SmemLayout {
   static constexpr int bars = a_ring + kStages * kBytesA;
   static constexpr int total = bars + 256;
 };
+struct Bars {
+  uint64_t full[kStages], empty[kStages], tmem_full[2], tmem_empty[2];
+  uint32_t tmem_slot;
+};
+static_assert(sizeof(Bars) <= SmemLayout::total - SmemLayout::bars, "barrier block overflows its region");
 
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kNumThreads, 1)
 dh_gemm_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CUtensorMap tmWmn, DhArgs p) {
   extern __shared__ uint8_t smem_raw[];
-  const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
-  const uint32_t b_ring = smem_base + SmemLayout::b_ring;
-  const uint32_t a_ring = smem_base + SmemLayout::a_ring;
-  const uint32_t bars = smem_base + SmemLayout::bars;
-  const uint32_t full = bars, empty = bars + 8 * kStages;
-  const uint32_t tmem_full = bars + 16 * kStages, tmem_empty = tmem_full + 16;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem_gen + SmemLayout::bars + 200);
+  const AlignedSmem smem = aligned_smem(smem_raw);
+  const uint32_t b_ring = smem.addr + SmemLayout::b_ring;
+  const uint32_t a_ring = smem.addr + SmemLayout::a_ring;
+  Bars* bars = reinterpret_cast<Bars*>(smem.ptr + SmemLayout::bars);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t rank = cluster_ctarank();
@@ -61,16 +62,11 @@ dh_gemm_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ 
   if (threadIdx.x == 0) {
     tma_prefetch_desc(&tmG);
     tma_prefetch_desc(&tmWmn);
-    for (int s = 0; s < kStages; ++s) { mbar_init(full + 8 * s, 2); mbar_init(empty + 8 * s, 1); }
-    for (int s = 0; s < 2; ++s) { mbar_init(tmem_full + 8 * s, 1); mbar_init(tmem_empty + 8 * s, 8 * kEpiSets); }
+    for (int s = 0; s < kStages; ++s) { mbar_init(smem_u32(&bars->full[s]), 2); mbar_init(smem_u32(&bars->empty[s]), 1); }
+    for (int s = 0; s < 2; ++s) { mbar_init(smem_u32(&bars->tmem_full[s]), 1); mbar_init(smem_u32(&bars->tmem_empty[s]), 8 * kEpiSets); }
     mbar_fence_init();
   }
-  if (warp == 1) { tmem_alloc_pair(smem_u32(tmem_slot), kTmemCols); tmem_relinquish_pair(); }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
+  const uint32_t tmem_base = tmem_setup<true>(warp, &bars->tmem_slot, kTmemCols);
 
   if (warp == 0) {
     if (lane == 0) {
@@ -80,10 +76,8 @@ dh_gemm_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ 
         const int k0 = hb * 256 + rank * 128;            // this CTA's hidden units
         for (int kc = 0; kc < nk; ++kc, ++it) {
           const uint32_t s = it % kStages, ph = (it / kStages) & 1;
-          mbar_wait(empty + 8 * s, ph ^ 1);
-          const uint32_t full_leader = mapa_shared(full + 8 * s, 0);
-          if (rank == 0) mbar_expect_tx(full + 8 * s, 2 * (kBytesA + kBytesB));
-          else mbar_arrive_cluster(full_leader);
+          mbar_wait(smem_u32(&bars->empty[s]), ph ^ 1);
+          const uint32_t full_leader = pair_stage_arrive(smem_u32(&bars->full[s]), rank, 2 * (kBytesA + kBytesB));
           tma_load_2d_pair(a_ring + s * kBytesA, &tmWmn, full_leader, k0, kc * kBK);
           tma_load_2d_pair(a_ring + s * kBytesA + 8192, &tmWmn, full_leader, k0 + 64, kc * kBK);
           tma_load_2d_pair(b_ring + s * kBytesB, &tmG, full_leader, kc * kBK, cb * 256 + rank * 128);
@@ -96,25 +90,20 @@ dh_gemm_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ 
     uint32_t it = 0, ic = 0;
     for (int item = pair; item < nitems; item += npairs, ++ic) {
       const uint32_t acc = ic & 1, accph = (ic >> 1) & 1;
-      mbar_wait(tmem_empty + 8 * acc, accph ^ 1);
+      mbar_wait(smem_u32(&bars->tmem_empty[acc]), accph ^ 1);
       tc_fence_after();
       for (int kc = 0; kc < nk; ++kc, ++it) {
         const uint32_t s = it % kStages, ph = (it / kStages) & 1;
-        mbar_wait(full + 8 * s, ph);
+        mbar_wait(smem_u32(&bars->full[s]), ph);
         tc_fence_after();
         if (lane == 0) {
-          const uint32_t a_addr = a_ring + s * kBytesA, b_addr = b_ring + s * kBytesB;
-#pragma unroll
-          for (int k = 0; k < kBK / 16; ++k) {
-            const uint64_t ad = make_smem_desc(a_addr + k * 2048, 8192, 1024);   // MN-major (W^T)
-            const uint64_t bd = make_smem_desc(b_addr + k * 32, 16, 1024);       // K-major (g)
-            umma_f16_pair(tmem_base + acc * kBN, ad, bd, idesc, (kc | k) != 0);
-          }
-          umma_commit_pair(empty + 8 * s, 3);
+          // A = W^T (MN-major), B = g (K-major)
+          mma_kchunk<true, true, false>(tmem_base + acc * kBN, a_ring + s * kBytesA, b_ring + s * kBytesB, idesc, kc != 0);
+          umma_commit_pair(smem_u32(&bars->empty[s]), 3);
         }
         __syncwarp();
       }
-      if (lane == 0) umma_commit_pair(tmem_full + 8 * acc, 3);
+      if (lane == 0) umma_commit_pair(smem_u32(&bars->tmem_full[acc]), 3);
       __syncwarp();
     }
    }
@@ -133,7 +122,7 @@ dh_gemm_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ 
       const bool k_ok = k < p.H;
       const int kk = k_ok ? k : 0;
       const uint32_t acc = ic & 1, accph = (ic >> 1) & 1;
-      mbar_wait(tmem_full + 8 * acc, accph);
+      mbar_wait(smem_u32(&bars->tmem_full[acc]), accph);
       tc_fence_after();
 #pragma unroll 1
       for (int hs = eset * (4 / kEpiSets); hs < (eset + 1) * (4 / kEpiSets); ++hs) {   // this set's half-tiles of the item
@@ -150,7 +139,7 @@ dh_gemm_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ 
 #pragma unroll 1
         for (int q = 0; q < 2; ++q) {           // 32 columns = t-rows 8q .. 8q+7 x 4 u
           float v[32];
-          tmem_ld32(tmem_base + (static_cast<uint32_t>(lane_grp * 32) << 16) + acc * kBN + hs * 64 + q * 32, v);
+          tmem_ld32(tmem_lane_addr(tmem_base, lane_grp, acc * kBN + hs * 64 + q * 32), v);
           const int tb = tc.t0 + q * 8;         // first of this thread's 8 frames
           float ev[8];
           if (enc_vec && tb + 7 < p.T) {        // T-contiguous encoder view: the 8 frames are 32 contiguous bytes
@@ -205,14 +194,11 @@ dh_gemm_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ 
       }
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) mbar_arrive_cluster(mapa_shared(tmem_empty + 8 * acc, 0));
+      if (lane == 0) mbar_arrive_cluster(mapa_shared(smem_u32(&bars->tmem_empty[acc]), 0));
     }
   }
 
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  if (warp == 1) { tc_fence_after(); tmem_dealloc_pair(tmem_base, kTmemCols); }
+  tmem_teardown<true>(warp, tmem_base, kTmemCols);
 }
 
 }  // namespace
@@ -220,10 +206,10 @@ dh_gemm_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ 
 int launch_dh_gemm(const CUtensorMap& tmG, const CUtensorMap& tmWmn, const DhArgs& args, long long chunk_slots,
                    cudaStream_t stream) {
   ProfScope prof_(kProfDh, stream);
-  const size_t smem = SmemLayout::total + 1024;
-  RB_CUDA_CHECK(cudaFuncSetAttribute(dh_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const size_t smem = SmemLayout::total + kSmemAlign;
+  int pairs;
+  if (int rc = pair_kernel_setup(reinterpret_cast<const void*>(dh_gemm_kernel), kNumThreads, smem, &pairs)) return rc;
   const long long items = ((chunk_slots + 3) / 4) * ((args.Hp + 255) / 256);
-  const int pairs = max_cta_pairs(reinterpret_cast<const void*>(dh_gemm_kernel), kNumThreads, smem);
   const int grid = 2 * static_cast<int>(std::max<long long>(1, std::min<long long>(pairs, items)));
   dh_gemm_kernel<<<grid, kNumThreads, smem, stream>>>(tmG, tmWmn, args);
   RB_CUDA_CHECK(cudaGetLastError());

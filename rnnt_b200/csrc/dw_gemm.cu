@@ -10,8 +10,8 @@
 // run, their (otherwise idle) epilogue warps sum every A stage over its 64 cells.
 #include <algorithm>
 
-#include "common.cuh"
 #include "kernels.h"
+#include "tc_kernel.cuh"
 
 namespace rb {
 namespace {
@@ -30,20 +30,22 @@ struct SmemLayout {
   static constexpr int db_red = bars + 256;                  // 128 threads x 8 fp32 partial column sums
   static constexpr int total = db_red + 128 * 8 * 4;
 };
+// b_full: the leader's copy collects both CTAs' boxes (one arrival per CTA).  a_full stays local (the db reducers of each
+// CTA read their own A stage); the peer's MMA warp forwards "my A stage landed" to the leader's a_peer.
+struct Bars {
+  uint64_t b_full[kStagesB], b_empty[kStagesB], a_full[kStagesA], a_empty[kStagesA], tmem_full;
+  uint64_t a_peer[kStagesA];   // leader only: the peer CTA's A stage has landed
+  uint32_t tmem_slot;
+};
+static_assert(sizeof(Bars) <= SmemLayout::db_red - SmemLayout::bars, "barrier block overflows its region");
 
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kNumThreads, 1)
 dw_gemm_kernel(const __grid_constant__ CUtensorMap tmGmn, const __grid_constant__ CUtensorMap tmHmn, DwArgs p) {
   extern __shared__ uint8_t smem_raw[];
-  const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
-  const uint32_t b_ring = smem_base + SmemLayout::b_ring;
-  const uint32_t a_ring = smem_base + SmemLayout::a_ring;
-  const uint32_t bars = smem_base + SmemLayout::bars;
-  const uint32_t b_full = bars, b_empty = bars + 8 * kStagesB;
-  const uint32_t a_full = bars + 16 * kStagesB, a_empty = a_full + 8 * kStagesA;
-  const uint32_t tmem_full = a_empty + 8 * kStagesA;
-  const uint32_t a_peer = tmem_full + 8;    // leader only: the peer CTA's A stage has landed
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem_gen + SmemLayout::bars + 200);
+  const AlignedSmem smem = aligned_smem(smem_raw);
+  const uint32_t b_ring = smem.addr + SmemLayout::b_ring;
+  const uint32_t a_ring = smem.addr + SmemLayout::a_ring;
+  Bars* bars = reinterpret_cast<Bars*>(smem.ptr + SmemLayout::bars);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t rank = cluster_ctarank();
@@ -67,43 +69,34 @@ dw_gemm_kernel(const __grid_constant__ CUtensorMap tmGmn, const __grid_constant_
   if (threadIdx.x == 0) {
     tma_prefetch_desc(&tmGmn);
     tma_prefetch_desc(&tmHmn);
-    // b_full: the leader's copy collects both CTAs' boxes (one arrival per CTA).  a_full stays local (the db reducers of
-    // each CTA read their own A stage); the peer's MMA warp forwards "my A stage landed" to the leader's a_peer.
-    for (int s = 0; s < kStagesB; ++s) { mbar_init(b_full + 8 * s, 2); mbar_init(b_empty + 8 * s, 1); }
+    for (int s = 0; s < kStagesB; ++s) { mbar_init(smem_u32(&bars->b_full[s]), 2); mbar_init(smem_u32(&bars->b_empty[s]), 1); }
     for (int s = 0; s < kStagesA; ++s) {
-      mbar_init(a_full + 8 * s, 1);
-      mbar_init(a_empty + 8 * s, do_db ? 5 : 1);
-      mbar_init(a_peer + 8 * s, 1);
+      mbar_init(smem_u32(&bars->a_full[s]), 1);
+      mbar_init(smem_u32(&bars->a_empty[s]), do_db ? 5 : 1);
+      mbar_init(smem_u32(&bars->a_peer[s]), 1);
     }
-    mbar_init(tmem_full, 1);
+    mbar_init(smem_u32(&bars->tmem_full), 1);
     mbar_fence_init();
   }
-  if (warp == 1) { tmem_alloc_pair(smem_u32(tmem_slot), kTmemCols); tmem_relinquish_pair(); }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
+  const uint32_t tmem_base = tmem_setup<true>(warp, &bars->tmem_slot, kTmemCols);
 
   if (warp == 0) {
     if (lane == 0) {
       uint32_t ita = 0, itb = 0;
       for (int kc = k_begin; kc < k_end; ++kc, ++ita) {
         const uint32_t sa = ita % kStagesA, pha = (ita / kStagesA) & 1;
-        mbar_wait(a_empty + 8 * sa, pha ^ 1);
-        mbar_expect_tx(a_full + 8 * sa, kBytesA);
+        const uint32_t a_full = smem_u32(&bars->a_full[sa]);
+        mbar_wait(smem_u32(&bars->a_empty[sa]), pha ^ 1);
+        mbar_expect_tx(a_full, kBytesA);
 #pragma unroll
         for (int j = 0; j < 2; ++j)
-          tma_load_2d(a_ring + sa * kBytesA + j * 8192, &tmGmn, a_full + 8 * sa,
-                      (vt * 2 + rank) * kTileM + j * 64, kc * kBK);
+          tma_load_2d(a_ring + sa * kBytesA + j * 8192, &tmGmn, a_full, (vt * 2 + rank) * kTileM + j * 64, kc * kBK);
         // activation rows of this 64-cell chunk: ring rows, or the forward's residual buffer (indexed by half-tile)
         const int hrow = (p.h_map == 0) ? __ldg(p.sub_list + p.slot_begin + kc) * kHalfRows : kc * kBK;
         for (int blk = 0; blk < nblk; ++blk, ++itb) {
           const uint32_t sb = itb % kStagesB, phb = (itb / kStagesB) & 1;
-          mbar_wait(b_empty + 8 * sb, phb ^ 1);
-          const uint32_t full_leader = mapa_shared(b_full + 8 * sb, 0);
-          if (rank == 0) mbar_expect_tx(b_full + 8 * sb, 2 * kBytesB);
-          else mbar_arrive_cluster(full_leader);
+          mbar_wait(smem_u32(&bars->b_empty[sb]), phb ^ 1);
+          const uint32_t full_leader = pair_stage_arrive(smem_u32(&bars->b_full[sb]), rank, 2 * kBytesB);
 #pragma unroll
           for (int j = 0; j < 2; ++j)
             tma_load_2d_pair(b_ring + sb * kBytesB + j * 8192, &tmHmn, full_leader,
@@ -113,12 +106,11 @@ dw_gemm_kernel(const __grid_constant__ CUtensorMap tmGmn, const __grid_constant_
     }
   } else if (warp == 1 && rank != 0) {
     // peer CTA: tell the leader when this CTA's A stage is in shared memory
-    const uint32_t peer0 = mapa_shared(a_peer, 0);
     uint32_t ita = 0;
     for (int kc = k_begin; kc < k_end; ++kc, ++ita) {
       const uint32_t sa = ita % kStagesA, pha = (ita / kStagesA) & 1;
-      mbar_wait(a_full + 8 * sa, pha);
-      if (lane == 0) mbar_arrive_cluster(peer0 + 8 * sa);
+      mbar_wait(smem_u32(&bars->a_full[sa]), pha);
+      if (lane == 0) mbar_arrive_cluster(mapa_shared(smem_u32(&bars->a_peer[sa]), 0));
       __syncwarp();
     }
   } else if (warp == 1) {
@@ -126,28 +118,23 @@ dw_gemm_kernel(const __grid_constant__ CUtensorMap tmGmn, const __grid_constant_
     uint32_t ita = 0, itb = 0;
     for (int kc = k_begin; kc < k_end; ++kc, ++ita) {
       const uint32_t sa = ita % kStagesA, pha = (ita / kStagesA) & 1;
-      mbar_wait(a_full + 8 * sa, pha);
-      mbar_wait(a_peer + 8 * sa, pha);
+      mbar_wait(smem_u32(&bars->a_full[sa]), pha);
+      mbar_wait(smem_u32(&bars->a_peer[sa]), pha);
       for (int blk = 0; blk < nblk; ++blk, ++itb) {
         const uint32_t sb = itb % kStagesB, phb = (itb / kStagesB) & 1;
-        mbar_wait(b_full + 8 * sb, phb);
+        mbar_wait(smem_u32(&bars->b_full[sb]), phb);
         tc_fence_after();
         if (lane == 0) {
-          const uint32_t a_addr = a_ring + sa * kBytesA, b_addr = b_ring + sb * kBytesB;
-#pragma unroll
-          for (int k = 0; k < kBK / 16; ++k) {
-            const uint64_t ad = make_smem_desc(a_addr + k * 2048, 8192, 1024);   // MN-major
-            const uint64_t bd = make_smem_desc(b_addr + k * 2048, 8192, 1024);   // MN-major
-            umma_f16_pair(tmem_base + blk * kBN, ad, bd, idesc, (kc > k_begin) || (k != 0));
-          }
-          umma_commit_pair(b_empty + 8 * sb, 3);
+          mma_kchunk<true, true, true>(tmem_base + blk * kBN, a_ring + sa * kBytesA, b_ring + sb * kBytesB, idesc,
+                                       kc > k_begin);
+          umma_commit_pair(smem_u32(&bars->b_empty[sb]), 3);
         }
         __syncwarp();
       }
-      if (lane == 0) umma_commit_pair(a_empty + 8 * sa, 3);
+      if (lane == 0) umma_commit_pair(smem_u32(&bars->a_empty[sa]), 3);
       __syncwarp();
     }
-    if (lane == 0) umma_commit_pair(tmem_full, 3);
+    if (lane == 0) umma_commit_pair(smem_u32(&bars->tmem_full), 3);
     __syncwarp();
   } else {
     const int lane_grp = warp & 3;
@@ -168,7 +155,7 @@ dw_gemm_kernel(const __grid_constant__ CUtensorMap tmGmn, const __grid_constant_
       uint32_t ita = 0;
       for (int kc = k_begin; kc < k_end; ++kc, ++ita) {
         const uint32_t sa = ita % kStagesA, pha = (ita / kStagesA) & 1;
-        mbar_wait(a_full + 8 * sa, pha);
+        mbar_wait(smem_u32(&bars->a_full[sa]), pha);
         const uint32_t base = a_ring + sa * kBytesA + col_off;
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
@@ -186,9 +173,9 @@ dw_gemm_kernel(const __grid_constant__ CUtensorMap tmGmn, const __grid_constant_
           }
         }
         __syncwarp();
-        if (lane == 0) mbar_arrive(a_empty + 8 * sa);
+        if (lane == 0) mbar_arrive(smem_u32(&bars->a_empty[sa]));
       }
-      float* red = reinterpret_cast<float*>(smem_gen + SmemLayout::db_red);
+      float* red = reinterpret_cast<float*>(smem.ptr + SmemLayout::db_red);
 #pragma unroll
       for (int e = 0; e < 8; ++e) red[(rg * 16 + c) * 8 + e] = dacc[e];
       named_bar_sync(1, 128);
@@ -206,13 +193,13 @@ dw_gemm_kernel(const __grid_constant__ CUtensorMap tmGmn, const __grid_constant_
         }
       }
     }
-    mbar_wait(tmem_full, 0);
+    mbar_wait(smem_u32(&bars->tmem_full), 0);
     tc_fence_after();
     for (int c32 = 0; c32 < nblk * (kBN / 32); ++c32) {
       const int col0 = ht * 2 * kBN + c32 * 32;
       if (col0 >= p.H) break;
       float acc[32];
-      tmem_ld32(tmem_base + (static_cast<uint32_t>(lane_grp * 32) << 16) + c32 * 32, acc);
+      tmem_ld32(tmem_lane_addr(tmem_base, lane_grp, c32 * 32), acc);
       tmem_ld_wait();
       if (v < p.V && p.dW_fx) {          // deterministic mode: order-independent fixed-point accumulation
         long long* dst = p.dW_fx + static_cast<long long>(v) * p.H + col0;
@@ -236,10 +223,7 @@ dw_gemm_kernel(const __grid_constant__ CUtensorMap tmGmn, const __grid_constant_
     }
   }
 
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  if (warp == 1) { tc_fence_after(); tmem_dealloc_pair(tmem_base, kTmemCols); }
+  tmem_teardown<true>(warp, tmem_base, kTmemCols);
 }
 
 }  // namespace
@@ -247,12 +231,12 @@ dw_gemm_kernel(const __grid_constant__ CUtensorMap tmGmn, const __grid_constant_
 int launch_dw_gemm(const CUtensorMap& tmGmn, const CUtensorMap& tmHmn, const DwArgs& args_in, long long chunk_slots,
                    cudaStream_t stream) {
   ProfScope prof_(kProfDw, stream);
-  const size_t smem = SmemLayout::total + 1024;
-  RB_CUDA_CHECK(cudaFuncSetAttribute(dw_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const size_t smem = SmemLayout::total + kSmemAlign;
+  int pairs;
+  if (int rc = pair_kernel_setup(reinterpret_cast<const void*>(dw_gemm_kernel), kNumThreads, smem, &pairs)) return rc;
   DwArgs args = args_in;
   const int nblk_total = (args.Hp + kBN - 1) / kBN;
   const int out_blocks = (args.Vp / (2 * kTileM)) * ((nblk_total + 1) / 2);   // 256 x 512 blocks of dW, one pair each
-  const int pairs = max_cta_pairs(reinterpret_cast<const void*>(dw_gemm_kernel), kNumThreads, smem);
   const long long kchunks = chunk_slots;
   args.ksplit = static_cast<int>(std::max<long long>(1, std::min<long long>(pairs / std::max(1, out_blocks), kchunks)));
   const int grid = 2 * out_blocks * args.ksplit;

@@ -68,18 +68,23 @@ int device_sm_count() {
   return cached[dev];
 }
 
-int max_cta_pairs(const void* kernel, int threads, size_t smem) {
+int pair_kernel_setup(const void* kernel, int threads, size_t smem, int* pairs) {
+  RB_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   // keyed on (device, kernel); a handful of kernels -> linear scan
   struct Entry { int dev; const void* fn; int pairs; };
   static std::mutex mu;
   static std::vector<Entry> cache;
   int dev = 0;
   const int fallback = device_sm_count() / 2;
-  if (cudaGetDevice(&dev) != cudaSuccess) return fallback;
+  *pairs = fallback;
+  if (cudaGetDevice(&dev) != cudaSuccess) return 0;
   {
     std::lock_guard<std::mutex> lk(mu);
     for (const Entry& e : cache)
-      if (e.dev == dev && e.fn == kernel) return e.pairs;
+      if (e.dev == dev && e.fn == kernel) {
+        *pairs = e.pairs;
+        return 0;
+      }
   }
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(2 * fallback);
@@ -94,10 +99,10 @@ int max_cta_pairs(const void* kernel, int threads, size_t smem) {
     cudaGetLastError();
     n = fallback;
   }
-  n = n < fallback ? n : fallback;
+  *pairs = n < fallback ? n : fallback;
   std::lock_guard<std::mutex> lk(mu);
-  cache.push_back({dev, kernel, n});
-  return n;
+  cache.push_back({dev, kernel, *pairs});
+  return 0;
 }
 
 namespace {

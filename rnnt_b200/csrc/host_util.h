@@ -33,9 +33,10 @@ int make_tmap_2d(CUtensorMap* out, const void* gptr, int elem_bytes, uint64_t in
                  uint64_t row_stride_bytes, uint32_t box_inner, uint32_t box_outer);
 
 int device_sm_count();
-// Number of 2-CTA clusters (CTA pairs, one CTA per SM) of `kernel` that can be co-resident on the current device; the
-// persistent pair kernels launch exactly that many.  The kernel's max-dynamic-smem attribute must already be set.
-int max_cta_pairs(const void* kernel, int threads, size_t smem);
+// Sets `kernel`'s maximum dynamic shared memory to `smem` bytes and stores in *pairs the number of its 2-CTA clusters
+// (CTA pairs, one CTA per SM) that can be co-resident on the current device; the persistent pair kernels launch at most
+// that many.  Returns 0 or the CUDA error of setting the attribute.
+int pair_kernel_setup(const void* kernel, int threads, size_t smem, int* pairs);
 
 // Opt-in per-kernel-family timing (CUDA events on the launch stream) and launch counting; used by bench.py to
 // compute the live roofline numbers.  Off by default: the hot path then records nothing.

@@ -27,8 +27,8 @@
 //             | 10-17 (PRODUCE only) activation producers
 #include <algorithm>
 
-#include "common.cuh"
 #include "kernels.h"
+#include "tc_kernel.cuh"
 
 namespace rb {
 
@@ -62,6 +62,11 @@ struct SmemLayout {
   static constexpr int total_noprod = g_stage + kNumEpiWarps * 32 * 64;
   static constexpr int total = enc_stage + 2 * 2 * kTileT * kBK * 4;
 };
+struct Bars {
+  uint64_t full[kStages], empty[kStages], tmem_full[2], tmem_empty[2], h_ready[2], tile_done[2];
+  uint32_t tmem_slot;
+};
+static_assert(sizeof(Bars) <= SmemLayout::bias_stage - SmemLayout::bars, "barrier block overflows its region");
 
 __device__ __forceinline__ void fence_proxy_async_all() { asm volatile("fence.proxy.async;" ::: "memory"); }
 
@@ -81,7 +86,6 @@ __device__ __forceinline__ float pick32(const float (&v)[32], int idx) {
 
 }  // namespace
 
-size_t joint_gemm_smem_bytes() { return SmemLayout::total + 1024; }
 int joint_gemm_scratch_tiles(int grid) { return grid * kScratchSlots; }
 
 // MODE 0 = forward (lse + gather), 1 = backward (gradient ring); PRODUCE: activation producer warps present;
@@ -91,17 +95,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(PRODUCE ? kThreadsPr
 joint_gemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmH,
                   const __grid_constant__ CUtensorMap tmH2, JointArgs p) {
   extern __shared__ uint8_t smem_raw[];
-  const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
+  const AlignedSmem smem = aligned_smem(smem_raw);
   using SL = SmemLayout;
 
-  const uint32_t ring = smem_base + SL::ring;
-  const uint32_t bars = smem_base + SL::bars;
-  // barrier map (8 bytes each)
-  const uint32_t full = bars, empty = bars + 8 * kStages;
-  const uint32_t tmem_full = bars + 16 * kStages, tmem_empty = tmem_full + 16;
-  const uint32_t h_ready = tmem_empty + 16, tile_done = h_ready + 16;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem_gen + SL::bars + 200);
+  const uint32_t ring = smem.addr + SL::ring;
+  Bars* bars = reinterpret_cast<Bars*>(smem.ptr + SL::bars);
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -133,27 +131,20 @@ joint_gemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant
     tma_prefetch_desc(&tmH);
     tma_prefetch_desc(&tmH2);
     for (int s = 0; s < kStages; ++s) {
-      mbar_init(full + 8 * s, 2);        // leader's copy: one expect_tx arrival per CTA of the pair
-      mbar_init(empty + 8 * s, 1);
+      mbar_init(smem_u32(&bars->full[s]), 2);        // leader's copy: one expect_tx arrival per CTA of the pair
+      mbar_init(smem_u32(&bars->empty[s]), 1);
     }
     for (int a = 0; a < 2; ++a) {
-      mbar_init(tmem_full + 8 * a, 1);
-      mbar_init(tmem_empty + 8 * a, kNumEpiWarps);   // leader's copy: 4 warps of set a in each CTA
-      mbar_init(h_ready + 8 * a, kNumProdWarps);
-      mbar_init(tile_done + 8 * a, 1);
+      mbar_init(smem_u32(&bars->tmem_full[a]), 1);
+      mbar_init(smem_u32(&bars->tmem_empty[a]), kNumEpiWarps);   // leader's copy: 4 warps of set a in each CTA
+      mbar_init(smem_u32(&bars->h_ready[a]), kNumProdWarps);
+      mbar_init(smem_u32(&bars->tile_done[a]), 1);
     }
     mbar_fence_init();
   }
-  if (warp == 1) {
-    tmem_alloc_pair(smem_u32(tmem_slot), kTmemCols);
-    tmem_relinquish_pair();
-  }
-  const LenTables lt = stage_len_tables(reinterpret_cast<int*>(smem_gen + SL::len_tab), p.tile_off, p.T_len, p.U_len, p.B);
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();      // barrier inits and TMEM allocation of both CTAs are visible before any remote arrive
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
+  tmem_alloc<true>(warp, &bars->tmem_slot, kTmemCols);
+  const LenTables lt = stage_len_tables(reinterpret_cast<int*>(smem.ptr + SL::len_tab), p.tile_off, p.T_len, p.U_len, p.B);
+  const uint32_t tmem_base = tmem_publish<true>(&bars->tmem_slot);
 
 // this CTA's units: q = base + rank for base = 2 * (pair + i * npairs); a pair whose second unit is past the end still
 // runs (the leader's MMA spans both CTAs) with that CTA's outputs suppressed
@@ -172,18 +163,17 @@ joint_gemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant
           hrow[sh] = hid >= 0 ? h_row0(q, sh, hid, cnt) : 0;     // nothing there: any resident rows (results unused)
         }
         if (PRODUCE) {
-          mbar_wait(h_ready + 8 * (cnt & 1), (cnt >> 1) & 1);
+          mbar_wait(smem_u32(&bars->h_ready[cnt & 1]), (cnt >> 1) & 1);
           fence_proxy_async_all();   // the producers' generic-proxy global stores -> TMA (async proxy) reads
         }
         for (int pass = 0; pass < npass; ++pass) {
           for (int kc = 0; kc < nk; ++kc, ++it) {
             const uint32_t s = it % kStages, ph = (it / kStages) & 1;
-            mbar_wait(empty + 8 * s, ph ^ 1);
-            const uint32_t full_leader = mapa_shared(full + 8 * s, 0);
+            mbar_wait(smem_u32(&bars->empty[s]), ph ^ 1);
             // (diagnostics: dbg bit 32 skips every other W load -- stale operands, used to measure what L2 traffic costs)
             const bool skipw = (p.dbg & 32) && (it & 1);
-            if (rank == 0) mbar_expect_tx(full + 8 * s, 2 * kStageBytes - (skipw ? 2 * kBytesB : 0));   // both CTAs' boxes
-            else mbar_arrive_cluster(full_leader);
+            const uint32_t full_leader =
+                pair_stage_arrive(smem_u32(&bars->full[s]), rank, 2 * kStageBytes - (skipw ? 2 * kBytesB : 0));
             if (!skipw)
               tma_load_2d_pair(ring + s * kStageBytes, &tmW, full_leader, kc * kBK, pass * kBN + rank * (kBN / 2));
             if (hrow[1] == hrow[0] + kHalfRows) {     // both halves of one tile / adjacent ring slots: one 128-row box
@@ -205,29 +195,24 @@ joint_gemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant
     RB_TILE_LOOP(cnt) {
       for (int pass = 0; pass < npass; ++pass, ++pc) {
         const uint32_t acc = pc & 1;
-        mbar_wait(tmem_empty + 8 * acc, ((pc >> 1) & 1) ^ 1);
+        mbar_wait(smem_u32(&bars->tmem_empty[acc]), ((pc >> 1) & 1) ^ 1);
         tc_fence_after();
         for (int kc = 0; kc < nk; ++kc, ++it) {
           const uint32_t s = it % kStages, ph = (it / kStages) & 1;
-          mbar_wait(full + 8 * s, ph);
+          mbar_wait(smem_u32(&bars->full[s]), ph);
           tc_fence_after();
           if (lane == 0) {
             const uint32_t b_addr = ring + s * kStageBytes, a_addr = b_addr + kBytesB;
-#pragma unroll
-            for (int k = 0; k < kBK / 16; ++k) {
-              const uint64_t ad = make_smem_desc(a_addr + k * 32, 16, 1024);
-              const uint64_t bd = make_smem_desc(b_addr + k * 32, 16, 1024);
-              umma_f16_pair(tmem_base + acc * kBN, ad, bd, idesc, (kc | k) != 0);
-            }
-            umma_commit_pair(empty + 8 * s, 3);
+            mma_kchunk<true, false, false>(tmem_base + acc * kBN, a_addr, b_addr, idesc, kc != 0);
+            umma_commit_pair(smem_u32(&bars->empty[s]), 3);
           }
           __syncwarp();
         }
-        if (lane == 0) umma_commit_pair(tmem_full + 8 * acc, 3);
+        if (lane == 0) umma_commit_pair(smem_u32(&bars->tmem_full[acc]), 3);
         __syncwarp();
       }
       if (PRODUCE) {
-        if (lane == 0) umma_commit_pair(tile_done + 8 * (cnt & 1), 3);   // both tiles' activation rows are consumed
+        if (lane == 0) umma_commit_pair(smem_u32(&bars->tile_done[cnt & 1]), 3);   // both tiles' activation rows are consumed
         __syncwarp();
       }
     }
@@ -239,8 +224,8 @@ joint_gemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant
     const int row = lane_grp * 32 + lane;
     const int sub = row >> 6;                     // which of the unit's two half-tiles this row belongs to
     const int ti = (row & 63) >> 2, ui = row & 3;
-    float4* xchg = reinterpret_cast<float4*>(smem_gen + SL::xchg);
-    const uint32_t tmem_empty_leader = mapa_shared(tmem_empty + 8 * eset, 0);
+    float4* xchg = reinterpret_cast<float4*>(smem.ptr + SL::xchg);
+    const uint32_t tmem_empty_leader = mapa_shared(smem_u32(&bars->tmem_empty[eset]), 0);
     uint32_t pc = 0, tcount = 0;
     RB_TILE_LOOP(tcount) {
       const int q = base_ + rank;
@@ -280,19 +265,19 @@ joint_gemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant
         // KB next to 220 KB of shared memory and the producers stream through it, so per-chunk __ldg's of the bias were
         // L2 round trips on the drain's critical path).  Buffer (pc >> 1) & 1 of this set: the set's barrier of pass
         // j orders every warp's reads of pass j-1 before any write of pass j+1.
-        float* bias_s = reinterpret_cast<float*>(smem_gen + SL::bias_stage) + (eset * 2 + ((pc >> 1) & 1)) * kBN;
+        float* bias_s = reinterpret_cast<float*>(smem.ptr + SL::bias_stage) + (eset * 2 + ((pc >> 1) & 1)) * kBN;
         {
           const int i2 = (lane_grp * 32 + lane) * 2;
           *reinterpret_cast<float2*>(bias_s + i2) = __ldg(reinterpret_cast<const float2*>(p.bias2 + pass * kBN + i2));
         }
         named_bar_sync(1 + eset, 128);
-        mbar_wait(tmem_full + 8 * eset, (pc >> 1) & 1);
+        mbar_wait(smem_u32(&bars->tmem_full[eset]), (pc >> 1) & 1);
         tc_fence_after();
         const int nchunk = ((p.dbg & 1) || !mine) ? 0 : (kBN / 32);
         for (int c32 = 0; c32 < nchunk; ++c32) {
           const int col0 = pass * kBN + c32 * 32;  // global column of v[0]
           float v[32];
-          tmem_ld32(tmem_base + (static_cast<uint32_t>(lane_grp * 32) << 16) + eset * kBN + c32 * 32, v);
+          tmem_ld32(tmem_lane_addr(tmem_base, lane_grp, eset * kBN + c32 * 32), v);
           tmem_ld_wait();
           const float4* b4 = reinterpret_cast<const float4*>(bias_s + c32 * 32);
 #pragma unroll
@@ -346,7 +331,7 @@ joint_gemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant
               // thread = row writes its 64 bytes (16-byte chunk c at c ^ (row >> 1), conflict-free), the one-hot columns
               // are patched in place, then 4 lanes per row store 64 contiguous bytes -- 8 full-sector segments per
               // instruction instead of 32 scattered 16-byte ones.
-              uint8_t* gs = smem_gen + SL::g_stage + (warp - kFirstEpiWarp) * (32 * 64);
+              uint8_t* gs = smem.ptr + SL::g_stage + (warp - kFirstEpiWarp) * (32 * 64);
               __syncwarp();                                     // the previous chunk's read-back is complete
 #pragma unroll
               for (int q = 0; q < 4; ++q)
@@ -420,15 +405,15 @@ joint_gemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant
     constexpr bool t_major = TMAJOR;
     const bool vec_ok = ((p.enc_sh | p.enc_sb) & 3) == 0;     // 16-byte aligned rows of the (B,H,T) tensor
     const int wl = rg & 3, kk = lane >> 2, tq4 = lane & 3;    // T-major fetch: k rows 16 wl + 2 kk, + 1; frames 4 tq4 .. +3
-    float* stage = reinterpret_cast<float*>(smem_gen + SL::enc_stage) + sub * (2 * kTileT * kBK);
+    float* stage = reinterpret_cast<float*>(smem.ptr + SL::enc_stage) + sub * (2 * kTileT * kBK);
     uint32_t cnt = 0, cc = 0;                                 // cc: running chunk counter = stage buffer parity
     RB_TILE_LOOP(cnt) {
       const int q = base_ + rank;
       const int hid = half_id(q, sub);
       if (hid < 0) {            // nothing to produce for this half (uniform over its 4 warps): keep the barrier protocol
-        if (cnt >= 2) mbar_wait(tile_done + 8 * (cnt & 1), ((cnt >> 1) - 1) & 1);
+        if (cnt >= 2) mbar_wait(smem_u32(&bars->tile_done[cnt & 1]), ((cnt >> 1) - 1) & 1);
         __syncwarp();
-        if (lane == 0) mbar_arrive(h_ready + 8 * (cnt & 1));
+        if (lane == 0) mbar_arrive(smem_u32(&bars->h_ready[cnt & 1]));
         continue;
       }
       const TileCoord tc = decode_half(lt.tile_off, lt.T_len, lt.U_len, p.B, p.T, p.U1, hid);
@@ -498,7 +483,7 @@ joint_gemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant
       load_pred(0, p_cur);
       // stay at most two units ahead of the tensor pipe: unit cnt-2 must be fully consumed (also keeps the
       // two-phase h_ready / tile_done barriers and the 4-slot scratch unambiguous)
-      if (cnt >= 2) mbar_wait(tile_done + 8 * (cnt & 1), ((cnt >> 1) - 1) & 1);
+      if (cnt >= 2) mbar_wait(smem_u32(&bars->tile_done[cnt & 1]), ((cnt >> 1) - 1) & 1);
       // row of (t-row tq + i, u = uq + j) inside the half-tile: (tq + i) * 4 + uq + j
       __half* out_base = p.h_out + static_cast<long long>(row0 + tq * 4 + uq) * p.Hp + 8 * c;
       for (int kc = 0; kc < nk; ++kc, ++cc) {
@@ -534,43 +519,32 @@ joint_gemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant
       }
       fence_proxy_async_all();   // generic-proxy global writes -> visible to the loader's TMA reads
       __syncwarp();
-      if (lane == 0) mbar_arrive(h_ready + 8 * (cnt & 1));
+      if (lane == 0) mbar_arrive(smem_u32(&bars->h_ready[cnt & 1]));
     }
   }
 
 #undef RB_TILE_LOOP
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();      // the peer may still be signalling this CTA's barriers / reading its shared memory
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc_pair(tmem_base, kTmemCols);
-  }
+  tmem_teardown<true>(warp, tmem_base, kTmemCols);
 }
 
 int launch_joint_gemm(int mode, bool produce, const CUtensorMap& tmW, const CUtensorMap& tmH, const CUtensorMap& tmH2,
                       const JointArgs& args, long long max_slots, cudaStream_t stream) {
   ProfScope prof_(mode == 0 ? kProfJointF : kProfJointG, stream);
-  const size_t smem = (produce ? SmemLayout::total : SmemLayout::total_noprod) + 1024;
+  RB_REQUIRE(mode != 0 || produce, -30, "forward joint kernel always produces the activations");
+  const bool t_major = produce && args.enc_sh != 1;
+  void (*const kernel)(CUtensorMap, CUtensorMap, CUtensorMap, JointArgs) =
+      !produce    ? joint_gemm_kernel<1, false, false>
+      : mode == 0 ? (t_major ? joint_gemm_kernel<0, true, true> : joint_gemm_kernel<0, true, false>)
+                  : (t_major ? joint_gemm_kernel<1, true, true> : joint_gemm_kernel<1, true, false>);
+  const int threads = produce ? kThreadsProd : kThreadsNoProd;
+  const size_t smem = (produce ? SmemLayout::total : SmemLayout::total_noprod) + kSmemAlign;
+  int pairs;
+  if (int rc = pair_kernel_setup(reinterpret_cast<const void*>(kernel), threads, smem, &pairs)) return rc;
   const long long want_pairs = std::max<long long>(1, (max_slots + 3) / 4);   // 2 slots per CTA, 2 CTAs per pair
-#define RB_LAUNCH_JG(M, P, TM)                                                                                     \
-  do {                                                                                                             \
-    RB_CUDA_CHECK(cudaFuncSetAttribute(joint_gemm_kernel<M, P, TM>, cudaFuncAttributeMaxDynamicSharedMemorySize,   \
-                                       (int)smem));                                                                \
-    const int grid = 2 * static_cast<int>(std::min<long long>(max_cta_pairs(reinterpret_cast<const void*>(joint_gemm_kernel<M, P, TM>), P ? kThreadsProd : kThreadsNoProd, smem), want_pairs));                 \
-    if (args.dbg & 8) fprintf(stderr, "rnnt_b200: joint gemm mode %d produce %d t-major %d grid %d\n", M, (int)P, (int)TM, grid); \
-    joint_gemm_kernel<M, P, TM><<<grid, P ? kThreadsProd : kThreadsNoProd, smem, stream>>>(tmW, tmH, tmH2, args);            \
-  } while (0)
-  const bool t_major = args.enc_sh != 1;
-  if (mode == 0) {
-    RB_REQUIRE(produce, -30, "forward joint kernel always produces the activations");
-    if (t_major) RB_LAUNCH_JG(0, true, true); else RB_LAUNCH_JG(0, true, false);
-  } else if (produce) {
-    if (t_major) RB_LAUNCH_JG(1, true, true); else RB_LAUNCH_JG(1, true, false);
-  } else {
-    RB_LAUNCH_JG(1, false, false);
-  }
-#undef RB_LAUNCH_JG
+  const int grid = 2 * static_cast<int>(std::min<long long>(pairs, want_pairs));
+  if (args.dbg & 8)
+    fprintf(stderr, "rnnt_b200: joint gemm mode %d produce %d t-major %d grid %d\n", mode, (int)produce, (int)t_major, grid);
+  kernel<<<grid, threads, smem, stream>>>(tmW, tmH, tmH2, args);
   RB_CUDA_CHECK(cudaGetLastError());
   return 0;
 }

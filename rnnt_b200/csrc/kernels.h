@@ -101,7 +101,6 @@ struct DecodeArgs {
 size_t greedy_decode_scratch_bytes(int B, int H, int V, int E);
 int launch_greedy_decode(DecodeArgs a, float* scratch, cudaStream_t stream);
 
-size_t joint_gemm_smem_bytes();
 int joint_gemm_scratch_tiles(int grid);   // tiles of per-CTA activation scratch the forward needs when h_map == 2
 // tmW: 64(k) x 128(v) boxes (each CTA of a pair loads half of a 256-class block); tmH / tmH2: 64(k) x 64 / 128 (row)
 // boxes of the activation buffer (one half-tile / two adjacent ones); max_slots bounds the work-list slots of this launch

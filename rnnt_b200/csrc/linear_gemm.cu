@@ -14,8 +14,8 @@
 // bench shape), so the kernel favours generality (any M, N; K % 8 == 0) over the last 20 % of tensor-pipe rate.
 #include <algorithm>
 
-#include "common.cuh"
 #include "kernels.h"
+#include "tc_kernel.cuh"
 
 namespace rb {
 namespace {
@@ -32,6 +32,11 @@ struct LinSmem {
   static constexpr int bars = b_ring + kLinStages * kLinBytes;
   static constexpr int total = bars + 256;
 };
+struct LinBars {
+  uint64_t full[kLinStages], empty[kLinStages], tmem_full[2], tmem_empty[2];
+  uint32_t tmem_slot;
+};
+static_assert(sizeof(LinBars) <= LinSmem::total - LinSmem::bars, "barrier block overflows its region");
 
 struct LinArgs {
   int M, N, K;             // D is M x N, contraction length K
@@ -46,13 +51,9 @@ template <bool A_MN, bool B_MN>
 __global__ void __launch_bounds__(kLinThreads, 1)
 linear_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, LinArgs p) {
   extern __shared__ uint8_t smem_raw[];
-  const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
-  const uint32_t a_ring = smem_base + LinSmem::a_ring, b_ring = smem_base + LinSmem::b_ring;
-  const uint32_t bars = smem_base + LinSmem::bars;
-  const uint32_t full = bars, empty = bars + 8 * kLinStages;
-  const uint32_t tmem_full = bars + 16 * kLinStages, tmem_empty = tmem_full + 16;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem_gen + LinSmem::bars + 200);
+  const AlignedSmem smem = aligned_smem(smem_raw);
+  const uint32_t a_ring = smem.addr + LinSmem::a_ring, b_ring = smem.addr + LinSmem::b_ring;
+  LinBars* bars = reinterpret_cast<LinBars*>(smem.ptr + LinSmem::bars);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
   const int tm = (p.M + kLinTile - 1) / kLinTile, tn = (p.N + kLinTile - 1) / kLinTile;
@@ -62,15 +63,11 @@ linear_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
   if (threadIdx.x == 0) {
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmB);
-    for (int s = 0; s < kLinStages; ++s) { mbar_init(full + 8 * s, 1); mbar_init(empty + 8 * s, 1); }
-    for (int a = 0; a < 2; ++a) { mbar_init(tmem_full + 8 * a, 1); mbar_init(tmem_empty + 8 * a, 4); }
+    for (int s = 0; s < kLinStages; ++s) { mbar_init(smem_u32(&bars->full[s]), 1); mbar_init(smem_u32(&bars->empty[s]), 1); }
+    for (int a = 0; a < 2; ++a) { mbar_init(smem_u32(&bars->tmem_full[a]), 1); mbar_init(smem_u32(&bars->tmem_empty[a]), 4); }
     mbar_fence_init();
   }
-  if (warp == 1) { tmem_alloc(smem_u32(tmem_slot), kLinTmemCols); tmem_relinquish(); }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
+  const uint32_t tmem_base = tmem_setup<false>(warp, &bars->tmem_slot, kLinTmemCols);
 
   // item -> (m tile, n tile, k range); consecutive items share the B tile column (n fastest would thrash A instead)
   auto decode = [&](int item, int& m0, int& n0, int& kc0, int& kc1) {
@@ -90,19 +87,20 @@ linear_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
         decode(item, m0, n0, kc0, kc1);
         for (int kc = kc0; kc < kc1; ++kc, ++it) {
           const uint32_t s = it % kLinStages, ph = (it / kLinStages) & 1;
-          mbar_wait(empty + 8 * s, ph ^ 1);
-          mbar_expect_tx(full + 8 * s, 2 * kLinBytes);
+          const uint32_t full = smem_u32(&bars->full[s]);
+          mbar_wait(smem_u32(&bars->empty[s]), ph ^ 1);
+          mbar_expect_tx(full, 2 * kLinBytes);
           if (A_MN) {          // [k][m] storage: two boxes of 64 (m) x 64 (k rows)
-            tma_load_2d(a_ring + s * kLinBytes, &tmA, full + 8 * s, m0, kc * kBK);
-            tma_load_2d(a_ring + s * kLinBytes + 8192, &tmA, full + 8 * s, m0 + 64, kc * kBK);
+            tma_load_2d(a_ring + s * kLinBytes, &tmA, full, m0, kc * kBK);
+            tma_load_2d(a_ring + s * kLinBytes + 8192, &tmA, full, m0 + 64, kc * kBK);
           } else {             // [m][k] storage: one box of 64 (k) x 128 (m rows)
-            tma_load_2d(a_ring + s * kLinBytes, &tmA, full + 8 * s, kc * kBK, m0);
+            tma_load_2d(a_ring + s * kLinBytes, &tmA, full, kc * kBK, m0);
           }
           if (B_MN) {
-            tma_load_2d(b_ring + s * kLinBytes, &tmB, full + 8 * s, n0, kc * kBK);
-            tma_load_2d(b_ring + s * kLinBytes + 8192, &tmB, full + 8 * s, n0 + 64, kc * kBK);
+            tma_load_2d(b_ring + s * kLinBytes, &tmB, full, n0, kc * kBK);
+            tma_load_2d(b_ring + s * kLinBytes + 8192, &tmB, full, n0 + 64, kc * kBK);
           } else {
-            tma_load_2d(b_ring + s * kLinBytes, &tmB, full + 8 * s, kc * kBK, n0);
+            tma_load_2d(b_ring + s * kLinBytes, &tmB, full, kc * kBK, n0);
           }
         }
       }
@@ -114,25 +112,20 @@ linear_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
       int m0, n0, kc0, kc1;
       decode(item, m0, n0, kc0, kc1);
       const uint32_t acc = ic & 1;
-      mbar_wait(tmem_empty + 8 * acc, ((ic >> 1) & 1) ^ 1);
+      mbar_wait(smem_u32(&bars->tmem_empty[acc]), ((ic >> 1) & 1) ^ 1);
       tc_fence_after();
       for (int kc = kc0; kc < kc1; ++kc, ++it) {
         const uint32_t s = it % kLinStages, ph = (it / kLinStages) & 1;
-        mbar_wait(full + 8 * s, ph);
+        mbar_wait(smem_u32(&bars->full[s]), ph);
         tc_fence_after();
         if (lane == 0) {
-          const uint32_t a_addr = a_ring + s * kLinBytes, b_addr = b_ring + s * kLinBytes;
-#pragma unroll
-          for (int k = 0; k < kBK / 16; ++k) {
-            const uint64_t ad = A_MN ? make_smem_desc(a_addr + k * 2048, 8192, 1024) : make_smem_desc(a_addr + k * 32, 16, 1024);
-            const uint64_t bd = B_MN ? make_smem_desc(b_addr + k * 2048, 8192, 1024) : make_smem_desc(b_addr + k * 32, 16, 1024);
-            umma_f16(tmem_base + acc * kLinTile, ad, bd, idesc, (kc > kc0) || (k != 0));
-          }
-          umma_commit(empty + 8 * s);
+          mma_kchunk<false, A_MN, B_MN>(tmem_base + acc * kLinTile, a_ring + s * kLinBytes, b_ring + s * kLinBytes, idesc,
+                                        kc > kc0);
+          umma_commit(smem_u32(&bars->empty[s]));
         }
         __syncwarp();
       }
-      if (lane == 0) umma_commit(tmem_full + 8 * acc);   // (an empty k range never happens: ksplit <= number of k chunks)
+      if (lane == 0) umma_commit(smem_u32(&bars->tmem_full[acc]));   // (an empty k range never happens: ksplit <= number of k chunks)
       __syncwarp();
     }
   } else {
@@ -143,7 +136,7 @@ linear_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
       int m0, n0, kc0, kc1;
       decode(item, m0, n0, kc0, kc1);
       const uint32_t acc = ic & 1;
-      mbar_wait(tmem_full + 8 * acc, (ic >> 1) & 1);
+      mbar_wait(smem_u32(&bars->tmem_full[acc]), (ic >> 1) & 1);
       tc_fence_after();
       const int m = m0 + row;
 #pragma unroll 1
@@ -151,7 +144,7 @@ linear_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
         const int col0 = n0 + c32 * 32;
         if (col0 >= p.N) break;                  // uniform
         float v[32];
-        tmem_ld32(tmem_base + (static_cast<uint32_t>(lane_grp * 32) << 16) + acc * kLinTile + c32 * 32, v);
+        tmem_ld32(tmem_lane_addr(tmem_base, lane_grp, acc * kLinTile + c32 * 32), v);
         tmem_ld_wait();
         if (m < p.M) {
           if (p.out_fx) {
@@ -189,13 +182,11 @@ linear_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
       }
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) mbar_arrive(tmem_empty + 8 * acc);
+      if (lane == 0) mbar_arrive(smem_u32(&bars->tmem_empty[acc]));
     }
   }
 
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) { tc_fence_after(); tmem_dealloc(tmem_base, kLinTmemCols); }
+  tmem_teardown<false>(warp, tmem_base, kLinTmemCols);
 }
 
 __global__ void f32_to_f16_kernel(const float* __restrict__ src, __half* __restrict__ dst, long long n) {
@@ -252,7 +243,7 @@ int launch_linear(const __half* A, const __half* Bm, const LinArgs& args, cudaSt
   if (B_MN) rc = make_tmap_2d(&tmB, Bm, 2, args.N, args.K, static_cast<uint64_t>(args.N) * 2, 64, 64);
   else rc = make_tmap_2d(&tmB, Bm, 2, args.K, args.N, static_cast<uint64_t>(args.K) * 2, 64, 128);
   if (rc) return rc;
-  const size_t smem = LinSmem::total + 1024;
+  const size_t smem = LinSmem::total + kSmemAlign;
   RB_CUDA_CHECK(cudaFuncSetAttribute(linear_gemm_kernel<A_MN, B_MN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const long long items = static_cast<long long>((args.M + kLinTile - 1) / kLinTile) * ((args.N + kLinTile - 1) / kLinTile) * args.ksplit;
   const int grid = static_cast<int>(std::max<long long>(1, std::min<long long>(items, device_sm_count())));
