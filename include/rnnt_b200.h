@@ -178,6 +178,37 @@ int rnnt_b200_greedy_decode_stream(const float* enc, int64_t enc_sb, int64_t enc
                                    int blank, int max_len, int max_per_frame, int32_t* tokens, int32_t* n_tokens,
                                    float* margins_out, void* state, void* stream);
 
+/* Batched beam-search decode in one persistent cooperative kernel (fp32): frame-synchronous "modified" beam search with
+ * at most one symbol per frame, for B utterances at once.  Inputs are those of rnnt_b200_greedy_decode (enc (B,T,H)
+ * with strides (enc_sb, enc_st, 1), multiples of 4; T_len (B), clamped to [0, T]; the 13 weights in the same layout);
+ * beam = K in [1, 8]; max_len counts the seed blank, as for greedy.
+ *
+ * A hypothesis is a token list y (seed excluded) with a log-score s; its predictor features are those of
+ * ConvPredictor([blank] + y)[-1] in eval mode.  The beam starts as {(empty, 0)}.  At each frame t < T_b every
+ * hypothesis h takes logp = log_softmax(W . tanh(enc[b,t] + feats(h)) + bias) in fp32, and its candidates are
+ * (y_h, s_h + logp[blank]) and, when 1 + len(y_h) + 1 <= max_len, (y_h + v, s_h + logp[v]) for every non-blank v.
+ * Candidates with equal token lists merge, with score logaddexp of the two (this only happens when the blank
+ * continuation of h equals the extension of the hypothesis p with y_p + v == y_h; the token lists decide).  The next
+ * beam is the top K merged candidates by score; ties go to the lower rank of the source hypothesis in the previous beam
+ * (a merged candidate counts as the blank continuation of h), then to the lower token index (blank at its own index).
+ * After the last frame the beam is the output, best first.  With K = 1 this is greedy search with one symbol per
+ * frame: the tokens of rnnt_b200_greedy_decode(..., max_per_frame = 1) wherever its top-2 margin is not a near-tie.
+ *
+ * Outputs: tokens (B, K, max_len) int32 (hypothesis k of utterance b in row (b, k), columns past its tokens untouched),
+ * n_tokens (B, K) int32 = 1 + its token count (the seed counted, as greedy), scores (B, K) fp32.  Slots that never fill
+ * (fewer than K distinct token lists exist) get n_tokens 0 and score -inf; T_b = 0 gives one empty hypothesis, score 0.
+ * Results are bit-identical run to run and do not depend on the batch an utterance sits in.
+ * scratch: rnnt_b200_beam_decode_scratch_bytes(B, K, H, V, E, max_len) bytes (0 for invalid arguments), 128-byte
+ * aligned; its first 64 bytes return the eight int64 counters of CTA 0, as for greedy (slot 6 counts frames).
+ * Error codes are those of the greedy entry; a beam size outside [1, 8] returns -1. */
+size_t rnnt_b200_beam_decode_scratch_bytes(int B, int K, int H, int V, int E, int max_len);
+int rnnt_b200_beam_decode(const float* enc, int64_t enc_sb, int64_t enc_st, const int32_t* T_len,
+                          const float* joint_w, const float* joint_b, const float* emb, const float* ln1_w,
+                          const float* ln1_b, const float* conv1_w, const float* conv1_b, const float* conv2_w,
+                          const float* conv2_b, const float* lin_w, const float* lin_b, const float* ln2_w,
+                          const float* ln2_b, int B, int T, int H, int V, int E, int blank, int beam, int max_len,
+                          int32_t* tokens, int32_t* n_tokens, float* scores, void* scratch, void* stream);
+
 /* Optional pre-projections of the joint (rnnt/joint.py:8-12, 26-30: audio_ln / text_ln of the non-"convjs" configs) as
  * tcgen05 GEMMs ahead of the fused call, with their backward.  Row-major contiguous fp32 tensors:
  *   fwd:  y[M,N] = x[M,K] . W[N,K]^T + bias[N]        (M = B*T or B*U1 rows, K = in features, N = hidden_features)

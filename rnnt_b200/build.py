@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "_C")
 LIB_PATH = os.path.join(OUT_DIR, "librnnt_b200.so")
-SOURCES = ["host_util.cu", "joint_gemm.cu", "dh_gemm.cu", "dw_gemm.cu", "linear_gemm.cu", "lattice.cu", "decode.cu", "decode_loop.cu", "api.cu"]
+SOURCES = ["host_util.cu", "joint_gemm.cu", "dh_gemm.cu", "dw_gemm.cu", "linear_gemm.cu", "lattice.cu", "decode.cu", "decode_loop.cu", "beam_loop.cu", "api.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-shared",

@@ -496,6 +496,31 @@ int rnnt_b200_greedy_decode_stream(const float* enc, int64_t enc_sb, int64_t enc
   return rb::launch_greedy_decode(a, static_cast<float*>(state), static_cast<cudaStream_t>(stream));
 }
 
+size_t rnnt_b200_beam_decode_scratch_bytes(int B, int K, int H, int V, int E, int max_len) {
+  if (B <= 0 || K < 1 || K > rb::kMaxBeam || H <= 0 || V <= 1 || E <= 0 || max_len < 1) return 0;
+  return rb::beam_decode_scratch_bytes(B, K, H, V, E, max_len);
+}
+
+int rnnt_b200_beam_decode(const float* enc, int64_t enc_sb, int64_t enc_st, const int32_t* T_len,
+                          const float* joint_w, const float* joint_b, const float* emb, const float* ln1_w,
+                          const float* ln1_b, const float* conv1_w, const float* conv1_b, const float* conv2_w,
+                          const float* conv2_b, const float* lin_w, const float* lin_b, const float* ln2_w,
+                          const float* ln2_b, int B, int T, int H, int V, int E, int blank, int beam, int max_len,
+                          int32_t* tokens, int32_t* n_tokens, float* scores, void* scratch, void* stream) {
+  RB_REQUIRE(T > 0, -1, "invalid shape");
+  if (int rc = check_decode(B, T, H, V, E, blank, max_len, 0, enc_sb, enc_st, scratch)) return rc;
+  RB_REQUIRE(beam >= 1 && beam <= rb::kMaxBeam, -1, "beam size must be in [1, %d] (got %d)", rb::kMaxBeam, beam);
+  RB_REQUIRE(tokens != nullptr && n_tokens != nullptr && scores != nullptr, -1,
+             "beam decode: tokens, n_tokens and scores are required");
+  rb::BeamArgs a{};
+  static_cast<rb::DecodeArgs&>(a) = decode_args(joint_w, joint_b, emb, ln1_w, ln1_b, conv1_w, conv1_b, conv2_w, conv2_b,
+                                                lin_w, lin_b, ln2_w, ln2_b, B, H, V, E);
+  a.enc = enc; a.enc_sb = enc_sb; a.enc_st = enc_st; a.T_len = T_len; a.T = T;
+  a.blank = blank; a.max_len = max_len; a.K = beam;
+  a.tokens = tokens; a.n_tokens = n_tokens; a.scores = scores;
+  return rb::launch_beam_decode(a, static_cast<float*>(scratch), static_cast<cudaStream_t>(stream));
+}
+
 size_t rnnt_b200_linear_workspace_bytes(int64_t M, int K, int N, int backward, int flags) {
   if (M <= 0 || K <= 0 || N <= 0) return 0;
   return rb::linear_workspace_bytes(M, K, N, backward != 0, (flags & RNNT_B200_DETERMINISTIC) != 0);

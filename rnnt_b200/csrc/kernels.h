@@ -101,6 +101,23 @@ struct DecodeArgs {
 size_t greedy_decode_scratch_bytes(int B, int H, int V, int E);
 int launch_greedy_decode(DecodeArgs a, float* scratch, cudaStream_t stream);
 
+// One launch of the persistent beam-search decode (beam_loop.cu).  Weights, sizes, enc / T_len, blank and max_len are
+// the DecodeArgs fields; the rows of the per-row buffers are the B*K hypothesis slots (row b*K + k = slot k of
+// utterance b).  feats, acc1, acc2 and ntok are double-buffered by frame parity ([2][B*K][...]): a frame reads one
+// copy and gathers each new hypothesis's state from its parent into the other.  lin, hbuf, logits, ynew, z, emit and
+// rows are single.  tokens (B,K,max_len) and n_tokens (B,K) are the outputs, as is `scores`.
+struct BeamArgs : DecodeArgs {
+  int K;                      // beam size, 1..kMaxBeam
+  float* scores;              // (B,K) output: log-scores, best first; -inf for slots that never fill
+  float* score;               // [2][B*K] running hypothesis scores
+  unsigned long long* hash;   // [2][B*K] rolling hash of each token list (pre-filter of the merge test)
+  int* hyp;                   // [2][B*K][max_len] token lists (seed blank excluded)
+};
+constexpr int kMaxBeam = 8;
+
+size_t beam_decode_scratch_bytes(int B, int K, int H, int V, int E, int max_len);
+int launch_beam_decode(BeamArgs a, float* scratch, cudaStream_t stream);
+
 int joint_gemm_scratch_tiles(int grid);   // tiles of per-CTA activation scratch the forward needs when h_map == 2
 // tmW: 64(k) x 128(v) boxes (each CTA of a pair loads half of a 256-class block); tmH / tmH2: 64(k) x 64 / 128 (row)
 // boxes of the activation buffer (one half-tile / two adjacent ones); max_slots bounds the work-list slots of this launch

@@ -488,6 +488,59 @@ def greedy_decode(audio_features, audio_feature_lens, joint_weight, joint_bias, 
     return result
 
 
+MAX_BEAM = 8
+
+
+def beam_decode(audio_features, audio_feature_lens, joint_weight, joint_bias, predictor, blank: int,
+                beam_size: int = 4, max_length: int = 200):
+    """Batched frame-synchronous beam search (at most one symbol per frame, equal token lists merged with logaddexp) in
+    ONE persistent CUDA kernel (`rnnt_b200_beam_decode`; include/rnnt_b200.h states the exact rule).
+
+    audio_features (B,T,H) fp32 (any strides), audio_feature_lens (B); `predictor` is ConvPredictor-shaped, as for
+    `greedy_decode`; beam_size in [1, 8]; max_length counts the seed blank.  Returns, per utterance, its n-best list:
+    up to beam_size (tokens, log-score) pairs, best first (fewer when fewer distinct token lists exist)."""
+    K = int(beam_size)
+    if not 1 <= K <= MAX_BEAM:
+        raise ValueError(f"beam_size must be in [1, {MAX_BEAM}] (got {beam_size})")
+    _require_cuda(audio_features, joint_weight, joint_bias)
+    L = _lib.lib()
+    dev = audio_features.device
+    B, T, H = audio_features.shape
+    V = joint_weight.shape[0]
+    _check_decode_sizes(predictor, joint_weight, H)
+    E = predictor.embedding.embedding_dim
+    enc = audio_features.detach().to(dev, torch.float32).contiguous()
+    params = _decode_params(joint_weight, joint_bias, predictor, dev)
+    lens = audio_feature_lens.to(dev, torch.int32).clamp(0, T).contiguous()
+    max_len = max(int(max_length), 1)
+    tokens = torch.zeros(B, K, max_len, dtype=torch.int32, device=dev)
+    ntok = torch.zeros(B, K, dtype=torch.int32, device=dev)
+    scores = torch.empty(B, K, dtype=torch.float32, device=dev)
+    scratch = torch.empty(L.rnnt_b200_beam_decode_scratch_bytes(B, K, H, V, E, max_len), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(L.rnnt_b200_beam_decode(
+            enc.data_ptr(), enc.stride(0), enc.stride(1), lens.data_ptr(), *[t.data_ptr() for t in params],
+            B, T, H, V, E, int(blank), K, max_len, tokens.data_ptr(), ntok.data_ptr(), scores.data_ptr(),
+            scratch.data_ptr(), _stream_ptr(dev)), "beam_decode")
+    global _last_decode_phase_cycles
+    _last_decode_phase_cycles = scratch[:64].view(torch.int64)
+    n, toks, sc = ntok.tolist(), tokens.tolist(), scores.tolist()
+    return [[(toks[b][k][: n[b][k] - 1], sc[b][k]) for k in range(K) if n[b][k] > 0] for b in range(B)]
+
+
+def _check_kernel_decode_modules(joint, predictor, what: str) -> None:
+    """The modules the persistent decode kernels accept: a ConvPredictor-shaped predictor, a joint without
+    pre-projections."""
+    from .model import _is_conv_predictor, _is_lstm_predictor
+    if _is_lstm_predictor(predictor):
+        raise ValueError(f"{what} needs a ConvPredictor; decode an LSTM predictor with "
+                         "RNNTModel.greedy_decode_features")
+    if not _is_conv_predictor(predictor):
+        raise ValueError("Unknown predictor type")
+    if hasattr(joint, "audio_ln") or hasattr(joint, "text_ln"):
+        raise ValueError(f"{what} does not support a joint with audio_ln / text_ln pre-projections")
+
+
 class StreamingGreedyDecoder:
     """Greedy decode of `slots` live streams whose encoder frames arrive chunk by chunk, in the persistent decode kernel
     (`rnnt_b200_greedy_decode_stream`).  The decoder state of every slot stays on the device between calls.
@@ -499,14 +552,7 @@ class StreamingGreedyDecoder:
     weights change (it empties every slot)."""
 
     def __init__(self, joint, predictor, slots: int, max_length: int = 200, max_outputs_per_step: int = 10):
-        from .model import _is_conv_predictor, _is_lstm_predictor
-        if _is_lstm_predictor(predictor):
-            raise ValueError("streaming decode needs a ConvPredictor; decode an LSTM predictor with "
-                             "RNNTModel.greedy_decode_features")
-        if not _is_conv_predictor(predictor):
-            raise ValueError("Unknown predictor type")
-        if hasattr(joint, "audio_ln") or hasattr(joint, "text_ln"):
-            raise ValueError("streaming decode does not support a joint with audio_ln / text_ln pre-projections")
+        _check_kernel_decode_modules(joint, predictor, "streaming decode")
         if int(slots) < 1:
             raise ValueError("slots must be >= 1")
         weight = joint.joint_ln.weight

@@ -95,6 +95,24 @@ class RNNTModel(torch.nn.Module):
         return StreamingGreedyDecoder(self.joint, self.predictor, slots, max_length, max_outputs_per_step)
 
     @torch.no_grad()
+    def beam_search_features(self, audio_features, audio_feature_lens, beam_size: int = 4, max_length: int = 200):
+        """Batched beam search on given encoder features (B,T,H) (e.g. the permuted view of the encoder's (B,H,T)
+        output) with per-utterance lengths, in one persistent CUDA kernel (`functional.beam_decode`): per utterance,
+        up to beam_size (tokens, log-score) pairs, best first."""
+        from .functional import _check_kernel_decode_modules, _require_cuda, beam_decode
+        _check_kernel_decode_modules(self.joint, self.predictor, "beam search")
+        _require_cuda(audio_features, self.joint.joint_ln.weight)
+        return beam_decode(audio_features, torch.as_tensor(audio_feature_lens), self.joint.joint_ln.weight,
+                           self.joint.joint_ln.bias, self.predictor, self.joint.blank_idx, beam_size, max_length)
+
+    @torch.no_grad()
+    def beam_search(self, mel_features, mel_feature_lens, beam_size: int = 4, max_length: int = 200):
+        """Beam search from mel features: the encoder and its output lengths first, then `beam_search_features`."""
+        audio_features = self.encoder(mel_features).permute(0, 2, 1)
+        audio_feature_lens = self.encoder.calc_output_lens(mel_feature_lens)
+        return self.beam_search_features(audio_features, audio_feature_lens, beam_size, max_length)
+
+    @torch.no_grad()
     def _greedy_decode_features_hostloop(self, audio_features, audio_feature_lens, max_length: int = 200,
                                          max_outputs_per_step: int = 10):
         """Host-driven variant (one device sync per step, predictor re-run on 7-token windows); kept as an independent
