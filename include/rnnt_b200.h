@@ -107,6 +107,29 @@ int rnnt_b200_loss_dense_bwd(const float* logits, const int32_t* targets, const 
 int rnnt_b200_lattice(const float* lp, const int32_t* T_len, const int32_t* U_len, int B, int T, int U1, float* alpha,
                       float* beta, float* costs, void* stream);
 
+/* Forced alignment, lattice only: the best path of each utterance through the (t, u) lattice of log-probs lp
+ * (B,T,U1,2) = (log p(blank), log p(label)), as rnnt_b200_joint_loss_fwd (with hidden = NULL) or
+ * rnnt_b200_loss_dense_fwd write them.  A path goes from (0,0) to (T_b-1, U_b): a blank step (t,u)->(t+1,u) adds
+ * lpB(t,u), a label step (t,u)->(t,u+1) adds lpE(t,u), and the final blank at (T_b-1, U_b) adds lpB(T_b-1, U_b) --
+ * the paths whose log-sum-exp is -cost.
+ *   scores (B) fp32: the largest path log-probability, computed in fp32 as
+ *     delta(0,0) = 0, delta(t,u) = max(delta(t-1,u) + lpB(t-1,u), delta(t,u-1) + lpE(t,u-1)),
+ *     score = delta(T_b-1,U_b) + lpB(T_b-1,U_b),
+ *   each sum one IEEE fp32 add (no FMA): the score equals the fp32 left-to-right sum of the path's edge log-probs.
+ *   frames (B, U1-1) int32 (may be NULL when U1 == 1): frames[b,u] for u < U_b is the frame t of the path's label step
+ *   (t,u)->(t,u+1); non-decreasing, in [0, T_b-1].  Columns u >= U_b are set to -1.
+ * Ties: the backtrace at (t,u) takes the label predecessor (t,u-1) only if its value is strictly greater; on an exact
+ * tie it takes the blank predecessor (t-1,u), so the token goes to the earlier frame.
+ * An utterance with T_b outside [1,T] or U_b outside [0,U1-1] gets score NaN and a frames row of -1; the others are not
+ * affected.  lp outside an utterance's valid cells, and lpE in its last column u = U_b, are never read.
+ * One CTA per utterance keeps the decision bits in shared memory: 4 * ceil(T/32) * round_up(U1,32) bytes plus
+ * 8 * (round_up(U1,32) + 2) must fit the 232448-byte per-block limit of sm_100a (T up to 1728 at U1 = 1024, 14432 at
+ * U1 = 101).  Returns -1 for an invalid shape or missing outputs, -5 for U1 > 1024 or T past that bound (the message
+ * gives the bound); both are checked before any device work.  Outputs are bit-identical run to run and do not depend on
+ * the batch an utterance sits in. */
+int rnnt_b200_viterbi(const float* lp, const int32_t* T_len, const int32_t* U_len, int B, int T, int U1,
+                      int32_t* frames, float* scores, void* stream);
+
 /* Greedy-decode joint step (fp32): tokens[n] = argmax_v(W . tanh(enc_rows[n] + pred_rows[n]) + bias), lowest index
  * on ties; margin[n] (optional) = top1 - top2 logit.  Row n of enc_rows / pred_rows starts at n * stride floats.
  * scratch: rnnt_b200_joint_argmax_scratch_bytes(N, V) bytes. */
@@ -225,7 +248,7 @@ int rnnt_b200_linear_bwd(const float* x, const float* W, const float* dy, int64_
  * CUDA events on its launch stream.  end() synchronises on those events and returns, per kernel family, the summed
  * device time in ms and the number of launches.  HOST pointers.  Families: 0 prep (tile table, weight conversion,
  * gradient coefficients), 1 joint GEMM forward, 2 lattice, 3 joint GEMM backward-recompute, 4 dh GEMM, 5 dW GEMM,
- * 6 db, 7 other (dense-logits kernels, decode). */
+ * 6 db, 7 other (dense-logits kernels, decode, Viterbi). */
 int rnnt_b200_profile_begin(void);
 int rnnt_b200_profile_end(float* ms /*[8]*/, int64_t* launches /*[8]*/);
 

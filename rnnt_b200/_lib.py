@@ -33,6 +33,7 @@ _SIGNATURES = {
     "rnnt_b200_loss_dense_bwd": (C.c_int, [_f32p, _i32p, _i32p, _i32p] + [C.c_int] * 5 + [_f32p] * 5
                                  + [C.c_float, _f32p, _f32p, _ptr]),
     "rnnt_b200_lattice": (C.c_int, [_f32p, _i32p, _i32p, C.c_int, C.c_int, C.c_int, _f32p, _f32p, _f32p, _ptr]),
+    "rnnt_b200_viterbi": (C.c_int, [_f32p, _i32p, _i32p, C.c_int, C.c_int, C.c_int, _i32p, _f32p, _ptr]),
     "rnnt_b200_joint_argmax_scratch_bytes": (C.c_size_t, [C.c_int, C.c_int]),
     "rnnt_b200_joint_argmax": (C.c_int, [_f32p, C.c_int64, _f32p, C.c_int64, _f32p, _f32p, C.c_int, C.c_int, C.c_int,
                                          _i32p, _f32p, _ptr, _ptr]),

@@ -252,6 +252,14 @@ int rnnt_b200_lattice(const float* lp, const int32_t* T_len, const int32_t* U_le
   return rb::launch_lattice(lp, T_len, U_len, B, T, U1, alpha, beta, costs, nullptr, static_cast<cudaStream_t>(stream));
 }
 
+int rnnt_b200_viterbi(const float* lp, const int32_t* T_len, const int32_t* U_len, int B, int T, int U1,
+                      int32_t* frames, float* scores, void* stream) {
+  RB_REQUIRE(B > 0 && T > 0 && U1 > 0, -1, "invalid shape");
+  RB_REQUIRE(scores != nullptr && (frames != nullptr || U1 == 1), -1,
+             "viterbi: scores and (for U+1 > 1) frames are required");
+  return rb::launch_viterbi(lp, T_len, U_len, B, T, U1, frames, scores, static_cast<cudaStream_t>(stream));
+}
+
 int rnnt_b200_joint_loss_fwd(const float* enc, int64_t enc_sb, int64_t enc_st, int64_t enc_sh, const float* pred,
                              const float* W, const float* bias, const int32_t* targets, const int32_t* T_len,
                              const int32_t* U_len, int B, int T, int U1, int H, int V, int blank, float* costs,

@@ -139,6 +139,12 @@ int launch_convert_weights(const float* W, const float* bias, int V, int H, int 
 // status (optional): device flag written by the tile table; a non-zero flag turns every cost into NaN
 int launch_lattice(const float* lp, const int* T_len, const int* U_len, int B, int T, int U1, float* alpha,
                    float* beta, float* costs, const int* status, cudaStream_t stream);
+// Viterbi walk + backtrace (forced alignment), one CTA of round_up(U1, 32) threads per utterance.  Its decision bits
+// live in shared memory: viterbi_smem_bytes(T, U1) must not exceed the sm_100a per-block opt-in limit.
+constexpr size_t kViterbiSmemLimit = 232448;
+size_t viterbi_smem_bytes(int T, int U1);
+int launch_viterbi(const float* lp, const int* T_len, const int* U_len, int B, int T, int U1, int* frames,
+                   float* scores, cudaStream_t stream);
 // deterministic mode: out[i] = fx[i] * 2^-36 * gscale[1]; dst strides in elements (n0 x n1 x n2 logical shape)
 int launch_finalize_fixed(const long long* fx, float* out, long long n0, long long n1, long long n2, long long s0,
                           long long s1, long long s2, const float* gscale, cudaStream_t stream);

@@ -1,5 +1,5 @@
-// Small kernels around the GEMMs: tile table, weight conversion, alpha/beta lattice, gradient coefficients,
-// and the dense-logits variants of the loss front/back end (for callers that already hold logits).
+// Small kernels around the GEMMs: tile table, weight conversion, alpha/beta lattice, Viterbi (forced alignment),
+// gradient coefficients, and the dense-logits variants of the loss front/back end (for callers that already hold logits).
 //
 // Lattice = torchaudio ComputeAlphasBetasCosts (reference call site rnnt/model.py:35-41):
 //   alpha[0,0]=0; alpha[t,u]=LSE(alpha[t-1,u]+lpB[t-1,u], alpha[t,u-1]+lpE[t,u-1])
@@ -192,6 +192,124 @@ __global__ void lattice_kernel(const float* __restrict__ lp, const int* __restri
   const bool poison = status != nullptr && *status != 0;
   if (blockIdx.y == 1) lattice_walk<true>(lp2, beta + off, costs + b, Tb, Ub, U1, u, sh0, sh1, poison);
   else lattice_walk<false>(lp2, alpha + off, costs + b, Tb, Ub, U1, u, sh0, sh1, poison);
+}
+
+// ---- Viterbi (forced alignment): the max-plus version of the alpha walk, with a backtrace.
+//   delta(0,0) = 0;  delta(t,u) = max(delta(t-1,u) + lpB(t-1,u), delta(t,u-1) + lpE(t,u-1));  score = delta(Tb-1,Ub) + lpB
+// Each sum is one fp32 add and the max a compare-select, so the score is the fp32 left-to-right sum of the best path's
+// edge log-probs.  Per step a thread keeps one decision bit, "came from the left" (the label predecessor is strictly
+// greater; an exact tie goes to the blank one, i.e. the token to the earlier frame), in a register word that goes to
+// shared memory every 32 steps of the thread and at its last: dec[(t >> 5) * ncols + u].
+__device__ __forceinline__ void viterbi_walk(const float2* __restrict__ lp2, int Tb, int Ub, int U1, int u, float* sh0,
+                                             float* sh1, unsigned* dec, int ncols, float* score) {
+  // Structure and hoisting as in lattice_walk<false>: one unsigned compare for the activity test, the last column's
+  // emit log-prob is -inf when fetched, the corner cell starts from own = 0 with side = -inf.
+  const int ndiag = Tb + Ub;
+  const int s0 = u <= Ub ? u : 0x40000000;
+  const float2* src = lp2 + min(u, U1 - 1);
+  const bool last_col = u >= Ub;
+  uint32_t rd_addr[2] = {smem_u32(sh1 + u - 1), smem_u32(sh0 + u - 1)};      // step parity 0 reads sh1, writes sh0
+  uint32_t wr_addr[2] = {smem_u32(sh0 + u), smem_u32(sh1 + u)};
+  uint32_t dec_addr = smem_u32(dec + u);
+#pragma unroll
+  for (int i = 0; i < 2; ++i) {
+    asm volatile("mov.u32 %0, %0;" : "+r"(rd_addr[i]));
+    asm volatile("mov.u32 %0, %0;" : "+r"(wr_addr[i]));
+  }
+  asm volatile("mov.u32 %0, %0;" : "+r"(dec_addr));
+  const uint32_t dec_row = static_cast<uint32_t>(ncols) * 4u;
+
+  float2 cur[kPre], nxt[kPre];
+  auto fetch = [&](int g, float2 (&d)[kPre]) {
+#pragma unroll
+    for (int i = 0; i < kPre; ++i) {
+      const int rel = g * kPre + i - s0;
+      float2 v = make_float2(0.f, 0.f);
+      if (static_cast<unsigned>(rel) < static_cast<unsigned>(Tb)) v = __ldg(src + static_cast<long long>(rel) * U1);
+      if (last_col) v.y = -INFINITY;
+      d[i] = v;
+    }
+  };
+  const int ngroups = (ndiag + kPre - 1) / kPre;
+  fetch(0, cur);
+  float own = u == 0 ? 0.f : -INFINITY;                      // delta(t-1,u) + lpB(t-1,u)
+  unsigned bits = 0u;
+  int t = 0;                                                 // this column's next cell
+  for (int g = 0; g < ngroups; ++g) {
+    if (g + 1 < ngroups) fetch(g + 1, nxt);
+#pragma unroll
+    for (int i = 0; i < kPre; ++i) {
+      const int s = g * kPre + i;
+      if (s < ndiag) {    // uniform over the block
+        const bool act = static_cast<unsigned>(s - s0) < static_cast<unsigned>(Tb);
+        float side;                                          // delta(t,u-1) + lpE(t,u-1); -inf guard at column -1
+        asm volatile("ld.shared.f32 %0, [%1];" : "=f"(side) : "r"(rd_addr[i & 1]) : "memory");
+        const bool left = side > own;
+        const float val = left ? side : own;                 // delta(t,u)
+        if (act) {
+          bits |= static_cast<unsigned>(left) << (t & 31);
+          if ((t & 31) == 31 || t == Tb - 1) {
+            asm volatile("st.shared.u32 [%0], %1;" ::"r"(dec_addr), "r"(bits) : "memory");
+            dec_addr += dec_row;
+            bits = 0u;
+          }
+          ++t;
+          own = val + cur[i].x;                              // at the last cell of column Ub: the score
+        }
+        const float pub = act ? val + cur[i].y : -INFINITY;
+        asm volatile("st.shared.f32 [%0], %1;" ::"r"(wr_addr[i & 1]), "f"(pub) : "memory");
+        __syncthreads();
+      }
+    }
+#pragma unroll
+    for (int i = 0; i < kPre; ++i) cur[i] = nxt[i];
+  }
+  if (u == Ub) *score = own;
+}
+
+// One CTA per utterance, thread u = lattice column u.  Dynamic shared memory: the two neighbour buffers of
+// 2 x (ncols + 2) floats (re-used for the frames after the walk), then ceil(T/32) x ncols decision words.
+__global__ void viterbi_kernel(const float* __restrict__ lp, const int* __restrict__ T_len,
+                               const int* __restrict__ U_len, int T, int U1, int* __restrict__ frames,
+                               float* __restrict__ scores) {
+  extern __shared__ float sh[];
+  const int b = blockIdx.x;
+  const int u = threadIdx.x;
+  const int ncols = blockDim.x;
+  const int Tb = T_len[b], Ub = U_len[b];
+  int* frow = frames + static_cast<long long>(b) * (U1 - 1);
+  if (Tb < 1 || Tb > T || Ub < 0 || Ub > U1 - 1) {          // this utterance only; uniform over the block
+    if (u < U1 - 1) frow[u] = -1;
+    if (u == 0) scores[b] = __int_as_float(0x7fc00000);
+    return;
+  }
+  const int stride = ncols + 2;
+  float* sh0 = sh + 1;                                       // sh0[-1] and sh0[ncols] are -inf guards
+  float* sh1 = sh + stride + 1;
+  unsigned* dec = reinterpret_cast<unsigned*>(sh + 2 * stride);
+  if (u == 0) {
+    sh0[-1] = -INFINITY; sh1[-1] = -INFINITY;
+    sh0[ncols] = -INFINITY; sh1[ncols] = -INFINITY;
+  }
+  sh0[u] = -INFINITY;
+  sh1[u] = -INFINITY;
+  __syncthreads();
+  float score = 0.f;
+  viterbi_walk(reinterpret_cast<const float2*>(lp) + static_cast<long long>(b) * T * U1, Tb, Ub, U1, u, sh0, sh1, dec,
+               ncols, &score);
+  // The walk ended with a __syncthreads: every decision word is in place and the neighbour buffers are free.
+  int* fr = reinterpret_cast<int*>(sh);
+  if (u == 0) {
+    int t = Tb - 1, c = Ub;
+    while (c > 0) {                                          // at t = 0 the left predecessor is the only one
+      const unsigned w = dec[(t >> 5) * ncols + c];
+      if (t == 0 || ((w >> (t & 31)) & 1u)) fr[--c] = t;
+      else --t;
+    }
+  }
+  __syncthreads();
+  if (u < U1 - 1) frow[u] = u < Ub ? fr[u] : -1;
+  if (u == Ub) scores[b] = score;
 }
 
 __global__ void coef_kernel(const float* __restrict__ lp, const float* __restrict__ lse,
@@ -397,6 +515,30 @@ int launch_lattice(const float* lp, const int* T_len, const int* U_len, int B, i
   RB_REQUIRE(threads <= 1024, -5, "lattice kernel supports U+1 <= 1024 (got %d)", U1);
   const size_t smem = 2 * (threads + 2) * sizeof(float);
   lattice_kernel<<<dim3(B, 2), threads, smem, stream>>>(lp, T_len, U_len, T, U1, alpha, beta, costs, status);
+  RB_CUDA_CHECK(cudaGetLastError());
+  return 0;
+}
+
+size_t viterbi_smem_bytes(int T, int U1) {
+  const size_t ncols = (static_cast<size_t>(U1) + 31) / 32 * 32;
+  return 2 * (ncols + 2) * sizeof(float) + (static_cast<size_t>(T) + 31) / 32 * ncols * sizeof(unsigned);
+}
+
+int launch_viterbi(const float* lp, const int* T_len, const int* U_len, int B, int T, int U1, int* frames,
+                   float* scores, cudaStream_t stream) {
+  const int threads = ((U1 + 31) / 32) * 32;
+  RB_REQUIRE(threads <= 1024, -5, "viterbi kernel supports U+1 <= 1024 (got %d)", U1);
+  const size_t smem = viterbi_smem_bytes(T, U1);
+  const size_t neighbours = 2 * (threads + 2) * sizeof(float);
+  const long long max_T = static_cast<long long>((kViterbiSmemLimit - neighbours) / (threads * sizeof(unsigned))) * 32;
+  RB_REQUIRE(smem <= kViterbiSmemLimit, -5,
+             "viterbi: the decisions of T=%d frames need %zu bytes of shared memory, over the %zu-byte per-block limit; "
+             "at U+1=%d the bound is T <= %lld",
+             T, smem, kViterbiSmemLimit, U1, max_T);
+  ProfScope prof_(kProfOther, stream);
+  RB_CUDA_CHECK(cudaFuncSetAttribute(viterbi_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                     static_cast<int>(smem)));
+  viterbi_kernel<<<B, threads, smem, stream>>>(lp, T_len, U_len, T, U1, frames, scores);
   RB_CUDA_CHECK(cudaGetLastError());
   return 0;
 }

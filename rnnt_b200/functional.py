@@ -8,7 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-from typing import Optional
+from typing import NamedTuple, Optional
 
 import torch
 
@@ -269,6 +269,21 @@ def _reduce(costs, reduction):
     raise ValueError('reduction should be one of "none", "mean", "sum"')
 
 
+def _check_joint_inputs(audio_frame, text_frame, weight, targets, logit_lengths, target_lengths, blank, validate):
+    """The fused entries' checks on dtypes, shapes, blank and (validate=True) lengths, with torchaudio's messages."""
+    if audio_frame.dtype != torch.float32 or text_frame.dtype != torch.float32:
+        raise RuntimeError("joint inputs must be float32 (the fused kernels convert to fp16 operands internally)")
+    if audio_frame.dim() != 3 or text_frame.dim() != 3 or audio_frame.shape[0] != text_frame.shape[0] \
+            or audio_frame.shape[2] != text_frame.shape[2] or weight.shape[1] != audio_frame.shape[2]:
+        raise RuntimeError("expected audio (B,T,H), text (B,U+1,H) and weight (V,H)")
+    _check_index_tensors(targets, logit_lengths, target_lengths)
+    if targets.shape[0] != audio_frame.shape[0] or targets.shape[1] != text_frame.shape[1] - 1:
+        raise RuntimeError("output length mismatch")
+    _check_blank(blank, weight.shape[0])
+    if validate:
+        _validate_lengths(audio_frame.shape[1], text_frame.shape[1], logit_lengths, target_lengths)
+
+
 def joint_rnnt_loss(audio_frame, text_frame, weight, bias, targets, logit_lengths, target_lengths, blank: int = -1,
                     clamp: float = -1, reduction: str = "mean", validate: bool = True,
                     ring_bytes: Optional[int] = None, return_residuals: bool = False,
@@ -290,17 +305,7 @@ def joint_rnnt_loss(audio_frame, text_frame, weight, bias, targets, logit_length
     With validate=False, lengths outside [1,T] / [0,U] (for which torchaudio raises) make every cost NaN instead.
     """
     _require_cuda(audio_frame, text_frame, weight, bias, targets, logit_lengths, target_lengths)
-    if audio_frame.dtype != torch.float32 or text_frame.dtype != torch.float32:
-        raise RuntimeError("joint inputs must be float32 (the fused kernels convert to fp16 operands internally)")
-    if audio_frame.dim() != 3 or text_frame.dim() != 3 or audio_frame.shape[0] != text_frame.shape[0] \
-            or audio_frame.shape[2] != text_frame.shape[2] or weight.shape[1] != audio_frame.shape[2]:
-        raise RuntimeError("expected audio (B,T,H), text (B,U+1,H) and weight (V,H)")
-    _check_index_tensors(targets, logit_lengths, target_lengths)
-    if targets.shape[0] != audio_frame.shape[0] or targets.shape[1] != text_frame.shape[1] - 1:
-        raise RuntimeError("output length mismatch")
-    _check_blank(blank, weight.shape[0])
-    if validate:
-        _validate_lengths(audio_frame.shape[1], text_frame.shape[1], logit_lengths, target_lengths)
+    _check_joint_inputs(audio_frame, text_frame, weight, targets, logit_lengths, target_lengths, blank, validate)
     costs, lp, lse, alpha, beta = _FusedJointLoss.apply(audio_frame, text_frame, weight.float(), bias.float(),
                                                         targets, logit_lengths, target_lengths, int(blank),
                                                         float(clamp), ring_bytes, bool(skip_zero_tiles), save_hidden,
@@ -311,24 +316,30 @@ def joint_rnnt_loss(audio_frame, text_frame, weight, bias, targets, logit_length
     return out
 
 
+def _dense_forward(logits, targets, logit_lengths, target_lengths, blank):
+    """rnnt_b200_loss_dense_fwd: costs and the residuals lp, lse, alpha, beta of dense fp32 logits (B,T,U+1,V)."""
+    L = _lib.lib()
+    B, T, U1, V = logits.shape
+    dev = logits.device
+    costs = torch.empty(B, dtype=torch.float32, device=dev)
+    lp = torch.empty(B, T, U1, 2, dtype=torch.float32, device=dev)
+    lse = torch.empty(B, T, U1, dtype=torch.float32, device=dev)
+    alpha = torch.empty(B, T, U1, dtype=torch.float32, device=dev)
+    beta = torch.empty(B, T, U1, dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(L.rnnt_b200_loss_dense_fwd(
+            logits.data_ptr(), targets.data_ptr(), logit_lengths.data_ptr(), target_lengths.data_ptr(),
+            B, T, U1, V, blank, costs.data_ptr(), lp.data_ptr(), lse.data_ptr(), alpha.data_ptr(),
+            beta.data_ptr(), _stream_ptr(dev)), "loss_dense_fwd")
+    return costs, lp, lse, alpha, beta
+
+
 class _DenseLoss(torch.autograd.Function):
     """torchaudio.functional.rnnt_loss on materialised logits: log-softmax gather, lattice, gradient kernel."""
 
     @staticmethod
     def forward(ctx, logits, targets, logit_lengths, target_lengths, blank, clamp):
-        L = _lib.lib()
-        B, T, U1, V = logits.shape
-        dev = logits.device
-        costs = torch.empty(B, dtype=torch.float32, device=dev)
-        lp = torch.empty(B, T, U1, 2, dtype=torch.float32, device=dev)
-        lse = torch.empty(B, T, U1, dtype=torch.float32, device=dev)
-        alpha = torch.empty(B, T, U1, dtype=torch.float32, device=dev)
-        beta = torch.empty(B, T, U1, dtype=torch.float32, device=dev)
-        with torch.cuda.device(dev):
-            _lib.check(L.rnnt_b200_loss_dense_fwd(
-                logits.data_ptr(), targets.data_ptr(), logit_lengths.data_ptr(), target_lengths.data_ptr(),
-                B, T, U1, V, blank, costs.data_ptr(), lp.data_ptr(), lse.data_ptr(), alpha.data_ptr(),
-                beta.data_ptr(), _stream_ptr(dev)), "loss_dense_fwd")
+        costs, lp, lse, alpha, beta = _dense_forward(logits, targets, logit_lengths, target_lengths, blank)
         ctx.save_for_backward(logits, targets, logit_lengths, target_lengths, lp, lse, alpha, beta)
         ctx.blank, ctx.clamp = blank, clamp
         return costs
@@ -354,6 +365,20 @@ class _DenseLoss(torch.autograd.Function):
         return grads, None, None, None, None, None
 
 
+def _check_dense_inputs(logits, targets, logit_lengths, target_lengths, blank):
+    """The dense entries' checks (torchaudio's messages): fp32 contiguous 4-D logits, int32 indices, lengths, blank."""
+    if logits.dtype != torch.float32:
+        raise RuntimeError("logits must be float32 or float16 (half) type" if logits.dtype not in
+                           (torch.float16,) else "rnnt_b200 dense loss supports float32 logits only")
+    if not logits.is_contiguous():
+        raise RuntimeError("logits must be contiguous")
+    if logits.dim() != 4:
+        raise RuntimeError("logits must be 4-D (batch, time, target, class)")
+    _check_index_tensors(targets, logit_lengths, target_lengths)
+    _validate_lengths(logits.shape[1], logits.shape[2], logit_lengths, target_lengths)
+    _check_blank(blank, logits.shape[-1])
+
+
 def rnnt_loss(logits, targets, logit_lengths, target_lengths, blank: int = -1, clamp: float = -1,
               reduction: str = "mean", fused_log_softmax: bool = True):
     """Same signature and error behaviour as torchaudio.functional.rnnt_loss (call site rnnt/model.py:35-41).
@@ -368,16 +393,7 @@ def rnnt_loss(logits, targets, logit_lengths, target_lengths, blank: int = -1, c
     if not fused_log_softmax:
         raise RuntimeError("rnnt_b200.rnnt_loss only implements fused_log_softmax=True (what the reference uses)")
     _require_cuda(logits, targets, logit_lengths, target_lengths)
-    if logits.dtype != torch.float32:
-        raise RuntimeError("logits must be float32 or float16 (half) type" if logits.dtype not in
-                           (torch.float16,) else "rnnt_b200 dense loss supports float32 logits only")
-    if not logits.is_contiguous():
-        raise RuntimeError("logits must be contiguous")
-    if logits.dim() != 4:
-        raise RuntimeError("logits must be 4-D (batch, time, target, class)")
-    _check_index_tensors(targets, logit_lengths, target_lengths)
-    _validate_lengths(logits.shape[1], logits.shape[2], logit_lengths, target_lengths)
-    _check_blank(blank, logits.shape[-1])
+    _check_dense_inputs(logits, targets, logit_lengths, target_lengths, blank)
     costs = _DenseLoss.apply(logits, targets, logit_lengths, target_lengths, int(blank), float(clamp))
     return _reduce(costs, reduction)
 
@@ -395,6 +411,70 @@ def lattice(lp, logit_lengths, target_lengths):
                                                 B, T, U1, alpha.data_ptr(), beta.data_ptr(), costs.data_ptr(),
                                                 _stream_ptr(lp.device)), "lattice")
     return alpha, beta, costs
+
+
+class Alignment(NamedTuple):
+    """Forced alignment of a batch (`forced_align`, `joint_forced_align`), device tensors without grad.
+    frames (B,U) int32: frame of each target token on the best path, -1 past U_b.  score (B) fp32: the best path's
+    log-probability.  log_prob (B) fp32: log P(targets | audio) = -cost of the same forward, so exp(score - log_prob)
+    is the best path's posterior."""
+    frames: torch.Tensor
+    score: torch.Tensor
+    log_prob: torch.Tensor
+
+
+def viterbi(lp, logit_lengths, target_lengths):
+    """frames (B,U) int32 and score (B) fp32 of the best lattice path from log-probs (B,T,U+1,2) -- the Viterbi kernel
+    alone (`rnnt_b200_viterbi`; include/rnnt_b200.h states the recursion and the tie rule).  An utterance whose lengths
+    are out of range gets score NaN and frames -1."""
+    if lp.dim() != 4 or lp.shape[-1] != 2:
+        raise RuntimeError("expected log-probs of shape (B,T,U+1,2)")
+    if logit_lengths.dtype != torch.int32:
+        raise RuntimeError("logit_lengths must be int32 type")
+    if target_lengths.dtype != torch.int32:
+        raise RuntimeError("target_lengths must be int32 type")
+    _require_cuda(lp, logit_lengths, target_lengths)
+    B, T, U1, _ = lp.shape
+    lp = lp.contiguous().float()
+    T_len, U_len = logit_lengths.contiguous(), target_lengths.contiguous()
+    frames = torch.empty(B, U1 - 1, dtype=torch.int32, device=lp.device)
+    score = torch.empty(B, dtype=torch.float32, device=lp.device)
+    with torch.cuda.device(lp.device):
+        _lib.check(_lib.lib().rnnt_b200_viterbi(lp.data_ptr(), T_len.data_ptr(), U_len.data_ptr(), B, T, U1,
+                                                frames.data_ptr() if U1 > 1 else None, score.data_ptr(),
+                                                _stream_ptr(lp.device)), "viterbi")
+    return frames, score
+
+
+def joint_forced_align(audio_frame, text_frame, weight, bias, targets, logit_lengths, target_lengths,
+                       blank: int = -1, validate: bool = True) -> Alignment:
+    """Forced alignment through the fused joint: the inputs, checks and messages of `joint_rnnt_loss`, the fused forward
+    without an activation residual (no logits, no autograd), then the Viterbi kernel on its log-probs.  audio_frame may
+    be the permuted (B,T,H) view of the encoder's (B,H,T) output; it is read in place.  With validate=False, lengths
+    outside [1,T] / [0,U] give that utterance score NaN and frames -1, and every log_prob NaN (as the loss's costs)."""
+    _check_joint_inputs(audio_frame, text_frame, weight, targets, logit_lengths, target_lengths, blank, validate)
+    _require_cuda(audio_frame, text_frame, weight, bias, targets, logit_lengths, target_lengths)
+    with torch.no_grad():
+        costs, lp, _, _, _ = _FusedJointLoss.apply(audio_frame.detach(), text_frame.detach(), weight.detach().float(),
+                                                   bias.detach().float(), targets, logit_lengths, target_lengths,
+                                                   int(blank), -1.0, None, True, False, None)
+        frames, score = viterbi(lp, logit_lengths, target_lengths)
+    return Alignment(frames, score, -costs)
+
+
+def forced_align(logits, targets, logit_lengths, target_lengths, blank: int = -1) -> Alignment:
+    """Forced alignment with the inputs of `rnnt_loss`: dense fp32 logits (B,T,U+1,V) go through the dense front end,
+    the lazy handle of a zero-edit-mode JointNetwork through `joint_forced_align`."""
+    from .joint import LazyJointLogits
+    if isinstance(logits, LazyJointLogits):
+        return joint_forced_align(logits.audio, logits.text, logits.weight, logits.bias, targets, logit_lengths,
+                                  target_lengths, blank=blank)
+    _check_dense_inputs(logits, targets, logit_lengths, target_lengths, blank)
+    _require_cuda(logits, targets, logit_lengths, target_lengths)
+    with torch.no_grad():
+        costs, lp, _, _, _ = _dense_forward(logits.detach(), targets, logit_lengths, target_lengths, int(blank))
+        frames, score = viterbi(lp, logit_lengths, target_lengths)
+    return Alignment(frames, score, -costs)
 
 
 def joint_argmax_scratch(N: int, V: int, device):

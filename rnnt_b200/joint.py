@@ -87,6 +87,16 @@ class JointNetwork(torch.nn.Module):
                                logit_lengths, target_lengths, blank=blank, clamp=clamp, reduction=reduction,
                                validate=validate)
 
+    def align(self, audio_frame, text_frame, targets, logit_lengths, target_lengths, blank: int = -1,
+              validate: bool = True):
+        """Forced alignment of `targets` (`functional.joint_forced_align`): the fused pre-projections, then the fused
+        forward and the Viterbi kernel.  Returns an `Alignment` (frames, score, log_prob) without grad."""
+        from .functional import joint_forced_align
+        with torch.no_grad():
+            audio_frame, text_frame = self._project(audio_frame, text_frame, fused=True)
+        return joint_forced_align(audio_frame, text_frame, self.joint_ln.weight, self.joint_ln.bias, targets,
+                                  logit_lengths, target_lengths, blank=blank, validate=validate)
+
     def argmax_step(self, audio_rows, text_rows, return_margin: bool = False, **kw):
         """argmax(single_forward(audio_rows, text_rows), -1) for a batch of rows in fp32 (decode step)."""
         from .functional import joint_argmax

@@ -45,6 +45,20 @@ class RNNTModel(torch.nn.Module):
                                input_id_lens.int(), blank=-1, clamp=-1, reduction="mean")
 
     @torch.no_grad()
+    def align(self, mel_features, mel_feature_lens, input_ids, input_id_lens, blank_idx: int):
+        """Forced alignment of the transcripts `input_ids`: the inputs and steps of `forward` (blank prepend, predictor,
+        the encoder's permuted view, calc_output_lens), then `JointNetwork.align`.  Returns an `Alignment`: per
+        utterance the frame of each token on the best path, the path's log-probability and log P(transcript | audio).
+        The modules run in their current mode (call eval() to align without dropout)."""
+        prepended = torch.cat([torch.full((input_ids.shape[0], 1), blank_idx, dtype=input_ids.dtype,
+                                          device=input_ids.device), input_ids], dim=1)
+        decoder_features = self.predictor(prepended)
+        audio_features = self.encoder(mel_features).permute(0, 2, 1)
+        audio_feature_lens = self.encoder.calc_output_lens(mel_feature_lens)
+        return self.joint.align(audio_features, decoder_features, input_ids.int(), audio_feature_lens.int(),
+                                input_id_lens.int(), blank=-1)
+
+    @torch.no_grad()
     def greedy_decode_features(self, audio_features, audio_feature_lens, max_length: int = 200,
                                max_outputs_per_step: int = 10, return_margins: bool = False,
                                use_cuda_graph: bool = True, sync_every: int = 16, engine: str = "kernel"):
