@@ -237,6 +237,12 @@ int rnnt_b200_beam_decode(const float* enc, int64_t enc_sb, int64_t enc_st, cons
  *   fwd:  y[M,N] = x[M,K] . W[N,K]^T + bias[N]        (M = B*T or B*U1 rows, K = in features, N = hidden_features)
  *   bwd:  dx[M,K] = dy . W,  dW[N,K] = dy^T . x,  db[N] = column sums of dy;  any of dx / dW / db may be NULL (skipped)
  * Operands are rounded to fp16, accumulation is fp32.  K and N must be multiples of 8.  flags: RNNT_B200_DETERMINISTIC.
+ * x and W are rounded as they are: they must stay below 65504 in magnitude, and entries under 2^-14 lose relative
+ * precision (fp16 subnormals).  dy is rounded as dy * S, S the exact power of two with max|dy| S in [2^11, 2^12) (found
+ * on the device; S = 1 when max|dy| is 0, inf or NaN), and the results are multiplied by 1/S, so dx, dW and db keep
+ * the same relative precision at any gradient scale; an inf / NaN at dy[m][n] makes row m of dx, row n of dW and db[n]
+ * non-finite, as in fp32.  Deterministic mode sums dW and db in 64-bit fixed point of the S-scaled values (2^-26 units:
+ * M max|x| must stay below 2^25).
  * workspace: rnnt_b200_linear_workspace_bytes(M, K, N, backward, flags) bytes, 256-byte aligned. */
 size_t rnnt_b200_linear_workspace_bytes(int64_t M, int K, int N, int backward, int flags);
 int rnnt_b200_linear_fwd(const float* x, const float* W, const float* bias, int64_t M, int K, int N, float* y,

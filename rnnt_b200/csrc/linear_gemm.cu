@@ -8,6 +8,12 @@
 // views -- no transposed copies.  Operands are rounded to fp16 (RN, one elementwise pass; the joint GEMM rounds
 // tanh(enc + pred) to fp16 right afterwards anyway), accumulation is fp32 in TMEM.
 //
+// dy is rounded as dy * S, with S the exact power of two that puts max|dy| S in [2^11, 2^12) -- the fused backward's
+// rule for its logit-gradients (common.cuh kGradShift) -- so that the gradient keeps fp16's full relative precision
+// whatever its scale (mean reductions, loss scaling); the epilogues multiply by 1/S, which is exact.  S is derived on
+// the device from a max-abs pass over dy (no host synchronisation); it is 1 when max|dy| is 0 or not finite, so zeros
+// stay zeros and inf / NaN propagate.  x and W are rounded as they are.
+//
 // Persistent single-CTA tiles of 128 x 128 (cta_group::1): warp 0 TMA loader (4-stage ring of 16 KB + 16 KB), warp 1
 // tcgen05.mma issuer with two ping-pong accumulators, warps 2-5 epilogue (thread = output row; bias, fp32 stores, or
 // vector reductions when the contraction is split over CTAs).  These GEMMs are ~1 % of the step (27 GFLOP each at the
@@ -44,7 +50,9 @@ struct LinArgs {
   long long ldo;
   const float* bias;       // [N] added in the epilogue (may be nullptr)
   int ksplit;              // > 1: the contraction is split over CTAs and partial tiles are added with red.global
-  long long* out_fx;       // deterministic split: 64-bit fixed-point accumulation instead (may be nullptr)
+  long long* out_fx;       // deterministic split: 64-bit fixed-point accumulation of the S-scaled partials instead
+                           // (may be nullptr); a non-finite partial goes to `out` (zeroed) with an fp32 atomic instead
+  const float* inv_scale;  // 1/S of dy (backward), applied to the products; nullptr: 1 (forward)
 };
 
 template <bool A_MN, bool B_MN>
@@ -131,6 +139,7 @@ linear_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
   } else {
     const int lane_grp = warp & 3;
     const int row = lane_grp * 32 + lane;
+    const float post = p.inv_scale ? *p.inv_scale : 1.f;
     uint32_t ic = 0;
     for (int item = blockIdx.x; item < nitems; item += gridDim.x, ++ic) {
       int m0, n0, kc0, kc1;
@@ -150,11 +159,16 @@ linear_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
           if (p.out_fx) {
             long long* dst = p.out_fx + static_cast<long long>(m) * p.N + col0;
 #pragma unroll
-            for (int e = 0; e < 32; ++e)
-              if (col0 + e < p.N) fx_add(dst + e, v[e]);
+            for (int e = 0; e < 32; ++e) {
+              if (col0 + e >= p.N) continue;
+              if (isfinite(v[e])) fx_add(dst + e, v[e]);
+              else atomicAdd(p.out + static_cast<long long>(m) * p.ldo + col0 + e, v[e]);   // inf / NaN reach the output
+            }
             continue;
           }
           float* dst = p.out + static_cast<long long>(m) * p.ldo + col0;
+#pragma unroll
+          for (int e = 0; e < 32; ++e) v[e] *= post;
           const bool vec = (p.ldo & 3) == 0 && col0 + 32 <= p.N;
           if (p.bias && kc0 == 0) {
 #pragma unroll
@@ -189,21 +203,66 @@ linear_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
   tmem_teardown<false>(warp, tmem_base, kLinTmemCols);
 }
 
-__global__ void f32_to_f16_kernel(const float* __restrict__ src, __half* __restrict__ dst, long long n) {
+// Scale of dy, kept in 256 bytes of the backward workspace: [0] max|dy| as the bits of a non-negative float (unsigned
+// order = float order, NaN above inf), [1] S, [2] 1/S.
+// S = 2^(kGradShift - e) for max|dy| = m 2^e, m in [0.5, 1): max|dy| S in [2^11, 2^12) (the exponent is capped at 126,
+// so that 1/S stays a normal fp32 number for subnormal maxima); S = 1 when max|dy| is 0, inf or NaN.
+__device__ __forceinline__ float dy_scale(uint32_t max_bits) {
+  if (max_bits == 0u || max_bits >= 0x7f800000u) return 1.f;
+  int e;
+  frexpf(__uint_as_float(max_bits), &e);
+  return ldexpf(1.f, min(kGradShift - e, 126));
+}
+
+__device__ __forceinline__ uint32_t abs_bits(float x) { return __float_as_uint(x) & 0x7fffffffu; }
+
+// max_bits = max over src of |src|'s bit pattern: one atomicMax per block (the slot is zeroed beforehand)
+__global__ void absmax_kernel(const float* __restrict__ src, long long n, uint32_t* __restrict__ max_bits) {
+  __shared__ uint32_t red[8];
+  uint32_t mx = 0;
+  const long long n4 = n >> 2;
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < n4;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const float4 v = __ldg(reinterpret_cast<const float4*>(src) + i);
+    mx = max(mx, max(max(abs_bits(v.x), abs_bits(v.y)), max(abs_bits(v.z), abs_bits(v.w))));
+  }
+  if (blockIdx.x == 0 && threadIdx.x < (n & 3)) mx = max(mx, abs_bits(src[(n4 << 2) + threadIdx.x]));
+  mx = __reduce_max_sync(0xffffffffu, mx);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = mx;
+  __syncthreads();
+  if (threadIdx.x < 32) {
+    mx = threadIdx.x < (blockDim.x >> 5) ? red[threadIdx.x] : 0u;
+    mx = __reduce_max_sync(0xffffffffu, mx);
+    if (threadIdx.x == 0) atomicMax(max_bits, mx);
+  }
+}
+
+// dst = fp16(src * S).  With `scale` (dy's): S = dy_scale(scale[0]), and block 0 stores S, 1/S in scale[1], scale[2]
+// for the kernels that follow.  Without it S = 1 (x, W).  Multiplying by S is exact.
+__global__ void f32_to_f16_kernel(const float* __restrict__ src, __half* __restrict__ dst, long long n,
+                                  float* __restrict__ scale) {
+  float S = 1.f;
+  if (scale) {
+    S = dy_scale(__float_as_uint(scale[0]));
+    if (blockIdx.x == 0 && threadIdx.x == 0) { scale[1] = S; scale[2] = 1.f / S; }
+  }
   const long long n4 = n >> 2;
   for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < n4;
        i += static_cast<long long>(gridDim.x) * blockDim.x) {
     const float4 v = __ldg(reinterpret_cast<const float4*>(src) + i);
     uint2 o;
-    o.x = pack_f16x2(v.x, v.y);
-    o.y = pack_f16x2(v.z, v.w);
+    o.x = pack_f16x2(v.x * S, v.y * S);
+    o.y = pack_f16x2(v.z * S, v.w * S);
     reinterpret_cast<uint2*>(dst)[i] = o;
   }
-  if (blockIdx.x == 0 && threadIdx.x < (n & 3)) dst[(n4 << 2) + threadIdx.x] = __float2half_rn(src[(n4 << 2) + threadIdx.x]);
+  if (blockIdx.x == 0 && threadIdx.x < (n & 3))
+    dst[(n4 << 2) + threadIdx.x] = __float2half_rn(src[(n4 << 2) + threadIdx.x] * S);
 }
 
-// db[n] = sum_m dy[m][n]: block = 32 columns x 8 row lanes, rows strided over blockIdx.y; fixed-point or fp32 atomics
-__global__ void colsum_kernel(const float* __restrict__ dy, int M, int N, float* __restrict__ db, long long* db_fx) {
+// db[n] = sum_m dy[m][n] of the fp32 dy: block = 32 columns x 8 row lanes, rows strided over blockIdx.y; fp32 atomics,
+// or (deterministic) fixed-point atomics of the S-scaled block sums, a non-finite block sum going to db (zeroed) instead
+__global__ void colsum_kernel(const float* __restrict__ dy, int M, int N, float* __restrict__ db, long long* db_fx,
+                              const float* __restrict__ scale) {
   __shared__ float red[8][33];
   const int n = blockIdx.x * 32 + threadIdx.x;
   float acc = 0.f;
@@ -215,19 +274,23 @@ __global__ void colsum_kernel(const float* __restrict__ dy, int M, int N, float*
     float t = 0.f;
 #pragma unroll
     for (int i = 0; i < 8; ++i) t += red[i][threadIdx.x];
-    if (db_fx) fx_add(db_fx + n, t); else atomicAdd(db + n, t);
+    if (db_fx && isfinite(t)) fx_add(db_fx + n, t * scale[1]); else atomicAdd(db + n, t);
   }
 }
 
-__global__ void fx_to_f32_kernel(const long long* __restrict__ fx, float* __restrict__ out, long long n) {
+// deterministic mode: out = fx 2^-26 / S + out, where out holds the (zeroed) sum of the non-finite partials -- adding
+// +0 is exact, so a finite result depends on the fixed-point sum alone (as in finalize_fixed_kernel)
+__global__ void fx_to_f32_kernel(const long long* __restrict__ fx, float* __restrict__ out, long long n,
+                                 const float* __restrict__ scale) {
+  const double mul = kFxInv * static_cast<double>(scale[2]);
   for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < n;
        i += static_cast<long long>(gridDim.x) * blockDim.x)
-    out[i] = static_cast<float>(static_cast<double>(fx[i]) * kFxInv);
+    out[i] = static_cast<float>(static_cast<double>(fx[i]) * mul) + out[i];
 }
 
-int to_f16(const float* src, __half* dst, long long n, cudaStream_t stream) {
+int to_f16(const float* src, __half* dst, long long n, cudaStream_t stream, float* scale = nullptr) {
   const int grid = static_cast<int>(std::min<long long>((n / 4 + 255) / 256 + 1, 148 * 8));
-  f32_to_f16_kernel<<<grid, 256, 0, stream>>>(src, dst, n);
+  f32_to_f16_kernel<<<grid, 256, 0, stream>>>(src, dst, n, scale);
   RB_CUDA_CHECK(cudaGetLastError());
   return 0;
 }
@@ -259,7 +322,7 @@ inline size_t al(size_t x) { return (x + 255) & ~static_cast<size_t>(255); }
 size_t linear_workspace_bytes(long long M, int K, int N, bool backward, bool deterministic) {
   size_t b = al(static_cast<size_t>(M) * K * 2) + al(static_cast<size_t>(N) * K * 2);
   if (backward) {
-    b += al(static_cast<size_t>(M) * N * 2);
+    b += al(static_cast<size_t>(M) * N * 2) + al(3 * sizeof(float));       // dy16, dy's scale
     if (deterministic) b += al((static_cast<size_t>(N) * K + N) * 8);
   }
   return b;
@@ -277,6 +340,7 @@ int launch_linear_fwd(const float* x, const float* W, const float* bias, long lo
   if (rc) return rc;
   LinArgs a{};
   a.M = static_cast<int>(M); a.N = N; a.K = K; a.out = y; a.ldo = N; a.bias = bias; a.ksplit = 1; a.out_fx = nullptr;
+  a.inv_scale = nullptr;
   return launch_linear<false, false>(x16, w16, a, stream);       // y = x . W^T : both operands K-major
 }
 
@@ -288,14 +352,20 @@ int launch_linear_bwd(const float* x, const float* W, const float* dy, long long
   __half* x16 = reinterpret_cast<__half*>(ws + off); off += al(static_cast<size_t>(M) * K * 2);
   __half* w16 = reinterpret_cast<__half*>(ws + off); off += al(static_cast<size_t>(N) * K * 2);
   __half* dy16 = reinterpret_cast<__half*>(ws + off); off += al(static_cast<size_t>(M) * N * 2);
+  float* scale = reinterpret_cast<float*>(ws + off); off += al(3 * sizeof(float));
   long long* fx = deterministic ? reinterpret_cast<long long*>(ws + off) : nullptr;
-  int rc = to_f16(dy, dy16, M * N, stream);
+  RB_CUDA_CHECK(cudaMemsetAsync(scale, 0, sizeof(float), stream));
+  const int grid_max = static_cast<int>(std::min<long long>((M * N / 4 + 255) / 256 + 1, 148 * 4));
+  absmax_kernel<<<grid_max, 256, 0, stream>>>(dy, M * N, reinterpret_cast<uint32_t*>(scale));
+  RB_CUDA_CHECK(cudaGetLastError());
+  int rc = to_f16(dy, dy16, M * N, stream, scale);
   if (rc) return rc;
   if (dx) {         // dx[M,K] = dy[M,N] . W[N,K]: A = dy (K-major over N), B(k', n) = W[n][k'] = MN-major view of W
     rc = to_f16(W, w16, static_cast<long long>(N) * K, stream);
     if (rc) return rc;
     LinArgs a{};
     a.M = static_cast<int>(M); a.N = K; a.K = N; a.out = dx; a.ldo = K; a.bias = nullptr; a.ksplit = 1; a.out_fx = nullptr;
+    a.inv_scale = scale + 2;
     rc = launch_linear<false, true>(dy16, w16, a, stream);
     if (rc) return rc;
   }
@@ -303,35 +373,37 @@ int launch_linear_bwd(const float* x, const float* W, const float* dy, long long
     rc = to_f16(x, x16, M * K, stream);
     if (rc) return rc;
     LinArgs a{};
-    a.M = N; a.N = K; a.K = static_cast<int>(M); a.out = dW; a.ldo = K; a.bias = nullptr;
+    a.M = N; a.N = K; a.K = static_cast<int>(M); a.out = dW; a.ldo = K; a.bias = nullptr; a.inv_scale = scale + 2;
     const long long tiles = static_cast<long long>((N + kLinTile - 1) / kLinTile) * ((K + kLinTile - 1) / kLinTile);
     const long long nkc = (M + kBK - 1) / kBK;
     a.ksplit = static_cast<int>(std::max<long long>(1, std::min<long long>(device_sm_count() / std::max<long long>(1, tiles), nkc)));
     a.out_fx = nullptr;
+    // Deterministic fixed point: a split-K partial is at most 2^12 (max|dy| S) * M * max|x16| in S-scaled units, and in
+    // 2^-26 units it must stay below 2^63, i.e. M max|x16| < 2^25 (M = 12800 rows allow |x| up to 2600).  The
+    // resolution is relative to dy's scale: 2^-27 / S per partial, at most 2^-38 max|dy|.
     if (a.ksplit > 1) {
       if (deterministic) {
         a.out_fx = fx;
         RB_CUDA_CHECK(cudaMemsetAsync(fx, 0, static_cast<size_t>(N) * K * 8, stream));
-      } else {
-        RB_CUDA_CHECK(cudaMemsetAsync(dW, 0, static_cast<size_t>(N) * K * 4, stream));
       }
+      RB_CUDA_CHECK(cudaMemsetAsync(dW, 0, static_cast<size_t>(N) * K * 4, stream));
     }
     rc = launch_linear<true, true>(dy16, x16, a, stream);
     if (rc) return rc;
     if (a.out_fx) {
-      fx_to_f32_kernel<<<148 * 4, 256, 0, stream>>>(fx, dW, static_cast<long long>(N) * K);
+      fx_to_f32_kernel<<<148 * 4, 256, 0, stream>>>(fx, dW, static_cast<long long>(N) * K, scale);
       RB_CUDA_CHECK(cudaGetLastError());
     }
   }
-  if (db) {
+  if (db) {        // fixed point as for dW with |x16| = 1: M < 2^25 rows
     long long* fxb = deterministic ? fx + static_cast<size_t>(N) * K : nullptr;
     if (fxb) RB_CUDA_CHECK(cudaMemsetAsync(fxb, 0, static_cast<size_t>(N) * 8, stream));
-    else RB_CUDA_CHECK(cudaMemsetAsync(db, 0, static_cast<size_t>(N) * 4, stream));
+    RB_CUDA_CHECK(cudaMemsetAsync(db, 0, static_cast<size_t>(N) * 4, stream));
     const int gy = static_cast<int>(std::max<long long>(1, std::min<long long>((M + 63) / 64, 64)));
-    colsum_kernel<<<dim3((N + 31) / 32, gy), dim3(32, 8), 0, stream>>>(dy, static_cast<int>(M), N, db, fxb);
+    colsum_kernel<<<dim3((N + 31) / 32, gy), dim3(32, 8), 0, stream>>>(dy, static_cast<int>(M), N, db, fxb, scale);
     RB_CUDA_CHECK(cudaGetLastError());
     if (fxb) {
-      fx_to_f32_kernel<<<1, 256, 0, stream>>>(fxb, db, N);
+      fx_to_f32_kernel<<<1, 256, 0, stream>>>(fxb, db, N, scale);
       RB_CUDA_CHECK(cudaGetLastError());
     }
   }
