@@ -241,7 +241,9 @@ def test_beam_one_matches_greedy_at_full_width():
 
 
 # (H, V, E, blank, K, T, lens, max_len, seed, scale, blank_bias): small odd sizes, blank at either end, ragged lengths
-# with T_b = 0 and 1, and max_length reached mid-utterance; then a few utterances at full width
+# with T_b = 0 and 1, and max_length reached mid-utterance; then a few utterances at full width, and two shapes whose
+# weights do not all fit in shared memory on 148 SMs (tests/decode_oracle.py::smem_plan): the joint read from L2
+# (V = 4096), and conv2 read from L2 with its tap GEMV and the conv1 table over two K-chunks (E = 1024)
 ORACLE_CASES = {
     "v29_k2": (36, 29, 36, 28, 2, 12, [12, 0, 1, 9, 5], 40, 1, 3.0, 0.0),
     "v33_k4_blank0": (36, 33, 36, 0, 4, 12, [12, 1, 0, 7, 11], 40, 7, 3.0, 0.0),
@@ -249,6 +251,8 @@ ORACLE_CASES = {
     "v33_k8_cap": (36, 33, 36, 32, 8, 10, [10, 0, 3, 8, 1], 6, 47, 3.0, -1.0),
     "v33_k2_cap": (36, 33, 36, 32, 2, 12, [12, 11, 0, 1, 4], 4, 5, 3.0, -2.0),
     "full_k4": (1024, 1024, 512, 1023, 4, 16, [16, 12, 9], 200, 6, 3.0, 2.5),
+    "joint_streamed_k4": (1024, 4096, 512, 4095, 4, 12, [12, 10, 7], 200, 27, 3.0, 2.5),
+    "conv2_streamed_k4": (1024, 1024, 1024, 1023, 4, 12, [12, 10, 7], 200, 22, 3.0, 2.5),
 }
 
 
