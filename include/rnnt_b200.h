@@ -232,6 +232,62 @@ int rnnt_b200_beam_decode(const float* enc, int64_t enc_sb, int64_t enc_st, cons
                           const float* ln2_b, int B, int T, int H, int V, int E, int blank, int beam, int max_len,
                           int32_t* tokens, int32_t* n_tokens, float* scores, void* scratch, void* stream);
 
+/* Token timing and confidence: the three decode entries with per-token frames and log-probabilities.  Each _aligned
+ * entry takes the arguments of its plain entry, then its new outputs; any of them may be NULL.  The plain entries are
+ * these calls with NULL outputs: same checks, same error codes, same tokens, n_tokens, margins and beam scores.
+ *
+ * Greedy (rnnt_b200_greedy_decode_aligned, rnnt_b200_greedy_decode_stream_aligned).  Every step of utterance b runs
+ * at a frame t and computes fp32 logits x; logp = x - (max(x) + log sum_v exp(x_v - max(x))), the sum taken in a fixed
+ * order (thread-strided partial sums, then a fixed block reduction).
+ *   - Emitting step: token k (1-based, the seed blank excluded) gets frames[b, k-1] = t, token_logp[b, k-1] =
+ *     logp[tok].  frames and token_logp are (B, max_len), laid out like tokens.
+ *   - Advancing step (a step that leaves the frame, on blank or because the max_per_frame cap fired): adds logp[blank]
+ *     to the path score, even when the argmax was not blank -- the lattice's blank edge.
+ *   - scores (B) fp32: the sum of these terms in step order.  For an utterance that ran to T_b it is the
+ *     log-probability of the greedy path through the (t, u) lattice, final blank included: the path sum that
+ *     rnnt_b200_viterbi maximises.  When max_len stopped the utterance (n_tokens == max_len) it covers the steps taken.
+ *     T_b = 0 gives 0; a row with no finite maximum gives NaN, as for the argmax.
+ *   - Streaming: frames count from the slot's last reset, not from the start of the call; frames and token_logp are
+ *     caller-owned arrays kept between calls, indexed like tokens; scores[b] after a call is the running path score
+ *     since the reset.  The per-slot frame base and running score live in the state (after the regions the one-shot
+ *     scratch also has), and every call of either stream entry maintains them, so plain and _aligned calls can be mixed
+ *     on one state.
+ *
+ * Beam (rnnt_b200_beam_decode_aligned).  Each hypothesis carries, per token, the frame of its extension step and
+ * logp[v] of that step, where logp = logits - lse of the extending hypothesis at that frame.  When two candidates with
+ * equal token lists merge (h's blank continuation and q's extension), the score stays their logaddexp and the merged
+ * hypothesis takes the frames and log-probabilities of the constituent with the larger term, s_h + logp_h[blank]
+ * against s_q + logp_q[last]; on an exact tie the blank continuation's, so the token keeps its earlier frame.
+ * frames and token_logp are (B, K, max_len), laid out like tokens.  rnnt_b200_beam_decode_scratch_bytes covers both
+ * entries; when both new outputs are NULL the kernel skips the lists.
+ *
+ * All outputs are bit-identical run to run and do not depend on the batch position; the streaming outputs do not
+ * depend on how an utterance is cut into chunks. */
+int rnnt_b200_greedy_decode_aligned(const float* enc, int64_t enc_sb, int64_t enc_st, const int32_t* T_len,
+                                    const float* joint_w, const float* joint_b, const float* emb, const float* ln1_w,
+                                    const float* ln1_b, const float* conv1_w, const float* conv1_b,
+                                    const float* conv2_w, const float* conv2_b, const float* lin_w, const float* lin_b,
+                                    const float* ln2_w, const float* ln2_b, int B, int T, int H, int V, int E,
+                                    int blank, int max_len, int max_per_frame, int32_t* tokens, int32_t* n_tokens,
+                                    float* margins_out, void* scratch, void* stream, int32_t* frames,
+                                    float* token_logp, float* scores);
+int rnnt_b200_greedy_decode_stream_aligned(const float* enc, int64_t enc_sb, int64_t enc_st,
+                                           const int32_t* chunk_len, const int32_t* reset, const float* joint_w,
+                                           const float* joint_b, const float* emb, const float* ln1_w,
+                                           const float* ln1_b, const float* conv1_w, const float* conv1_b,
+                                           const float* conv2_w, const float* conv2_b, const float* lin_w,
+                                           const float* lin_b, const float* ln2_w, const float* ln2_b, int B, int Tc,
+                                           int H, int V, int E, int blank, int max_len, int max_per_frame,
+                                           int32_t* tokens, int32_t* n_tokens, float* margins_out, void* state,
+                                           void* stream, int32_t* frames, float* token_logp, float* scores);
+int rnnt_b200_beam_decode_aligned(const float* enc, int64_t enc_sb, int64_t enc_st, const int32_t* T_len,
+                                  const float* joint_w, const float* joint_b, const float* emb, const float* ln1_w,
+                                  const float* ln1_b, const float* conv1_w, const float* conv1_b, const float* conv2_w,
+                                  const float* conv2_b, const float* lin_w, const float* lin_b, const float* ln2_w,
+                                  const float* ln2_b, int B, int T, int H, int V, int E, int blank, int beam,
+                                  int max_len, int32_t* tokens, int32_t* n_tokens, float* scores, void* scratch,
+                                  void* stream, int32_t* frames, float* token_logp);
+
 /* Optional pre-projections of the joint (rnnt/joint.py:8-12, 26-30: audio_ln / text_ln of the non-"convjs" configs) as
  * tcgen05 GEMMs ahead of the fused call, with their backward.  Row-major contiguous fp32 tensors:
  *   fwd:  y[M,N] = x[M,K] . W[N,K]^T + bias[N]        (M = B*T or B*U1 rows, K = in features, N = hidden_features)

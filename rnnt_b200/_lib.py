@@ -47,6 +47,13 @@ _SIGNATURES = {
     "rnnt_b200_beam_decode_scratch_bytes": (C.c_size_t, [C.c_int] * 6),
     "rnnt_b200_beam_decode": (C.c_int, [_f32p, C.c_int64, C.c_int64, _i32p] + [_f32p] * 13 + [C.c_int] * 8
                               + [_i32p, _i32p, _f32p, _ptr, _ptr]),
+    "rnnt_b200_greedy_decode_aligned": (C.c_int, [_f32p, C.c_int64, C.c_int64, _i32p] + [_f32p] * 13
+                                        + [C.c_int] * 8 + [_i32p, _i32p, _f32p, _ptr, _ptr, _i32p, _f32p, _f32p]),
+    "rnnt_b200_greedy_decode_stream_aligned": (C.c_int, [_f32p, C.c_int64, C.c_int64, _i32p, _i32p] + [_f32p] * 13
+                                               + [C.c_int] * 8 + [_i32p, _i32p, _f32p, _ptr, _ptr, _i32p, _f32p,
+                                                                  _f32p]),
+    "rnnt_b200_beam_decode_aligned": (C.c_int, [_f32p, C.c_int64, C.c_int64, _i32p] + [_f32p] * 13 + [C.c_int] * 8
+                                      + [_i32p, _i32p, _f32p, _ptr, _ptr, _i32p, _f32p]),
     "rnnt_b200_linear_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int]),
     "rnnt_b200_linear_fwd": (C.c_int, [_f32p, _f32p, _f32p, C.c_int64, C.c_int, C.c_int, _f32p, _ptr, C.c_size_t, _ptr]),
     "rnnt_b200_linear_bwd": (C.c_int, [_f32p, _f32p, _f32p, C.c_int64, C.c_int, C.c_int, _f32p, _f32p, _f32p, C.c_int,

@@ -451,13 +451,14 @@ rb::DecodeArgs decode_args(const float* joint_w, const float* joint_b, const flo
 
 }  // namespace
 
-int rnnt_b200_greedy_decode(const float* enc, int64_t enc_sb, int64_t enc_st, const int32_t* T_len,
-                            const float* joint_w, const float* joint_b, const float* emb, const float* ln1_w,
-                            const float* ln1_b, const float* conv1_w, const float* conv1_b, const float* conv2_w,
-                            const float* conv2_b, const float* lin_w, const float* lin_b, const float* ln2_w,
-                            const float* ln2_b, int B, int T, int H, int V, int E, int blank, int max_len,
-                            int max_per_frame, int32_t* tokens, int32_t* n_tokens, float* margins_out, void* scratch,
-                            void* stream) {
+int rnnt_b200_greedy_decode_aligned(const float* enc, int64_t enc_sb, int64_t enc_st, const int32_t* T_len,
+                                    const float* joint_w, const float* joint_b, const float* emb, const float* ln1_w,
+                                    const float* ln1_b, const float* conv1_w, const float* conv1_b,
+                                    const float* conv2_w, const float* conv2_b, const float* lin_w, const float* lin_b,
+                                    const float* ln2_w, const float* ln2_b, int B, int T, int H, int V, int E,
+                                    int blank, int max_len, int max_per_frame, int32_t* tokens, int32_t* n_tokens,
+                                    float* margins_out, void* scratch, void* stream, int32_t* frames,
+                                    float* token_logp, float* scores) {
   RB_REQUIRE(T > 0, -1, "invalid shape");
   if (int rc = check_decode(B, T, H, V, E, blank, max_len, max_per_frame, enc_sb, enc_st, scratch)) return rc;
   // one launch: build the tables, reset every slot, consume the whole utterance
@@ -467,7 +468,22 @@ int rnnt_b200_greedy_decode(const float* enc, int64_t enc_sb, int64_t enc_st, co
   a.init = 1; a.reset_all = 1; a.reset = nullptr;
   a.blank = blank; a.max_len = max_len; a.max_per_frame = max_per_frame; a.max_steps = T + max_len + 1;
   a.tokens = tokens; a.n_tokens = n_tokens; a.margins = margins_out;
+  a.frames = frames; a.token_logp = token_logp; a.path_scores = scores;
+  a.want_lp = token_logp != nullptr || scores != nullptr;
   return rb::launch_greedy_decode(a, static_cast<float*>(scratch), static_cast<cudaStream_t>(stream));
+}
+
+int rnnt_b200_greedy_decode(const float* enc, int64_t enc_sb, int64_t enc_st, const int32_t* T_len,
+                            const float* joint_w, const float* joint_b, const float* emb, const float* ln1_w,
+                            const float* ln1_b, const float* conv1_w, const float* conv1_b, const float* conv2_w,
+                            const float* conv2_b, const float* lin_w, const float* lin_b, const float* ln2_w,
+                            const float* ln2_b, int B, int T, int H, int V, int E, int blank, int max_len,
+                            int max_per_frame, int32_t* tokens, int32_t* n_tokens, float* margins_out, void* scratch,
+                            void* stream) {
+  return rnnt_b200_greedy_decode_aligned(enc, enc_sb, enc_st, T_len, joint_w, joint_b, emb, ln1_w, ln1_b, conv1_w,
+                                         conv1_b, conv2_w, conv2_b, lin_w, lin_b, ln2_w, ln2_b, B, T, H, V, E, blank,
+                                         max_len, max_per_frame, tokens, n_tokens, margins_out, scratch, stream,
+                                         nullptr, nullptr, nullptr);
 }
 
 int rnnt_b200_greedy_decode_stream_init(const float* joint_w, const float* joint_b, const float* emb,
@@ -483,13 +499,15 @@ int rnnt_b200_greedy_decode_stream_init(const float* joint_w, const float* joint
   return rb::launch_greedy_decode(a, static_cast<float*>(state), static_cast<cudaStream_t>(stream));
 }
 
-int rnnt_b200_greedy_decode_stream(const float* enc, int64_t enc_sb, int64_t enc_st, const int32_t* chunk_len,
-                                   const int32_t* reset, const float* joint_w, const float* joint_b, const float* emb,
-                                   const float* ln1_w, const float* ln1_b, const float* conv1_w, const float* conv1_b,
-                                   const float* conv2_w, const float* conv2_b, const float* lin_w, const float* lin_b,
-                                   const float* ln2_w, const float* ln2_b, int B, int Tc, int H, int V, int E,
-                                   int blank, int max_len, int max_per_frame, int32_t* tokens, int32_t* n_tokens,
-                                   float* margins_out, void* state, void* stream) {
+int rnnt_b200_greedy_decode_stream_aligned(const float* enc, int64_t enc_sb, int64_t enc_st,
+                                           const int32_t* chunk_len, const int32_t* reset, const float* joint_w,
+                                           const float* joint_b, const float* emb, const float* ln1_w,
+                                           const float* ln1_b, const float* conv1_w, const float* conv1_b,
+                                           const float* conv2_w, const float* conv2_b, const float* lin_w,
+                                           const float* lin_b, const float* ln2_w, const float* ln2_b, int B, int Tc,
+                                           int H, int V, int E, int blank, int max_len, int max_per_frame,
+                                           int32_t* tokens, int32_t* n_tokens, float* margins_out, void* state,
+                                           void* stream, int32_t* frames, float* token_logp, float* scores) {
   if (int rc = check_decode(B, Tc, H, V, E, blank, max_len, max_per_frame, enc_sb, enc_st, state)) return rc;
   RB_REQUIRE(chunk_len != nullptr && tokens != nullptr && n_tokens != nullptr, -1,
              "decode stream: chunk_len, tokens and n_tokens are required");
@@ -501,7 +519,22 @@ int rnnt_b200_greedy_decode_stream(const float* enc, int64_t enc_sb, int64_t enc
   // steps of one launch: every step of a slot either consumes a frame or emits a token
   a.max_steps = static_cast<int>(Tc + std::min<int64_t>(static_cast<int64_t>(Tc) * max_per_frame, max_len - 1) + 1);
   a.tokens = tokens; a.n_tokens = n_tokens; a.margins = margins_out;
+  // the running path score lives in the state: every call keeps it, so plain and aligned calls can share a state
+  a.frames = frames; a.token_logp = token_logp; a.path_scores = scores; a.want_lp = 1;
   return rb::launch_greedy_decode(a, static_cast<float*>(state), static_cast<cudaStream_t>(stream));
+}
+
+int rnnt_b200_greedy_decode_stream(const float* enc, int64_t enc_sb, int64_t enc_st, const int32_t* chunk_len,
+                                   const int32_t* reset, const float* joint_w, const float* joint_b, const float* emb,
+                                   const float* ln1_w, const float* ln1_b, const float* conv1_w, const float* conv1_b,
+                                   const float* conv2_w, const float* conv2_b, const float* lin_w, const float* lin_b,
+                                   const float* ln2_w, const float* ln2_b, int B, int Tc, int H, int V, int E,
+                                   int blank, int max_len, int max_per_frame, int32_t* tokens, int32_t* n_tokens,
+                                   float* margins_out, void* state, void* stream) {
+  return rnnt_b200_greedy_decode_stream_aligned(enc, enc_sb, enc_st, chunk_len, reset, joint_w, joint_b, emb, ln1_w,
+                                                ln1_b, conv1_w, conv1_b, conv2_w, conv2_b, lin_w, lin_b, ln2_w, ln2_b,
+                                                B, Tc, H, V, E, blank, max_len, max_per_frame, tokens, n_tokens,
+                                                margins_out, state, stream, nullptr, nullptr, nullptr);
 }
 
 size_t rnnt_b200_beam_decode_scratch_bytes(int B, int K, int H, int V, int E, int max_len) {
@@ -509,12 +542,13 @@ size_t rnnt_b200_beam_decode_scratch_bytes(int B, int K, int H, int V, int E, in
   return rb::beam_decode_scratch_bytes(B, K, H, V, E, max_len);
 }
 
-int rnnt_b200_beam_decode(const float* enc, int64_t enc_sb, int64_t enc_st, const int32_t* T_len,
-                          const float* joint_w, const float* joint_b, const float* emb, const float* ln1_w,
-                          const float* ln1_b, const float* conv1_w, const float* conv1_b, const float* conv2_w,
-                          const float* conv2_b, const float* lin_w, const float* lin_b, const float* ln2_w,
-                          const float* ln2_b, int B, int T, int H, int V, int E, int blank, int beam, int max_len,
-                          int32_t* tokens, int32_t* n_tokens, float* scores, void* scratch, void* stream) {
+int rnnt_b200_beam_decode_aligned(const float* enc, int64_t enc_sb, int64_t enc_st, const int32_t* T_len,
+                                  const float* joint_w, const float* joint_b, const float* emb, const float* ln1_w,
+                                  const float* ln1_b, const float* conv1_w, const float* conv1_b, const float* conv2_w,
+                                  const float* conv2_b, const float* lin_w, const float* lin_b, const float* ln2_w,
+                                  const float* ln2_b, int B, int T, int H, int V, int E, int blank, int beam,
+                                  int max_len, int32_t* tokens, int32_t* n_tokens, float* scores, void* scratch,
+                                  void* stream, int32_t* frames, float* token_logp) {
   RB_REQUIRE(T > 0, -1, "invalid shape");
   if (int rc = check_decode(B, T, H, V, E, blank, max_len, 0, enc_sb, enc_st, scratch)) return rc;
   RB_REQUIRE(beam >= 1 && beam <= rb::kMaxBeam, -1, "beam size must be in [1, %d] (got %d)", rb::kMaxBeam, beam);
@@ -526,7 +560,19 @@ int rnnt_b200_beam_decode(const float* enc, int64_t enc_sb, int64_t enc_st, cons
   a.enc = enc; a.enc_sb = enc_sb; a.enc_st = enc_st; a.T_len = T_len; a.T = T;
   a.blank = blank; a.max_len = max_len; a.K = beam;
   a.tokens = tokens; a.n_tokens = n_tokens; a.scores = scores;
+  a.frames = frames; a.token_logp = token_logp;
   return rb::launch_beam_decode(a, static_cast<float*>(scratch), static_cast<cudaStream_t>(stream));
+}
+
+int rnnt_b200_beam_decode(const float* enc, int64_t enc_sb, int64_t enc_st, const int32_t* T_len,
+                          const float* joint_w, const float* joint_b, const float* emb, const float* ln1_w,
+                          const float* ln1_b, const float* conv1_w, const float* conv1_b, const float* conv2_w,
+                          const float* conv2_b, const float* lin_w, const float* lin_b, const float* ln2_w,
+                          const float* ln2_b, int B, int T, int H, int V, int E, int blank, int beam, int max_len,
+                          int32_t* tokens, int32_t* n_tokens, float* scores, void* scratch, void* stream) {
+  return rnnt_b200_beam_decode_aligned(enc, enc_sb, enc_st, T_len, joint_w, joint_b, emb, ln1_w, ln1_b, conv1_w,
+                                       conv1_b, conv2_w, conv2_b, lin_w, lin_b, ln2_w, ln2_b, B, T, H, V, E, blank,
+                                       beam, max_len, tokens, n_tokens, scores, scratch, stream, nullptr, nullptr);
 }
 
 size_t rnnt_b200_linear_workspace_bytes(int64_t M, int K, int N, int backward, int flags) {

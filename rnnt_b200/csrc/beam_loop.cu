@@ -11,6 +11,7 @@
 //   P3  one CTA per live utterance, one warp per hypothesis: log-sum-exp, merge test, the top K extensions of the row
 //       that no merge takes; then the K(K+1)-candidate selection, the gather of every new hypothesis's state from its
 //       parent's slot into the other half of the double-buffered state, and conv1 of the extended ones
+//       (+ with token timing: each token's frame and log-probability, gathered with the token lists)
 // with a grid barrier after each phase: 5 per frame (P5 / P6 are skipped in a frame that extends nothing).  Every sum
 // runs in a fixed order and every selection is a total order, so results are bit-identical run to run and do not
 // depend on the batch an utterance sits in.
@@ -34,6 +35,9 @@ __device__ __forceinline__ float log_add_exp(float a, float b) {
   return m + log1pf(expf(-fabsf(a - b)));
 }
 
+// ALIGN: the instance that also keeps each token's frame and log-probability (frames or token_logp requested); the
+// plain decode runs the ALIGN = false instance, which has none of that code.
+template <bool ALIGN>
 __global__ void __launch_bounds__(kThreads, 1) beam_decode_kernel(BeamArgs p) {
   extern __shared__ __align__(16) float smem[];
   __shared__ float red[kThreads / 32];
@@ -48,6 +52,7 @@ __global__ void __launch_bounds__(kThreads, 1) beam_decode_kernel(BeamArgs p) {
   __shared__ int s_extv[kMaxBeam][kMaxBeam];
   __shared__ float c_sc[kMaxCand];
   __shared__ int c_key[kMaxCand];
+  __shared__ int c_dom[kMaxCand];       // merged candidates: the slot q whose extension dominates the merge, else -1
   __shared__ int s_sel[kMaxBeam];
   __shared__ int s_nsel;
   const int B = p.B, H = p.H, V = p.V, E = p.E, K = p.K, L = p.max_len;
@@ -101,6 +106,8 @@ __global__ void __launch_bounds__(kThreads, 1) beam_decode_kernel(BeamArgs p) {
   auto score = [&](int par) { return p.score + par * R; };
   auto hash = [&](int par) { return p.hash + par * R; };
   auto hyp = [&](int par, int r) { return p.hyp + (static_cast<long long>(par) * R + r) * L; };
+  auto hyp_fr = [&](int par, int r) { return p.hyp_fr + (static_cast<long long>(par) * R + r) * L; };
+  auto hyp_lp = [&](int par, int r) { return p.hyp_lp + (static_cast<long long>(par) * R + r) * L; };
   auto frames = [&](int b) { return max(0, min(__ldg(p.T_len + b), p.T)); };
 
   // ---- the initial beam {(empty, 0)}: slot 0 of every utterance holds the seed blank's predictor state (zero tap
@@ -304,14 +311,16 @@ __global__ void __launch_bounds__(kThreads, 1) beam_decode_kernel(BeamArgs p) {
       if (tid < nc) {
         const int hh = tid / (K + 1), i = tid % (K + 1) - 1;
         float sc = -INFINITY;
-        int key = 0x7fffffff;
+        int key = 0x7fffffff, dom = -1;
         if (i < 0) {
           const float* row = p.logits + static_cast<long long>(r0 + hh) * V;
           sc = s_sc[hh] + (__ldcg(row + p.blank) - s_lse[hh]);
           const int q = s_par[hh];
           if (q >= 0) {
             const float* rq = p.logits + static_cast<long long>(r0 + q) * V;
-            sc = log_add_exp(sc, s_sc[q] + (__ldcg(rq + s_last[hh]) - s_lse[q]));
+            const float sq = s_sc[q] + (__ldcg(rq + s_last[hh]) - s_lse[q]);
+            if (ALIGN && sq > sc) dom = q;   // the merge keeps the timing of its larger term; a tie keeps the blank's
+            sc = log_add_exp(sc, sq);
           }
           key = hh * V + p.blank;
         } else if (i < s_next[hh]) {
@@ -320,6 +329,7 @@ __global__ void __launch_bounds__(kThreads, 1) beam_decode_kernel(BeamArgs p) {
         }
         c_sc[tid] = sc;
         c_key[tid] = key;
+        if (ALIGN) c_dom[tid] = dom;
       }
       __syncthreads();
       // rank of each candidate in the selection order = number of candidates before it (a total order: keys differ)
@@ -335,6 +345,23 @@ __global__ void __launch_bounds__(kThreads, 1) beam_decode_kernel(BeamArgs p) {
       }
       __syncthreads();
       const int nsel = s_nsel;
+      // frames and log-probabilities of candidate c's token list: those of the constituent that dominates it (the
+      // source hypothesis, or for a merge whose extension term is larger, the extended slot q), plus this frame's token
+      auto copy_lists = [&](int c, int* dfr, float* dlp) {
+        const int src = c_key[c] / V, v = c_key[c] % V, q = c_dom[c];
+        const int base = q >= 0 ? q : src, nb = s_nt[base] - 1;
+        const int* sf = hyp_fr(cur, r0 + base);
+        const float* sl = hyp_lp(cur, r0 + base);
+        for (int i = tid; i < nb; i += kThreads) {
+          if (dfr) dfr[i] = __ldcg(sf + i);
+          if (dlp) dlp[i] = __ldcg(sl + i);
+        }
+        if (tid == 0 && (v != p.blank || q >= 0)) {
+          const int tok = q >= 0 ? s_last[src] : v;
+          if (dfr) dfr[nb] = t;
+          if (dlp) dlp[nb] = __ldcg(p.logits + static_cast<long long>(r0 + base) * V + tok) - s_lse[base];
+        }
+      };
       if (t == Tb - 1) {
         // last frame of the utterance: the new beam, best first, is the output
         for (int j = 0; j < K; ++j) {
@@ -354,6 +381,11 @@ __global__ void __launch_bounds__(kThreads, 1) beam_decode_kernel(BeamArgs p) {
             p.scores[o] = -INFINITY;
           }
         }
+        if (ALIGN)
+          for (int j = 0; j < nsel; ++j) {
+            const long long o = static_cast<long long>(r0 + j) * L;
+            copy_lists(s_sel[j], p.frames ? p.frames + o : nullptr, p.token_logp ? p.token_logp + o : nullptr);
+          }
       } else {
         // gather: new slot j takes its parent's state (always copied: parents may feed several slots), extended slots
         // then run conv1 on their new token; feats only matter for blank continuations (the others recompute it)
@@ -392,6 +424,8 @@ __global__ void __launch_bounds__(kThreads, 1) beam_decode_kernel(BeamArgs p) {
                          p.ynew + static_cast<long long>(rd) * E, E, nt);
           }
         }
+        if (ALIGN)
+          for (int j = 0; j < nsel; ++j) copy_lists(s_sel[j], hyp_fr(nxt, r0 + j), hyp_lp(nxt, r0 + j));
       }
       __syncthreads();
     }
@@ -410,7 +444,8 @@ size_t beam_decode_scratch_bytes(int B, int K, int H, int V, int E, int max_len)
   const size_t floats = 2 * pad4(r * H) /*feats x2*/ + 2 * pad4(r * H) /*hbuf, lin*/ + pad4(r * V) /*logits*/ +
                         2 * pad4(r * 3 * E) + 2 * pad4(r * 5 * E) + 2 * pad4(r * E) /*ynew, z*/ + pad4(2 * r) /*scores*/ +
                         pad4(static_cast<size_t>(V) * E) + pad4(static_cast<size_t>(V) * 3 * E) /*symbol tables*/;
-  const size_t ints = 2 * r /*ntok*/ + r /*emit*/ + 2 * r /*rows*/ + 16 + 2 * r * max_len /*token lists*/;
+  const size_t ints = 2 * r /*ntok*/ + r /*emit*/ + 2 * r /*rows*/ + 16 + 2 * r * max_len /*token lists*/ +
+                      4 * r * max_len /*their frames and log-probabilities*/;
   return kTimerBytes + kBarBytes + 2 * r * 8 + floats * 4 + ints * 4 + 256;
 }
 
@@ -447,13 +482,17 @@ int launch_beam_decode(BeamArgs a, float* scratch, cudaStream_t stream) {
   a.rows = ip; ip += 2 * r;
   a.flags = ip; ip += 16;
   a.hyp = ip; ip += 2 * r * a.max_len;
-  RB_CUDA_CHECK(cudaFuncSetAttribute(beam_decode_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  a.hyp_fr = ip; ip += 2 * r * a.max_len;
+  a.hyp_lp = reinterpret_cast<float*>(ip); ip += 2 * r * a.max_len;
+  void (*kernel)(BeamArgs) =
+      a.frames != nullptr || a.token_logp != nullptr ? beam_decode_kernel<true> : beam_decode_kernel<false>;
+  RB_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int per_sm = 0;
-  RB_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, beam_decode_kernel, kThreads, smem));
+  RB_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, smem));
   RB_REQUIRE(per_sm >= 1, -6, "decode kernel does not fit on an SM");
   void* args[] = {&a};
   // cooperative launch: guarantees that all CTAs are co-resident, which the kernel's own grid barrier relies on
-  RB_CUDA_CHECK(cudaLaunchCooperativeKernel(reinterpret_cast<void*>(beam_decode_kernel), dim3(grid), dim3(kThreads),
+  RB_CUDA_CHECK(cudaLaunchCooperativeKernel(reinterpret_cast<void*>(kernel), dim3(grid), dim3(kThreads),
                                             args, smem, stream));
   return 0;
 }

@@ -14,6 +14,7 @@
 //   P1  feats = LayerNorm(lin) for utterances that just emitted; h = tanh(enc[b, t_b] + feats[b])
 //   P2  logits[b, v] = W_j[v,:] . h[b,:] + b_j[v]        (CTA = its ~V/148 classes, warp = 4 rows, lanes split K; gemv_phase)
 //   P3  argmax (lowest index on ties) + top-2 margin, blank / max-per-frame rule, token append
+//       (+ with token timing: the row's log-sum-exp, the token's frame and log-probability, the running path score)
 //       conv1 of an emitted token, inside P3: its tap products W1_j . LN(emb[tok]) depend on the token alone, so they are a
 //       (symbols, 3E) TABLE built once at kernel start (1.6 GFLOP, ~3 decode steps' worth) -- the step adds three table
 //       rows to the utterance's tap accumulators and applies bias + GELU: no GEMV phase, no grid barrier for conv1
@@ -130,6 +131,7 @@ __global__ void __launch_bounds__(kThreads, 1) greedy_decode_kernel(DecodeArgs p
       const bool r = b < B && is_reset(b);
       if (b < B) {
         p.t_idx[b] = 0; p.per[b] = 0;
+        if (r || p.init) { p.frame_base[b] = 0; p.path_score[b] = 0.f; }
         if (r) { p.ntok[b] = 1; p.emit[b] = 1; p.last_tok[b] = p.blank; }
         else if (p.init) { p.ntok[b] = 0; p.emit[b] = 0; }
       }
@@ -244,13 +246,27 @@ __global__ void __launch_bounds__(kThreads, 1) greedy_decode_kernel(DecodeArgs p
       const int tok = static_cast<unsigned>(s_idx[0]) < static_cast<unsigned>(V) ? s_idx[0] : 0;
       const bool advance = (tok == p.blank) || (__ldcg(p.per + b) >= p.max_per_frame);
       const int nt_old = __ldcg(p.ntok + b);        // every thread reads it before thread 0 bumps it
+      // log-probability of the step's edge: logp = x - (max + log sum exp(x - max)), the sum thread-strided then
+      // block-reduced in a fixed order; the row was just read, so the second pass hits L2
+      float lp_step = 0.f;
+      if (p.want_lp) {
+        const float mx = s_best[0];
+        float s = 0.f;
+        for (int v = tid; v < V; v += kThreads) s += expf(__ldcg(row + v) - mx);
+        const float lse = mx + logf(block_sum(s, red));
+        lp_step = __ldcg(row + (advance ? p.blank : tok)) - lse;
+      }
       __syncthreads();
       if (tid == 0) {
         if (p.margins) p.margins[static_cast<long long>(step) * B + b] = s_best[0] - s_second[0];
+        if (p.want_lp) p.path_score[b] = __ldcg(p.path_score + b) + lp_step;
         if (advance) {
           p.t_idx[b] = __ldcg(p.t_idx + b) + 1; p.per[b] = 0; p.emit[b] = 0;
         } else {
           const int nt = __ldcg(p.ntok + b);
+          const long long o = static_cast<long long>(b) * p.max_len + nt - 1;
+          if (p.frames) p.frames[o] = __ldcg(p.frame_base + b) + __ldcg(p.t_idx + b);
+          if (p.token_logp) p.token_logp[o] = lp_step;
           p.tokens[static_cast<long long>(b) * p.max_len + nt - 1] = tok;
           p.ntok[b] = nt + 1; p.per[b] = __ldcg(p.per + b) + 1; p.emit[b] = 1; p.last_tok[b] = tok;
           rows_emit[atomicAdd(&counts[1], 1)] = b;
@@ -266,9 +282,14 @@ __global__ void __launch_bounds__(kThreads, 1) greedy_decode_kernel(DecodeArgs p
     grid_barrier(bar_counter, bar_target);
     lap(7);
   }
-  // every exit of the loop follows a grid barrier, so all ntok updates are visible here
-  if (cta == 0 && p.n_tokens != nullptr)
-    for (int b = tid; b < B; b += kThreads) p.n_tokens[b] = __ldcg(p.ntok + b);
+  // every exit of the loop follows a grid barrier, so all ntok updates are visible here; the frames this launch
+  // consumed move into the slot's frame base (a finished slot's count stops with it and restarts at its reset)
+  if (cta == 0)
+    for (int b = tid; b < B; b += kThreads) {
+      if (p.n_tokens != nullptr) p.n_tokens[b] = __ldcg(p.ntok + b);
+      if (p.path_scores != nullptr) p.path_scores[b] = __ldcg(p.path_score + b);
+      p.frame_base[b] = __ldcg(p.frame_base + b) + __ldcg(p.t_idx + b);
+    }
 }
 
 }  // namespace
@@ -282,7 +303,7 @@ size_t greedy_decode_scratch_bytes(int B, int H, int V, int E) {
   const size_t floats = 3 * pad4(b * H) /*feats, hbuf, lin*/ + pad4(b * V) /*logits*/ + pad4(b * 3 * E) + pad4(b * 5 * E) +
                         2 * pad4(b * E) /*ynew, z*/ + pad4(static_cast<size_t>(V) * E) /*LayerNorm(embedding) table*/ +
                         pad4(static_cast<size_t>(V) * 3 * E) /*conv1 tap table*/;
-  const size_t ints = b * 7 + 16;
+  const size_t ints = b * 7 + 16 + b /*frame_base*/ + b /*path_score (fp32, after the int regions)*/;
   return kTimerBytes + kBarBytes + floats * 4 + ints * 4 + 256;
 }
 
@@ -319,6 +340,8 @@ int launch_greedy_decode(DecodeArgs a, float* scratch, cudaStream_t stream) {
   a.rows = ip; ip += 2 * B;
   a.last_tok = ip; ip += B;
   a.flags = ip; ip += 16;
+  a.frame_base = ip; ip += B;
+  a.path_score = reinterpret_cast<float*>(ip); ip += B;
   RB_CUDA_CHECK(cudaFuncSetAttribute(greedy_decode_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int per_sm = 0;
   RB_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, greedy_decode_kernel, kThreads, smem));

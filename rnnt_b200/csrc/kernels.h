@@ -88,7 +88,8 @@ struct DecodeArgs {
   int* tokens;             // (B, max_len) emitted tokens (seed blank excluded)
   int* n_tokens;           // (B) output copy of ntok at the end of the launch (may be null)
   float* margins;          // (max_steps, B) top-2 logit gap per step (may be null)
-  // state (carved by the launcher): kept across launches -- feats, lin, acc1, acc2, emb_ln, t1, ntok, emit, last_tok;
+  // state (carved by the launcher): kept across launches -- feats, lin, acc1, acc2, emb_ln, t1, ntok, emit, last_tok,
+  // frame_base, path_score;
   // per-launch scratch -- hbuf, logits, ynew, z, t_idx, per, rows, flags
   float *feats, *hbuf, *logits, *acc1, *acc2, *ynew, *z, *lin, *emb_ln, *t1 /* conv1 tap table (NS, 3E) */;
   int* ntok;               // (B) 0 = empty slot, else 1 + number of emitted tokens (the predictor's next position)
@@ -96,6 +97,14 @@ struct DecodeArgs {
   unsigned* bar;           // grid-barrier counters (one per 128-byte line)
   int NS;                  // number of symbols = rows of the embedding table
   long long* prof;         // 8 cycle counters (block 0): P1, P2, P3, conv1 table build (once), P5, P6, -, grid barriers
+  // token timing and confidence: per emitted token its frame and log-probability, per slot the greedy path's score
+  int* frames;             // (B, max_len) frame of each emitted token, counted from the slot's reset (may be null)
+  float* token_logp;       // (B, max_len) log-softmax of the emitted token at its step (may be null)
+  float* path_scores;      // (B) output copy of path_score at the end of the launch (may be null)
+  int want_lp;             // 1: P3 takes each row's log-sum-exp and accumulates path_score (token_logp or path_scores
+                           // requested, and every streaming launch)
+  int* frame_base;         // state (B): frames consumed since the slot's reset, before this launch
+  float* path_score;       // state (B): sum of the step log-probabilities since the slot's reset
 };
 
 size_t greedy_decode_scratch_bytes(int B, int H, int V, int E);
@@ -112,6 +121,8 @@ struct BeamArgs : DecodeArgs {
   float* score;               // [2][B*K] running hypothesis scores
   unsigned long long* hash;   // [2][B*K] rolling hash of each token list (pre-filter of the merge test)
   int* hyp;                   // [2][B*K][max_len] token lists (seed blank excluded)
+  int* hyp_fr;                // [2][B*K][max_len] frame of each token (read and written only when `frames` or
+  float* hyp_lp;              // [2][B*K][max_len] its log-probability   `token_logp` is set)
 };
 constexpr int kMaxBeam = 8;
 

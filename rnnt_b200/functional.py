@@ -10,6 +10,7 @@ import ctypes as C
 import os
 from typing import NamedTuple, Optional
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -530,13 +531,26 @@ def _decode_params(joint_weight, joint_bias, p, dev):
             f(p.linear.bias), f(p.output_layer_norm.weight), f(p.output_layer_norm.bias)]
 
 
+class DecodedHypothesis(NamedTuple):
+    """One decoded hypothesis as host values: tokens (list[int]), frames (list[int], the encoder frame at which each
+    token was emitted), log_probs (list[float], each token's log-probability at its step) and score (float).  For greedy
+    decode the score is the log-probability of the greedy path through the transducer lattice, its blank steps
+    included; for beam search it is the hypothesis's beam score.  Seconds are frame * the encoder's frame shift."""
+    tokens: list
+    frames: list
+    log_probs: list
+    score: float
+
+
 def greedy_decode(audio_features, audio_feature_lens, joint_weight, joint_bias, predictor, blank: int,
-                  max_length: int = 200, max_outputs_per_step: int = 10, return_margins: bool = False):
+                  max_length: int = 200, max_outputs_per_step: int = 10, return_margins: bool = False,
+                  return_hypotheses: bool = False):
     """Batched greedy decode (rnnt/model.py:90-128 for every utterance of a batch) in ONE persistent CUDA kernel.
 
     audio_features (B,T,H) fp32, audio_feature_lens (B); `predictor` is a ConvPredictor-shaped module (embedding,
     input_layer_norm, conv1.conv, conv2.conv, linear, output_layer_norm).  Returns list[list[int]] (and, optionally,
-    per-utterance lists of top-2 logit margins for every step the utterance was active in)."""
+    per-utterance lists of top-2 logit margins for every step the utterance was active in).  With return_hypotheses,
+    one `DecodedHypothesis` per utterance replaces its token list (`rnnt_b200_greedy_decode_aligned`)."""
     _require_cuda(audio_features, joint_weight, joint_bias)
     L = _lib.lib()
     dev = audio_features.device
@@ -552,16 +566,26 @@ def greedy_decode(audio_features, audio_feature_lens, joint_weight, joint_bias, 
     ntok = torch.ones(B, dtype=torch.int32, device=dev)
     margins = torch.full((T + max_len + 2, B), float("inf"), device=dev) if return_margins else None
     scratch = torch.empty(L.rnnt_b200_greedy_decode_scratch_bytes(B, H, V, E), dtype=torch.uint8, device=dev)
-    with torch.cuda.device(dev):
-        _lib.check(L.rnnt_b200_greedy_decode(
-            enc.data_ptr(), enc.stride(0), enc.stride(1), lens.data_ptr(), *[t.data_ptr() for t in params],
+    args = (enc.data_ptr(), enc.stride(0), enc.stride(1), lens.data_ptr(), *[t.data_ptr() for t in params],
             B, T, H, V, E, int(blank), max_len, int(max_outputs_per_step), tokens.data_ptr(), ntok.data_ptr(),
-            margins.data_ptr() if return_margins else None, scratch.data_ptr(), _stream_ptr(dev)), "greedy_decode")
+            margins.data_ptr() if return_margins else None, scratch.data_ptr(), _stream_ptr(dev))
+    with torch.cuda.device(dev):
+        if return_hypotheses:
+            frames = torch.zeros(B, max_len, dtype=torch.int32, device=dev)
+            logp = torch.zeros(B, max_len, dtype=torch.float32, device=dev)
+            scores = torch.zeros(B, dtype=torch.float32, device=dev)
+            _lib.check(L.rnnt_b200_greedy_decode_aligned(*args, frames.data_ptr(), logp.data_ptr(),
+                                                         scores.data_ptr()), "greedy_decode_aligned")
+        else:
+            _lib.check(L.rnnt_b200_greedy_decode(*args), "greedy_decode")
     global _last_decode_phase_cycles
     _last_decode_phase_cycles = scratch[:64].view(torch.int64)
     n = (ntok - 1).tolist()
     toks = tokens.tolist()
     result = [toks[b][: n[b]] for b in range(B)]
+    if return_hypotheses:
+        fr, lp, sc = frames.tolist(), logp.tolist(), scores.tolist()
+        result = [DecodedHypothesis(result[b], fr[b][: n[b]], lp[b][: n[b]], sc[b]) for b in range(B)]
     if return_margins:
         ml = margins.t().tolist()
         return result, [[x for x in ml[b] if x != float("inf")] for b in range(B)]
@@ -572,13 +596,15 @@ MAX_BEAM = 8
 
 
 def beam_decode(audio_features, audio_feature_lens, joint_weight, joint_bias, predictor, blank: int,
-                beam_size: int = 4, max_length: int = 200):
+                beam_size: int = 4, max_length: int = 200, return_hypotheses: bool = False):
     """Batched frame-synchronous beam search (at most one symbol per frame, equal token lists merged with logaddexp) in
     ONE persistent CUDA kernel (`rnnt_b200_beam_decode`; include/rnnt_b200.h states the exact rule).
 
     audio_features (B,T,H) fp32 (any strides), audio_feature_lens (B); `predictor` is ConvPredictor-shaped, as for
     `greedy_decode`; beam_size in [1, 8]; max_length counts the seed blank.  Returns, per utterance, its n-best list:
-    up to beam_size (tokens, log-score) pairs, best first (fewer when fewer distinct token lists exist)."""
+    up to beam_size (tokens, log-score) pairs, best first (fewer when fewer distinct token lists exist).  With
+    return_hypotheses the pairs are `DecodedHypothesis` objects carrying each token's frame and log-probability too
+    (`rnnt_b200_beam_decode_aligned`)."""
     K = int(beam_size)
     if not 1 <= K <= MAX_BEAM:
         raise ValueError(f"beam_size must be in [1, {MAX_BEAM}] (got {beam_size})")
@@ -597,14 +623,24 @@ def beam_decode(audio_features, audio_feature_lens, joint_weight, joint_bias, pr
     ntok = torch.zeros(B, K, dtype=torch.int32, device=dev)
     scores = torch.empty(B, K, dtype=torch.float32, device=dev)
     scratch = torch.empty(L.rnnt_b200_beam_decode_scratch_bytes(B, K, H, V, E, max_len), dtype=torch.uint8, device=dev)
-    with torch.cuda.device(dev):
-        _lib.check(L.rnnt_b200_beam_decode(
-            enc.data_ptr(), enc.stride(0), enc.stride(1), lens.data_ptr(), *[t.data_ptr() for t in params],
+    args = (enc.data_ptr(), enc.stride(0), enc.stride(1), lens.data_ptr(), *[t.data_ptr() for t in params],
             B, T, H, V, E, int(blank), K, max_len, tokens.data_ptr(), ntok.data_ptr(), scores.data_ptr(),
-            scratch.data_ptr(), _stream_ptr(dev)), "beam_decode")
+            scratch.data_ptr(), _stream_ptr(dev))
+    with torch.cuda.device(dev):
+        if return_hypotheses:
+            frames = torch.zeros(B, K, max_len, dtype=torch.int32, device=dev)
+            logp = torch.zeros(B, K, max_len, dtype=torch.float32, device=dev)
+            _lib.check(L.rnnt_b200_beam_decode_aligned(*args, frames.data_ptr(), logp.data_ptr()),
+                       "beam_decode_aligned")
+        else:
+            _lib.check(L.rnnt_b200_beam_decode(*args), "beam_decode")
     global _last_decode_phase_cycles
     _last_decode_phase_cycles = scratch[:64].view(torch.int64)
     n, toks, sc = ntok.tolist(), tokens.tolist(), scores.tolist()
+    if return_hypotheses:
+        fr, lp = frames.tolist(), logp.tolist()
+        return [[DecodedHypothesis(toks[b][k][: n[b][k] - 1], fr[b][k][: n[b][k] - 1], lp[b][k][: n[b][k] - 1],
+                                   sc[b][k]) for k in range(K) if n[b][k] > 0] for b in range(B)]
     return [[(toks[b][k][: n[b][k] - 1], sc[b][k]) for k in range(K) if n[b][k] > 0] for b in range(B)]
 
 
@@ -629,7 +665,11 @@ class StreamingGreedyDecoder:
     its previous call stopped.  However an utterance's frames are split into chunks, its tokens (and per-step margins)
     are bit-identical to `greedy_decode` on the whole utterance with the same max_length / max_outputs_per_step.  The
     weights are re-laid for the kernel once and the per-symbol tables are built from them: call `refresh()` after the
-    weights change (it empties every slot)."""
+    weights change (it empties every slot).
+
+    Every call also records each new token's frame (counted from the slot's reset) and log-probability, and the slot's
+    running path score (`rnnt_b200_greedy_decode_stream_aligned`): `hypothesis(slot)` returns them, and
+    `decode_chunk(..., return_hypotheses=True)` returns the new tokens with theirs."""
 
     def __init__(self, joint, predictor, slots: int, max_length: int = 200, max_outputs_per_step: int = 10):
         _check_kernel_decode_modules(joint, predictor, "streaming decode")
@@ -653,6 +693,9 @@ class StreamingGreedyDecoder:
                                  device=self.dev)
         self.tokens = torch.zeros(S, self.max_length, **i32)     # column k-1 = k-th token of the slot's utterance
         self.n_tokens = torch.zeros(S, **i32)                    # 0 = empty slot, else 1 + tokens (seed blank counted)
+        self.frames = torch.zeros(S, self.max_length, **i32)     # frame of each token, counted from the slot's reset
+        self.token_logp = torch.zeros(S, self.max_length, dtype=torch.float32, device=self.dev)
+        self.scores = torch.zeros(S, dtype=torch.float32, device=self.dev)   # running path score since the reset
         self._reset_mask = torch.zeros(S, **i32)
         self._pending = set()                                    # host copy of the reset mask
         self._n_host = [0] * S                                   # host copy of n_tokens
@@ -667,6 +710,7 @@ class StreamingGreedyDecoder:
                 *[t.data_ptr() for t in self._params], self.slots, self.H, self.V, self.E, self.state.data_ptr(),
                 _stream_ptr(self.dev)), "greedy_decode_stream_init")
         self.n_tokens.zero_()
+        self.scores.zero_()
         self._n_host = [0] * self.slots
 
     def reset(self, slots) -> None:
@@ -687,11 +731,21 @@ class StreamingGreedyDecoder:
         """Every token the slot's current utterance has emitted so far."""
         return self.tokens[slot, : max(self._n_host[slot] - 1, 0)].tolist()
 
-    def decode_chunk(self, features, lens=None, return_margins: bool = False):
+    def hypothesis(self, slot: int) -> DecodedHypothesis:
+        """Everything the slot's current utterance has emitted so far: tokens, their frames (counted from the slot's
+        reset) and log-probabilities, and the running path score (log-probability of the greedy path so far).  Like
+        `transcript`, after `reset(slot)` it keeps returning the previous utterance until the next `decode_chunk`."""
+        n = max(self._n_host[slot] - 1, 0)
+        return DecodedHypothesis(self.tokens[slot, :n].tolist(), self.frames[slot, :n].tolist(),
+                                 self.token_logp[slot, :n].tolist(), float(self.scores[slot]))
+
+    def decode_chunk(self, features, lens=None, return_margins: bool = False, return_hypotheses: bool = False):
         """Feed the next chunk of encoder frames: features (slots, Tc, H) (any strides, e.g. the permuted view of the
         encoder's (slots, H, Tc) output), lens (slots,) = frames of the chunk each slot takes (default Tc, clamped to
         [0, Tc]).  Returns the tokens this call added per slot (and, optionally, the top-2 logit margins of every step
-        the slot took in this call).  Synchronises once, to return the tokens."""
+        the slot took in this call).  With return_hypotheses, each slot's entry is a `DecodedHypothesis` of the new
+        tokens, their frames and log-probabilities, and the slot's running path score.  Synchronises once, to return
+        the tokens."""
         _require_cuda(features)
         S, H = self.slots, self.H
         if features.dim() != 3 or features.shape[0] != S or features.shape[2] != H:
@@ -709,22 +763,32 @@ class StreamingGreedyDecoder:
         start = [0 if b in self._pending else max(n - 1, 0) for b, n in enumerate(self._n_host)]
         L = _lib.lib()
         with torch.cuda.device(self.dev):
-            _lib.check(L.rnnt_b200_greedy_decode_stream(
+            _lib.check(L.rnnt_b200_greedy_decode_stream_aligned(
                 enc.data_ptr(), enc.stride(0), enc.stride(1), chunk.data_ptr(), self._reset_mask.data_ptr(),
                 *[t.data_ptr() for t in self._params], S, Tc, H, self.V, self.E, self.blank, self.max_length,
                 self.max_outputs_per_step, self.tokens.data_ptr(), self.n_tokens.data_ptr(),
-                margins.data_ptr() if return_margins else None, self.state.data_ptr(), _stream_ptr(self.dev)),
-                "greedy_decode_stream")
+                margins.data_ptr() if return_margins else None, self.state.data_ptr(), _stream_ptr(self.dev),
+                self.frames.data_ptr(), self.token_logp.data_ptr(), self.scores.data_ptr()), "greedy_decode_stream")
             self._reset_mask.zero_()
             self._pending.clear()
             # the columns this call can have written, gathered on the device: one copy to the host
             cols = (torch.tensor(start, dtype=torch.int64, device=self.dev).view(S, 1)
                     + torch.arange(most, device=self.dev)).clamp(max=self.max_length - 1)
-            rows = torch.cat([self.n_tokens.view(S, 1), self.tokens.gather(1, cols)], 1).tolist()
+            parts = [self.n_tokens.view(S, 1), self.tokens.gather(1, cols)]
+            if return_hypotheses:   # the same single copy: frames, then log-probs and scores as their fp32 bits
+                parts += [self.frames.gather(1, cols), self.token_logp.gather(1, cols).view(torch.int32),
+                          self.scores.view(S, 1).view(torch.int32)]
+            host = torch.cat(parts, 1).cpu().numpy()
+            rows = host[:, : 1 + most].tolist()
         global _last_decode_phase_cycles
         _last_decode_phase_cycles = self.state[:64].view(torch.int64)
         self._n_host = [r[0] for r in rows]
         new = [rows[b][1: 1 + max(rows[b][0] - 1, 0) - start[b]] for b in range(S)]
+        if return_hypotheses:
+            fr = host[:, 1 + most: 1 + 2 * most].tolist()
+            lp = host[:, 1 + 2 * most: 1 + 3 * most].view(np.float32).tolist()
+            sc = host[:, 1 + 3 * most].view(np.float32).tolist()
+            new = [DecodedHypothesis(new[b], fr[b][: len(new[b])], lp[b][: len(new[b])], sc[b]) for b in range(S)]
         if return_margins:
             ml = margins.t().tolist()
             return new, [[x for x in ml[b] if x != float("inf")] for b in range(S)]

@@ -61,7 +61,8 @@ class RNNTModel(torch.nn.Module):
     @torch.no_grad()
     def greedy_decode_features(self, audio_features, audio_feature_lens, max_length: int = 200,
                                max_outputs_per_step: int = 10, return_margins: bool = False,
-                               use_cuda_graph: bool = True, sync_every: int = 16, engine: str = "kernel"):
+                               use_cuda_graph: bool = True, sync_every: int = 16, engine: str = "kernel",
+                               return_hypotheses: bool = False):
         """Batched greedy decode on given encoder features (B,T,H) with per-utterance lengths.
 
         Same per-utterance algorithm as rnnt/model.py:90-128 (blank or 10 emits advances the frame; stop at T_b or
@@ -70,12 +71,16 @@ class RNNTModel(torch.nn.Module):
         handful of elementwise ops.  engine="kernel" (default) runs everything inside ONE persistent cooperative CUDA
         kernel (`rnnt_b200_greedy_decode`); engine="graph" replays a captured CUDA graph of torch ops + the argmax
         kernel per step and checks for completion every `sync_every` steps (kept as an independent cross-check and
-        for joints with audio_ln / text_ln).  The reference syncs on `.item()` every step (model.py:113)."""
+        for joints with audio_ln / text_ln).  The reference syncs on `.item()` every step (model.py:113).
+        return_hypotheses=True (kernel engine only) returns one `DecodedHypothesis` per utterance: tokens with their
+        frames and log-probabilities, and the greedy path's score."""
         if not audio_features.is_cuda:
             raise RuntimeError("rnnt_b200 decode runs on CUDA tensors only; there is no CPU fallback")
         if _is_lstm_predictor(self.predictor):
             if return_margins:
                 raise ValueError("return_margins is only available with a ConvPredictor")
+            if return_hypotheses:
+                raise ValueError("return_hypotheses is only available with a ConvPredictor")
             return self._greedy_decode_features_stateful(audio_features, audio_feature_lens, max_length,
                                                          max_outputs_per_step)
         if not _is_conv_predictor(self.predictor):
@@ -85,7 +90,9 @@ class RNNTModel(torch.nn.Module):
             from .functional import greedy_decode
             return greedy_decode(audio_features, audio_feature_lens, self.joint.joint_ln.weight,
                                  self.joint.joint_ln.bias, self.predictor, self.joint.blank_idx, max_length,
-                                 max_outputs_per_step, return_margins)
+                                 max_outputs_per_step, return_margins, return_hypotheses)
+        if return_hypotheses:
+            raise ValueError("return_hypotheses needs engine='kernel' and a joint without audio_ln / text_ln")
         was_training = self.predictor.training
         self.predictor.eval()
         try:
@@ -109,22 +116,26 @@ class RNNTModel(torch.nn.Module):
         return StreamingGreedyDecoder(self.joint, self.predictor, slots, max_length, max_outputs_per_step)
 
     @torch.no_grad()
-    def beam_search_features(self, audio_features, audio_feature_lens, beam_size: int = 4, max_length: int = 200):
+    def beam_search_features(self, audio_features, audio_feature_lens, beam_size: int = 4, max_length: int = 200,
+                             return_hypotheses: bool = False):
         """Batched beam search on given encoder features (B,T,H) (e.g. the permuted view of the encoder's (B,H,T)
         output) with per-utterance lengths, in one persistent CUDA kernel (`functional.beam_decode`): per utterance,
-        up to beam_size (tokens, log-score) pairs, best first."""
+        up to beam_size (tokens, log-score) pairs, best first; with return_hypotheses, `DecodedHypothesis` objects
+        that also carry each token's frame and log-probability."""
         from .functional import _check_kernel_decode_modules, _require_cuda, beam_decode
         _check_kernel_decode_modules(self.joint, self.predictor, "beam search")
         _require_cuda(audio_features, self.joint.joint_ln.weight)
         return beam_decode(audio_features, torch.as_tensor(audio_feature_lens), self.joint.joint_ln.weight,
-                           self.joint.joint_ln.bias, self.predictor, self.joint.blank_idx, beam_size, max_length)
+                           self.joint.joint_ln.bias, self.predictor, self.joint.blank_idx, beam_size, max_length,
+                           return_hypotheses)
 
     @torch.no_grad()
-    def beam_search(self, mel_features, mel_feature_lens, beam_size: int = 4, max_length: int = 200):
+    def beam_search(self, mel_features, mel_feature_lens, beam_size: int = 4, max_length: int = 200,
+                    return_hypotheses: bool = False):
         """Beam search from mel features: the encoder and its output lengths first, then `beam_search_features`."""
         audio_features = self.encoder(mel_features).permute(0, 2, 1)
         audio_feature_lens = self.encoder.calc_output_lens(mel_feature_lens)
-        return self.beam_search_features(audio_features, audio_feature_lens, beam_size, max_length)
+        return self.beam_search_features(audio_features, audio_feature_lens, beam_size, max_length, return_hypotheses)
 
     @torch.no_grad()
     def _greedy_decode_features_hostloop(self, audio_features, audio_feature_lens, max_length: int = 200,
